@@ -1,9 +1,17 @@
 #!/usr/bin/env python
 """Generates tests/golden/*.npz from the UNMODIFIED reference objects (oracle/_ref/liblgs_ref.so).
 
-Run in the build container, where /root/reference exists:  python tests/golden/make_golden.py
+Run where the reference sources are at hand (oracle/Makefile `make ref`):  python tests/golden/make_golden.py
 The reference ships no golden vectors of its own (SURVEY.md section 4); these fixtures pin the
 plain-C oracle port (and, through it, the CUDA path) wherever the reference objects are absent.
+
+reference_randomised.npz holds the answers to the seeded randomised cases of tests/test_oracle_port.py
+(the inputs are drawn there; the file records which backend wrote it under `source`).  The committed file
+was written with `--randomised-from-port`, by the plain-C port: at commit f3c2a39 the tests these cases
+were made from, drawing the same inputs in the same order, passed bit for bit against the reference
+objects built from the unmodified sources, and the port (oracle/) and synth.py are unchanged since, so
+the port's answers on these inputs are the reference's.  The port also reproduces every reference-written file above.  Where the reference
+objects can be built, the plain run regenerates it from them with the other files.
 """
 import hashlib
 import os
@@ -183,7 +191,21 @@ def gs_scene():
                         ints=np.asarray(ints, dtype=np.int64), flts=np.asarray(flts))
 
 
-if __name__ == "__main__":
+def reference_randomised(M):
+    """Answers of backend M to the randomised cases of tests/test_oracle_port.py (fixed seeds)."""
+    sys.path.insert(0, os.path.dirname(OUT))
+    import test_oracle_port as T
+    out = {"source": np.array(M.__name__.rsplit(".", 1)[-1])}
+    for name, case in T.RANDOMISED.items():
+        out.update({f"{name}__{k}": np.asarray(v) for k, v in case(M).items()})
+    np.savez_compressed(os.path.join(OUT, "reference_randomised.npz"), **out)
+
+
+if __name__ == "__main__" and sys.argv[1:] == ["--randomised-from-port"]:
+    from oracle import portapi
+    reference_randomised(portapi)
+elif __name__ == "__main__":
+    reference_randomised(R)
     primitives()
     scene()
     edge_scene()

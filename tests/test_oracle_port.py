@@ -4,14 +4,12 @@ import hashlib
 import os
 
 import numpy as np
-import pytest
 
 from my_lidar_graph_slam_b200 import synth
 from oracle import portapi as P
 from oracle import refapi as R
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-needs_ref = pytest.mark.skipif(not R.available(), reason="oracle/_ref/liblgs_ref.so not built here")
 
 RT_PARAMS = [dict(low_res=5, range_x=0.2, range_y=0.2, range_theta=0.5, scan_range_max=20.0),
              dict(low_res=5, range_x=1.0, range_y=1.0, range_theta=1.0471975512, scan_range_max=5.7296),
@@ -150,75 +148,125 @@ def test_grid_search_golden():
         assert r.score == gf[0]
 
 
-@needs_ref
-def test_port_cost_matches_reference_objects_randomised():
+# ---- randomised cases: the port against the reference objects' answers on the same seeded inputs ----------------
+# Each case draws its inputs from a fixed seed and runs them through backend M (the port P or the reference
+# objects R).  tests/golden/reference_randomised.npz holds the reference's answers (make_golden.py); where
+# oracle/_ref/liblgs_ref.so is built, the port is also compared with the live objects.
+REF_GOLD = os.path.join(GOLD, "reference_randomised.npz")
+
+
+def _map(M, dense, min_x, min_y):
+    return (R.RefMap if M is R else P.PortMap).from_dense(dense, min_x, min_y)
+
+
+def _drawn(*arrays):
+    return sha(np.concatenate([np.ravel(np.asarray(a, dtype=np.float64)) for a in arrays]))
+
+
+def cost_case(M):
     rng = np.random.default_rng(31)
     dense = np.where(rng.random((128, 192)) < 0.5, np.round(rng.uniform(1e-3, 0.999, (128, 192)), 2), 0.0)
-    pm, rm = P.PortMap.from_dense(dense, -3.0, -2.0), R.RefMap.from_dense(dense, -3.0, -2.0)
+    m = _map(M, dense, -3.0, -2.0)
     angles = synth.beam_angles(91, 360.0)
+    drawn, cost, tail_n, tail_cov = [dense], [], [], []
     for _ in range(40):
         ranges = rng.uniform(0.0, 4.0, angles.shape)
         pose = np.array([rng.uniform(-3.5, 3.5), rng.uniform(-2.5, 3.0), rng.uniform(-4, 4)])   # partly off the map
         cs = (rng.uniform(0.0, 0.5), rng.uniform(2.0, 5.0), rng.uniform(0.02, 0.2), rng.uniform(0.05, 0.6),
               float(rng.integers(0, 4)), rng.uniform(0.1, 3.0), rng.uniform(0.02, 1.0))
         kw = dict(scan_min_range=float(rng.uniform(0, 0.3)), scan_max_range=float(rng.uniform(3, 6)), cost=cs)
-        assert P.cost_greedy_endpoint(pm, pose, angles, ranges, **kw) == \
-            R.cost_greedy_endpoint(rm, pose, angles, ranges, **kw)
-        n, _, cov = P.host_tail(pm, pose, angles, ranges, **kw)
-        rn, _, rcov = R.host_tail(rm, pose, angles, ranges, **kw)
-        assert n == rn and np.array_equal(cov, rcov)
+        drawn += [ranges, pose, cs, [kw["scan_min_range"], kw["scan_max_range"]]]
+        cost.append(M.cost_greedy_endpoint(m, pose, angles, ranges, **kw))
+        n, _, cov = M.host_tail(m, pose, angles, ranges, **kw)
+        tail_n.append(n)
+        tail_cov.append(cov)
+    return dict(inputs=_drawn(*drawn), cost=np.array(cost), tail_n=np.array(tail_n), tail_cov=np.array(tail_cov))
 
 
-@needs_ref
-def test_port_matches_reference_objects_randomised():
+def primitives_case(M):
     rng = np.random.default_rng(11)
+    ends, cells, offs = [], [], [0]
     for _ in range(300):
         e = [int(v) for v in rng.integers(-60, 61, 4)]
-        assert np.array_equal(P.bresenham(*e), R.bresenham(*e))
-    v = w = 0.0
-    for h in rng.random(500) < 0.45:
-        v, w = P.bayes_update(v, 0.6 if h else 0.45), R.bayes_update(w, 0.6 if h else 0.45)
-        assert v == w
+        c = np.asarray(M.bresenham(*e))
+        ends.append(e)
+        cells.append(c.reshape(-1, 2))
+        offs.append(offs[-1] + len(cells[-1]))
+    v, trace, hits = 0.0, [], rng.random(500) < 0.45
+    for h in hits:
+        v = M.bayes_update(v, 0.6 if h else 0.45)
+        trace.append(v)
+    sw_in, sw_out = [], []
     for n, win in [(50, 7), (50, 50), (50, 64), (7, 3), (1, 1), (130, 33)]:
         a = np.where(rng.random(n) < 0.6, rng.random(n), 0.0)
-        assert np.array_equal(P.sliding_window_max(a, win), R.sliding_window_max(a, win))
+        sw_in.append(a)
+        sw_out.append(np.asarray(M.sliding_window_max(a, win)))
     dense = np.where(rng.random((128, 192)) < 0.3, rng.uniform(1e-3, 0.999, (128, 192)), 0.0)
-    pm, rm = P.PortMap.from_dense(dense, -3.0, 2.0), R.RefMap.from_dense(dense, -3.0, 2.0)
-    for win in (1, 2, 5, 9, 64, 150, 400):
-        assert np.array_equal(pm.precompute(win).dense(), rm.precompute(win).dense())
-    for a, b in zip(pm.pyramid(7), rm.pyramid(7)):
-        assert np.array_equal(a.dense(), b.dense())
+    m = _map(M, dense, -3.0, 2.0)
+    return dict(inputs=_drawn(np.ravel(ends), hits, *sw_in, dense), bres_cells=np.concatenate(cells),
+                bres_offs=np.array(offs), bayes_trace=np.array(trace), sw_out=np.concatenate(sw_out),
+                pre_sha=np.array([sha(m.precompute(win).dense()) for win in (1, 2, 5, 9, 64, 150, 400)]),
+                pyr_sha=np.array([sha(p.dense()) for p in m.pyramid(7)]))
 
 
-@needs_ref
-def test_port_builder_and_matchers_match_reference_objects():
+def builder_case(M):
     world = synth.RoomsWorld(30.0, 5.0, seed=13)
     angles = synth.beam_angles(271, 270.0)
     traj = synth.trajectory(world, 30, step=0.3, seed=13)
     noise = np.random.default_rng(14)
     scans = [synth.make_scan(world, p, angles, noise) for p in traj]
-    rb, pb = R.RefBuilder(travel_thr=4.0), P.PortBuilder(travel_thr=4.0)   # forces several local maps
-    for p, s in zip(traj[:24], scans[:24]):
-        assert rb.append_scan(p, angles, s) == pb.append_scan(p, angles, s)
-    assert rb.num_local_maps() == pb.num_local_maps() >= 2
-    for i in range(rb.num_local_maps()):
-        a, b = rb.local_map(i), pb.local_map(i)
-        assert a.geometry() == b.geometry() and np.array_equal(a.dense(), b.dense())
-        assert rb.local_map_nodes(i) == pb.local_map_nodes(i)
-    a, b = rb.latest_map(), pb.latest_map()
-    assert a.geometry() == b.geometry() and np.array_equal(a.dense(), b.dense())
-    rm, pm = rb.local_map(1), pb.local_map(1)
-    rpyr, ppyr = rm.pyramid(5), pm.pyramid(5)
+    b = (R.RefBuilder if M is R else P.PortBuilder)(travel_thr=4.0)   # forces several local maps
+    appended = [b.append_scan(p, angles, s) for p, s in zip(traj[:24], scans[:24])]
+    n_local = b.num_local_maps()
+    maps = [b.local_map(i) for i in range(n_local)]
+    latest, lm = b.latest_map(), b.local_map(1)
+    pyr = lm.pyramid(5)
     prng = np.random.default_rng(15)
+    inits, rt_int, rt_f, bb_int, bb_score = [], [], [], [], []
     for k in range(24, 30):
         init = traj[k] + np.array([prng.uniform(-0.3, 0.3), prng.uniform(-0.3, 0.3), prng.uniform(-0.2, 0.2)])
+        inits.append(init)
         for p in RT_PARAMS:
-            x, y = R.rtcsm_match(a, angles, scans[k], init, **p), P.rtcsm_match(b, angles, scans[k], init, **p)
-            assert ints(x) == ints(y) and x.score == y.score and x.stepT == y.stepT
+            r = M.rtcsm_match(latest, angles, scans[k], init, **p)
+            rt_int.append(ints(r))
+            rt_f.append([r.score, r.stepT])
         for thr in (0.55, 0.2):
-            kw = dict(height_max=5, range_x=1.5, range_y=1.5, range_theta=0.6, thr=thr)
-            x = R.bb_match(rm, angles, scans[k], init, pyramid=rpyr, **kw)
-            y = P.bb_match(pm, angles, scans[k], init, pyramid=ppyr, **kw)
-            assert ints(x) == ints(y)
-            if x.found:
-                assert x.score == y.score
+            r = M.bb_match(lm, angles, scans[k], init, pyramid=pyr, thr=thr, height_max=5, range_x=1.5,
+                           range_y=1.5, range_theta=0.6)
+            bb_int.append(ints(r))
+            bb_score.append(r.score if r.found else 0.0)           # a score is only defined when found
+    return dict(inputs=_drawn(traj, *scans, *inits), appended=np.array(appended), n_local=np.array(n_local),
+                local_geom=np.array([m.geometry() for m in maps], dtype=np.float64),
+                local_sha=np.array([sha(m.dense()) for m in maps]),
+                local_nodes=np.array([b.local_map_nodes(i) for i in range(n_local)]),
+                latest_geom=np.array(latest.geometry(), dtype=np.float64), latest_sha=np.array(sha(latest.dense())),
+                rt_int=np.array(rt_int), rt_f=np.array(rt_f), bb_int=np.array(bb_int), bb_score=np.array(bb_score))
+
+
+RANDOMISED = {"cost": cost_case, "primitives": primitives_case, "builder": builder_case}
+
+
+def check_randomised(name):
+    got = RANDOMISED[name](P)
+    gold = np.load(REF_GOLD)
+    want = {k.split("__", 1)[1]: gold[k] for k in gold.files if k.startswith(name + "__")}
+    assert sorted(got) == sorted(want)
+    for k, v in got.items():
+        assert np.array_equal(np.asarray(v), want[k]), (name, k)
+    if R.available():
+        live = RANDOMISED[name](R)
+        for k, v in got.items():
+            assert np.array_equal(np.asarray(v), np.asarray(live[k])), (name, k, "live reference objects")
+
+
+def test_port_cost_matches_reference_objects_randomised():
+    check_randomised("cost")
+
+
+def test_port_matches_reference_objects_randomised():
+    check_randomised("primitives")
+
+
+def test_port_builder_and_matchers_match_reference_objects():
+    check_randomised("builder")
+    assert int(np.load(REF_GOLD)["builder__n_local"]) >= 2
