@@ -169,6 +169,21 @@ int lgs_grid_integrate_scans(lgs_ctx* ctx, lgs_grid* grid, const lgs_hit_batch* 
 int lgs_grid_integrate_submit(lgs_ctx* ctx, lgs_grid* grid, const lgs_hit_batch* scans,
                               double p_hit, double p_miss);
 int lgs_grid_integrate_wait(lgs_ctx* ctx, long long* n_updates);
+/* Many maps in one synchronous call: scans[i] into grids[i], i < n_maps -- every cell and n_updates[i]
+ * (optional) exactly as n_maps calls of lgs_grid_integrate_scans would leave them.  The rebuild after a
+ * loop closure (GridMapBuilder::AfterLoopClosure, grid_map_builder.cpp:62-80: every local map again from
+ * its corrected poses) is the intended caller -- GridMapBuilderCuda::AfterLoopClosure.  One staging copy,
+ * one pre-pass and one host sync for the whole call; a round of launches takes the next chunk of <= 64
+ * scans of every map, so maps of <= 64 scans cost a constant number of launches however many there are.
+ * All or nothing: if any scan of any map touches a cell outside its grid, the call fails with
+ * LGS_ERR_INVALID naming the map and the scan before any grid is written.  Grids may differ in size,
+ * resolution and apron and may belong to other contexts of the same device (ordered like lgs_grid_copy);
+ * maps without scans and scans without hits are allowed.  Refused (LGS_ERR_INVALID): a grid twice, a
+ * windowed grid, a grid on another device, and a call while a submitted integration on `ctx` has not
+ * been waited for. */
+int lgs_grid_integrate_many(lgs_ctx* ctx, int n_maps, lgs_grid* const* grids,
+                            const lgs_hit_batch* scans, double p_hit, double p_miss,
+                            long long* n_updates);
 
 /* Diagnostics: cells (cumulative over this context) whose fast candidate search disagreed with
  * the mark pass and were redone by the exhaustive exact path; expected to stay 0. */
@@ -196,6 +211,14 @@ int lgs_geometry_expand(const lgs_geometry* cur, double min_x, double min_y, dou
 int lgs_precompute(lgs_ctx* ctx, const lgs_grid* in, int win, lgs_grid* out);
 /* Levels 0..height_max with windows 1, 2, ..., 2^height_max (PrecomputeGridMaps). */
 int lgs_pyramid_create(lgs_ctx* ctx, const lgs_grid* in, int height_max, lgs_pyramid** out);
+/* The pyramids of n grids at once: out[i] is an ordinary pyramid of grids[i] (its own slab, freed by
+ * lgs_pyramid_destroy), level by level identical to lgs_pyramid_create's.  The apron clear, the level-0
+ * copy and each doubling level are one launch over all grids, so the launch count depends on height_max
+ * only.  The loop detector's pyramid cache, refilled after every loop closure, is the intended caller.
+ * Grids may belong to other contexts of the same device.  If an allocation fails, everything made so
+ * far is released, out[] is all NULL and the call returns LGS_ERR_NOMEM. */
+int lgs_pyramid_create_many(lgs_ctx* ctx, int n, const lgs_grid* const* grids, int height_max,
+                            lgs_pyramid** out);
 int lgs_pyramid_destroy(lgs_pyramid* p);
 int lgs_pyramid_download(const lgs_pyramid* p, int level, double* dense);
 int lgs_pyramid_levels(const lgs_pyramid* p);

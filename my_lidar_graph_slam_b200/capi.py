@@ -306,6 +306,21 @@ class Pyramid:
         ctx.check(lib().lgs_pyramid_create(ctx.h, grid.h, self.height_max, C.byref(self.h)))
         ctx.adopt(self)
 
+    @classmethod
+    def create_many(cls, ctx: Context, grids, height_max: int) -> list:
+        """The pyramids of all `grids` in one call (lgs_pyramid_create_many): one launch per pass."""
+        n = len(grids)
+        handles = (vp * max(n, 1))(*[g.h for g in grids])
+        out = (vp * max(n, 1))()
+        ctx.check(lib().lgs_pyramid_create_many(ctx.h, n, handles, int(height_max), out))
+        pyrs = []
+        for g, h in zip(grids, out):
+            p = cls.__new__(cls)
+            p.ctx, p.grid, p.height_max, p.h = ctx, g, int(height_max), vp(h)
+            ctx.adopt(p)
+            pyrs.append(p)
+        return pyrs
+
     def download(self, level: int):
         out = np.empty((self.grid.ny, self.grid.nx), dtype=np.float64)
         self.ctx.check(lib().lgs_pyramid_download(self.h, int(level), _dptr(out)))
@@ -710,6 +725,9 @@ SIGNATURES.update({
                                            C.POINTER(C.c_longlong)]),
     "lgs_grid_integrate_submit": (C.c_int, [vp, vp, C.POINTER(HitBatch), C.c_double, C.c_double]),
     "lgs_grid_integrate_wait": (C.c_int, [vp, C.POINTER(C.c_longlong)]),
+    "lgs_grid_integrate_many": (C.c_int, [vp, C.c_int, C.POINTER(vp), C.POINTER(HitBatch), C.c_double, C.c_double,
+                                          C.POINTER(C.c_longlong)]),
+    "lgs_pyramid_create_many": (C.c_int, [vp, C.c_int, C.POINTER(vp), C.c_int, C.POINTER(vp)]),
     "lgs_ctx_integrate_fallback_cells": (C.c_longlong, [vp]),
     "lgs_scan_hit_points": (C.c_int, [c_dp, C.c_int, c_dp, c_dp, C.c_double, C.c_double, c_dp,
                                       c_ip, c_dp]),
@@ -817,6 +835,20 @@ def integrate_wait(ctx: Context) -> int:
 def integrate_scans(ctx: Context, grid: Grid, sensor_xy, hits_list, p_hit=0.6, p_miss=0.45) -> int:
     """lgs_grid_integrate_scans for scans given as (sensor_xy[k][2], [hit_xy arrays]) -> updates."""
     return integrate_packed(ctx, grid, PackedHits(sensor_xy, hits_list), p_hit, p_miss)
+
+
+def integrate_many(ctx: Context, grids, sensor_xy_list, hits_lists, p_hit=0.6, p_miss=0.45) -> np.ndarray:
+    """lgs_grid_integrate_many: the scans of map i (sensor_xy_list[i], hits_lists[i]) into grids[i], all
+    maps in one call -> updates per map (int64 array)."""
+    n = len(grids)
+    assert len(sensor_xy_list) == n and len(hits_lists) == n
+    packs = [PackedHits(s, h) for s, h in zip(sensor_xy_list, hits_lists)]
+    batches = (HitBatch * max(n, 1))(*[p.c for p in packs])
+    handles = (vp * max(n, 1))(*[g.h for g in grids])
+    out = np.zeros(max(n, 1), dtype=np.int64)
+    ctx.check(lib().lgs_grid_integrate_many(ctx.h, n, handles, batches, p_hit, p_miss,
+                                            out.ctypes.data_as(C.POINTER(C.c_longlong))))
+    return out[:n]
 
 
 def measure_gather_peak(ctx: Context, nx=960, ny=640, row_lanes=25, aligned=False, local=True) -> float:

@@ -65,6 +65,50 @@ struct GridRef {
     double minX, minY, res;
 };
 
+// Grid of each scan in the pre-pass: one grid for the one-map entry points, a per-scan map index into a
+// device table of grids for lgs_grid_integrate_many.
+struct OneGrid {
+    GridRef g;
+    __device__ __forceinline__ GridRef of(int) const { return g; }
+};
+struct GridTable {
+    const GridRef* __restrict__ g;
+    const int* __restrict__ mapOf;
+    __device__ __forceinline__ GridRef of(int s) const { return g[mapOf[s]]; }
+};
+
+// A chunk's tile region (x0, y0, tw) inside a ROUND, the set of chunks -- of different maps -- that one
+// launch of each pass covers: the round's regions share one tile index space and one mark-pass grid.
+struct Region {
+    GridRef g;
+    int x0, y0, tw;      // tile-aligned origin (cells), tiles per region row
+    int tileBase;        // first tile of the region in the round's tile index space
+    int scanBase;        // first scan of the chunk (index into the call's ScanMeta)
+    int rowBase;         // first mark-pass row (blockIdx.y) of the chunk
+};
+
+// Region source of a round with one chunk (every round of the one-map entry points): nothing to look up.
+struct OneRegion {
+    Region r;            // tileBase == rowBase == 0
+    __device__ __forceinline__ Region byTile(int) const { return r; }
+    __device__ __forceinline__ Region byRow(int) const { return r; }
+};
+// Region source of a round with several chunks: the last region whose base is <= the index (bases ascend).
+struct RegionTable {
+    const Region* __restrict__ r;
+    int n;
+    __device__ __forceinline__ Region byTile(int t) const {
+        int lo = 0, hi = n - 1;
+        while (lo < hi) { const int mid = (lo + hi + 1) >> 1; if (r[mid].tileBase <= t) lo = mid; else hi = mid - 1; }
+        return r[lo];
+    }
+    __device__ __forceinline__ Region byRow(int y) const {
+        int lo = 0, hi = n - 1;
+        while (lo < hi) { const int mid = (lo + hi + 1) >> 1; if (r[mid].rowBase <= y) lo = mid; else hi = mid - 1; }
+        return r[lo];
+    }
+};
+
 __device__ __forceinline__ double clampProb(double v) {
     // std::clamp(v, ProbabilityMin, ProbabilityMax)  (binary_bayes_grid_cell.hpp:50-52, :97-101)
     const double lo = 1e-3, hi = 1.0 - 1e-3;
@@ -114,10 +158,12 @@ __device__ __forceinline__ int minorAt(int amin, int amaj, int k) {
 }
 
 // ---- pre-pass A: sensor cells ---------------------------------------------------------------------
+template <class Grids>
 __global__ void integ_sensor_kernel(const double* __restrict__ sensorXY, const int* __restrict__ hitBegin,
-                                    int nScans, GridRef g, ScanMeta* __restrict__ meta) {
+                                    int nScans, Grids grids, ScanMeta* __restrict__ meta) {
     const int s = blockIdx.x * blockDim.x + threadIdx.x;
     if (s >= nScans) return;
+    const GridRef g = grids.of(s);
     ScanMeta m;
     // WorldCoordinateToGridCellIndex (grid_map.hpp:779-790)
     m.sx = __double2int_rd(__ddiv_rn(__dsub_rn(sensorXY[2 * s], g.minX), g.res));
@@ -130,9 +176,12 @@ __global__ void integ_sensor_kernel(const double* __restrict__ sensorXY, const i
 }
 
 // ---- pre-pass B: per beam end cell relative to the sensor cell ---------------------------------------
-__global__ void integ_beam_kernel(const double* __restrict__ hitXY, GridRef g, ScanMeta* __restrict__ meta,
-                                  int2* __restrict__ rel) {
+// touches (NULL = not wanted): per scan, the Update calls of the CPU, one per cell of each ray.
+template <class Grids>
+__global__ void integ_beam_kernel(const double* __restrict__ hitXY, Grids grids, ScanMeta* __restrict__ meta,
+                                  int2* __restrict__ rel, unsigned long long* __restrict__ touches) {
     const int s = blockIdx.y;
+    const GridRef g = grids.of(s);
     const int n = meta[s].n, beamBegin = meta[s].beamBegin, sx = meta[s].sx, sy = meta[s].sy;
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     int len = 0;
@@ -146,6 +195,11 @@ __global__ void integ_beam_kernel(const double* __restrict__ hitXY, GridRef g, S
         rel[b] = make_int2(dx, dy);
         len = max(abs(dx), abs(dy));
     }
+    if (touches) {
+        unsigned cells = i < n ? (unsigned)len + 1u : 0u;
+        for (int o = 16; o > 0; o >>= 1) cells += __shfl_xor_sync(0xffffffffu, cells, o);
+        if ((threadIdx.x & 31) == 0 && cells) atomicAdd(touches + s, (unsigned long long)cells);
+    }
     for (int o = 16; o > 0; o >>= 1) len = max(len, __shfl_xor_sync(0xffffffffu, len, o));
     if ((threadIdx.x & 31) == 0 && len > 0) atomicMax(&meta[s].maxLen, len);
 }
@@ -155,12 +209,14 @@ __global__ void integ_beam_kernel(const double* __restrict__ hitXY, GridRef g, S
 // distance from the sensor, which mostly cross the same tiles.  A 16-step piece of a (monotone)
 // Bresenham path visits at most 3 tiles; for each of them the warp groups the lanes that share the
 // tile and issues ONE atomicMin (lowest beam of the group) and ONE atomicMax (highest beam).
-// (x0, y0) = tile-aligned origin of the chunk's region, tw = tiles per region row.
+// Row blockIdx.y = scan s of the chunk of region R; its tiles are R.tileBase + the tile in R's region.
+template <class Regions>
 __global__ void __launch_bounds__(128)
-integ_mark_kernel(const ScanMeta* __restrict__ meta, const int2* __restrict__ rel, int x0, int y0, int tw,
+integ_mark_kernel(const ScanMeta* __restrict__ meta, const int2* __restrict__ rel, Regions regions,
                   int beamsPad, unsigned* __restrict__ kmin, unsigned* __restrict__ kmax) {
-    const int s = blockIdx.y;
-    const ScanMeta m = meta[s];
+    const Region R = regions.byRow(blockIdx.y);
+    const int s = blockIdx.y - R.rowBase;
+    const ScanMeta m = meta[R.scanBase + s];
     const int t = blockIdx.x * blockDim.x + threadIdx.x;        // beamsPad is a multiple of 32:
     const int i = t % beamsPad, piece = t / beamsPad;           // a warp never straddles two pieces
     const int lane = threadIdx.x & 31;
@@ -174,7 +230,7 @@ integ_mark_kernel(const ScanMeta* __restrict__ meta, const int2* __restrict__ re
         if (kBegin <= amaj) {
             const int kEnd = min(kBegin + kTile - 1, amaj);
             const int sMaj = (xMajor ? e.x : e.y) < 0 ? -1 : 1, sMin = (xMajor ? e.y : e.x) < 0 ? -1 : 1;
-            const int bx = m.sx - x0, by = m.sy - y0;
+            const int bx = m.sx - R.x0, by = m.sy - R.y0;
             const int m2 = 2 * amaj, d2 = 2 * amin;
             int minor = amaj ? minorAt(amin, amaj, kBegin) : 0;
             int rem = d2 * kBegin + amaj - minor * m2;
@@ -182,7 +238,7 @@ integ_mark_kernel(const ScanMeta* __restrict__ meta, const int2* __restrict__ re
             for (int k = kBegin; k <= kEnd; ++k) {
                 const int x = bx + (xMajor ? sMaj * k : sMin * minor);
                 const int y = by + (xMajor ? sMin * minor : sMaj * k);
-                const int tile = (y >> kTileShift) * tw + (x >> kTileShift);
+                const int tile = R.tileBase + (y >> kTileShift) * R.tw + (x >> kTileShift);
                 if (tile != last) {
                     last = tile;
                     if (nt == 0) tiles[0] = tile; else if (nt == 1) tiles[1] = tile; else tiles[2] = tile;
@@ -215,13 +271,16 @@ integ_mark_kernel(const ScanMeta* __restrict__ meta, const int2* __restrict__ re
 // Descriptor = two int4: {ox, oy, k0, k1} (tile origin relative to the scan's sensor cell, beam range)
 // and {beamBegin, tile, scan, 0}, so the touch pass needs no further dependent look-ups.
 // One warp per tile: lanes read the tile's 64 kmax entries (non-zero = the scan touches the tile).
+template <class Regions>
 __global__ void __launch_bounds__(128)
-integ_pairs_kernel(int nTiles, const ScanMeta* __restrict__ meta, int x0, int y0, int tw,
+integ_pairs_kernel(int nTiles, const ScanMeta* __restrict__ meta, Regions regions,
                    unsigned* __restrict__ kmin, unsigned* __restrict__ kmax,
                    uint2* __restrict__ tileInfo, int4* __restrict__ pairs, unsigned* __restrict__ nPairs) {
     const int t = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
     if (t >= nTiles) return;
+    const Region R = regions.byTile(t);
+    const int lt = t - R.tileBase;
     const size_t idx = (size_t)t * kChunk + lane;
     const unsigned hiA = kmax[idx], hiB = kmax[idx + 32];
     const unsigned mA = __ballot_sync(0xffffffffu, hiA != 0u), mB = __ballot_sync(0xffffffffu, hiB != 0u);
@@ -231,9 +290,9 @@ integ_pairs_kernel(int nTiles, const ScanMeta* __restrict__ meta, int x0, int y0
     base = __shfl_sync(0xffffffffu, base, 0);
     if (lane == 0) tileInfo[t] = make_uint2(base, cnt);
     const unsigned below = (1u << lane) - 1u;
-    const int tx = x0 + (t % tw) * kTile, ty = y0 + (t / tw) * kTile;
+    const int tx = R.x0 + (lt % R.tw) * kTile, ty = R.y0 + (lt / R.tw) * kTile;
     auto emit = [&](unsigned slot, int s, unsigned lo, unsigned hi) {
-        const ScanMeta m = meta[s];
+        const ScanMeta m = meta[R.scanBase + s];
         pairs[2 * (size_t)slot] = make_int4(tx - m.sx, ty - m.sy, (int)lo, (int)hi);
         pairs[2 * (size_t)slot + 1] = make_int4(m.beamBegin, t, s, 0);
     };
@@ -487,13 +546,17 @@ struct Folder {
     }
 };
 
+template <class Regions>
 __global__ void __launch_bounds__(kTileCells)
-integ_fold_kernel(FoldArgs a, GridRef g, int x0, int y0, int tw) {
+integ_fold_kernel(FoldArgs a, Regions regions) {
     const uint2 info = a.tileInfo[blockIdx.x];
     if (info.y == 0u) return;
+    const Region reg = regions.byTile(blockIdx.x);
+    const GridRef& g = reg.g;
+    const int lt = blockIdx.x - reg.tileBase;
     const int tid = threadIdx.x;
-    const int cx = x0 + (blockIdx.x % tw) * kTile + (tid & (kTile - 1));
-    const int cy = y0 + (blockIdx.x / tw) * kTile + (tid >> kTileShift);
+    const int cx = reg.x0 + (lt % reg.tw) * kTile + (tid & (kTile - 1));
+    const int cy = reg.y0 + (lt / reg.tw) * kTile + (tid >> kTileShift);
     const bool inside = cx < g.nx && cy < g.ny;
     double* cell = g.origin + (size_t)cy * g.pitch + cx;
     const double v0 = inside ? *cell : 0.0;
@@ -602,17 +665,35 @@ int integ_wait(lgs_ctx* c, long long* nUpdatesOut) {
 }
 
 // Everything of a call up to the last enqueue; the host waits only for the pre-pass (scan bounds).
-int integ_submit(lgs_ctx* c, lgs_grid* grid, const lgs_hit_batch* scans, double pHit, double pMiss) {
-    const int n = scans->n_scans;
-    if (n < 0 || (n > 0 && (!scans->sensor_xy || !scans->hit_begin)))
-        return lgs_fail(c, LGS_ERR_INVALID, "integrate: bad scan batch");
-    if (n == 0) return LGS_OK;                       // nothing in flight: the matching wait reports 0 updates
-    if (grid->off_x || grid->off_y)
-        return lgs_fail(c, LGS_ERR_INVALID, "integrate: windowed grids (lgs_grid_set_window) are not supported");
-    const long long total = n > 0 ? scans->hit_begin[n] : 0;
-    if (total > 0 && !scans->hit_xy) return lgs_fail(c, LGS_ERR_INVALID, "integrate: hit_xy is NULL");
+// A call integrates batches[i] into grids[i], i < nMaps.  The one-map entry points pass one map; `many`
+// (lgs_grid_integrate_many, arguments checked by the caller) stages every map into one blob behind a
+// device table of grids, returns each map's update count in perMap, and packs the next chunk of every
+// map into one round of launches.
+int integ_submit(lgs_ctx* c, int nMaps, lgs_grid* const* grids, const lgs_hit_batch* batches, double pHit,
+                 double pMiss, bool many, long long* perMap) {
+    if (!many) {
+        const lgs_hit_batch* scans = batches;
+        const int n = scans->n_scans;
+        if (n < 0 || (n > 0 && (!scans->sensor_xy || !scans->hit_begin)))
+            return lgs_fail(c, LGS_ERR_INVALID, "integrate: bad scan batch");
+        if (n == 0) return LGS_OK;                   // nothing in flight: the matching wait reports 0 updates
+        if (grids[0]->off_x || grids[0]->off_y)
+            return lgs_fail(c, LGS_ERR_INVALID, "integrate: windowed grids (lgs_grid_set_window) are not supported");
+        if (scans->hit_begin[n] > 0 && !scans->hit_xy) return lgs_fail(c, LGS_ERR_INVALID, "integrate: hit_xy is NULL");
+    }
+    // scans of map i are scans [scanBase[i], scanBase[i + 1]) of the call, their hits start at hitBase[i]
+    std::vector<int> scanBase(nMaps + 1, 0);
+    std::vector<long long> hitBase(nMaps + 1, 0);
+    for (int i = 0; i < nMaps; ++i) {
+        scanBase[i + 1] = scanBase[i] + batches[i].n_scans;
+        hitBase[i + 1] = hitBase[i] + (batches[i].n_scans > 0 ? batches[i].hit_begin[batches[i].n_scans] : 0);
+    }
+    const int n = scanBase[nMaps];
+    const long long total = hitBase[nMaps];
+    if (n == 0) return LGS_OK;
+    if (total > 0x7fffffffLL) return lgs_fail(c, LGS_ERR_INVALID, "integrate: %lld hits in one call (at most 2^31 - 1)", total);
     LGS_CUDA(c, cudaSetDevice(c->device));
-    LGS_CUDA(c, lgs_grid_acquire(c, grid));
+    for (int i = 0; i < nMaps; ++i) LGS_CUDA(c, lgs_grid_acquire(c, grids[i]));
     if (!c->integ) c->integ = new lgs_integ_ws();
     lgs_integ_ws& ws = *c->integ;
     if (ws.nPending >= 2 || ws.stage[ws.calls & 1].pending)
@@ -652,33 +733,98 @@ int integ_submit(lgs_ctx* c, lgs_grid* grid, const lgs_hit_batch* scans, double 
     LGS_CUDA(c, w.counters.reserve(8));
     LGS_CUDA(c, w.hMeta.reserve((size_t)n * sizeof(ScanMeta)));
     LGS_CUDA(c, w.hCounters.reserve(8));
-    LGS_CUDA(c, cudaMemcpyAsync(w.sensor.p, scans->sensor_xy, (size_t)n * 2 * sizeof(double), cudaMemcpyHostToDevice, cs0));
-    if (total)
-        LGS_CUDA(c, cudaMemcpyAsync(w.hit.p, scans->hit_xy, (size_t)total * 2 * sizeof(double), cudaMemcpyHostToDevice, cs0));
-    LGS_CUDA(c, cudaMemcpyAsync(w.begin.p, scans->hit_begin, (size_t)(n + 1) * sizeof(int), cudaMemcpyHostToDevice, cs0));
+    // lgs_grid_integrate_many: hit offsets rebased into the blob, per-scan map index, grid table (pageable
+    // host vectors: the copies have taken them when cudaMemcpyAsync returns)
+    std::vector<int> hBegin;
+    std::vector<char> hTab;
+    const GridRef* dGrids = nullptr;
+    const int* dMapOf = nullptr;
+    unsigned long long* dTouches = nullptr;
+    if (many) {
+        hBegin.resize((size_t)n + 1);
+        hTab.resize((size_t)nMaps * sizeof(GridRef) + (size_t)n * sizeof(int));
+        GridRef* tg = reinterpret_cast<GridRef*>(hTab.data());
+        int* mapOf = reinterpret_cast<int*>(hTab.data() + (size_t)nMaps * sizeof(GridRef));
+        for (int i = 0; i < nMaps; ++i) {
+            const lgs_grid* gr = grids[i];
+            tg[i] = GridRef{const_cast<lgs_grid*>(gr)->origin(), gr->nx, gr->ny, gr->pitch, gr->min_x, gr->min_y, gr->res};
+            for (int s = 0; s < batches[i].n_scans; ++s) {
+                hBegin[scanBase[i] + s] = (int)(hitBase[i] + batches[i].hit_begin[s]);
+                mapOf[scanBase[i] + s] = i;
+            }
+        }
+        hBegin[n] = (int)total;
+        LGS_CUDA(c, ws.manyTab.reserve(hTab.size()));
+        LGS_CUDA(c, ws.manyTouches.reserve((size_t)n));
+        LGS_CUDA(c, ws.hManyTouches.reserve((size_t)n));
+        dGrids = reinterpret_cast<const GridRef*>(ws.manyTab.p);
+        dMapOf = reinterpret_cast<const int*>(ws.manyTab.p + (size_t)nMaps * sizeof(GridRef));
+        dTouches = ws.manyTouches.p;
+        for (int i = 0; i < nMaps; ++i) {
+            const lgs_hit_batch& b = batches[i];
+            if (b.n_scans == 0) continue;
+            LGS_CUDA(c, cudaMemcpyAsync(w.sensor.p + 2 * (size_t)scanBase[i], b.sensor_xy,
+                                        (size_t)b.n_scans * 2 * sizeof(double), cudaMemcpyHostToDevice, cs0));
+            if (hitBase[i + 1] > hitBase[i])
+                LGS_CUDA(c, cudaMemcpyAsync(w.hit.p + 2 * (size_t)hitBase[i], b.hit_xy,
+                                            (size_t)(hitBase[i + 1] - hitBase[i]) * 2 * sizeof(double),
+                                            cudaMemcpyHostToDevice, cs0));
+        }
+        LGS_CUDA(c, cudaMemcpyAsync(w.begin.p, hBegin.data(), (size_t)(n + 1) * sizeof(int), cudaMemcpyHostToDevice, cs0));
+        LGS_CUDA(c, cudaMemcpyAsync(ws.manyTab.p, hTab.data(), hTab.size(), cudaMemcpyHostToDevice, cs0));
+        LGS_CUDA(c, cudaMemsetAsync(dTouches, 0, (size_t)n * sizeof(unsigned long long), cs0));
+    } else {
+        const lgs_hit_batch* scans = batches;
+        LGS_CUDA(c, cudaMemcpyAsync(w.sensor.p, scans->sensor_xy, (size_t)n * 2 * sizeof(double), cudaMemcpyHostToDevice, cs0));
+        if (total)
+            LGS_CUDA(c, cudaMemcpyAsync(w.hit.p, scans->hit_xy, (size_t)total * 2 * sizeof(double), cudaMemcpyHostToDevice, cs0));
+        LGS_CUDA(c, cudaMemcpyAsync(w.begin.p, scans->hit_begin, (size_t)(n + 1) * sizeof(int), cudaMemcpyHostToDevice, cs0));
+    }
     LGS_CUDA(c, cudaMemsetAsync(w.counters.p, 0, 8 * sizeof(unsigned long long), cs0));
     tStage = msSince(tStart);
 
     int maxBeams = 0;
-    for (int s = 0; s < n; ++s) maxBeams = std::max(maxBeams, scans->hit_begin[s + 1] - scans->hit_begin[s]);
+    for (int i = 0; i < nMaps; ++i)
+        for (int s = 0; s < batches[i].n_scans; ++s)
+            maxBeams = std::max(maxBeams, batches[i].hit_begin[s + 1] - batches[i].hit_begin[s]);
     ScanMeta* dMeta = reinterpret_cast<ScanMeta*>(w.meta.p);
     ScanMeta* hMeta = reinterpret_cast<ScanMeta*>(w.hMeta.p);
-    GridRef g{grid->origin(), grid->nx, grid->ny, grid->pitch, grid->min_x, grid->min_y, grid->res};
     // Pre-pass over the whole batch: sensor cells, relative end cells, ray lengths, bounds check.
-    integ_sensor_kernel<<<(n + 127) / 128, 128, 0, cs0>>>(w.sensor.p, w.begin.p, n, g, dMeta);
-    LGS_LAUNCH_CHECK(c);
-    if (maxBeams > 0) {
-        dim3 gb((maxBeams + 127) / 128, n);
-        integ_beam_kernel<<<gb, 128, 0, cs0>>>(w.hit.p, g, dMeta, w.rel.p);
+    if (many) {
+        integ_sensor_kernel<<<(n + 127) / 128, 128, 0, cs0>>>(w.sensor.p, w.begin.p, n, GridTable{dGrids, dMapOf}, dMeta);
         LGS_LAUNCH_CHECK(c);
+        for (int s0 = 0; maxBeams > 0 && s0 < n; s0 += 65535) {       // grid rows: at most 65535 scans a launch
+            dim3 gb((maxBeams + 127) / 128, std::min(n - s0, 65535));
+            integ_beam_kernel<<<gb, 128, 0, cs0>>>(w.hit.p, GridTable{dGrids, dMapOf + s0}, dMeta + s0, w.rel.p,
+                                                   dTouches + s0);
+            LGS_LAUNCH_CHECK(c);
+        }
+        LGS_CUDA(c, cudaMemcpyAsync(ws.hManyTouches.p, dTouches, (size_t)n * sizeof(unsigned long long),
+                                    cudaMemcpyDeviceToHost, cs0));
+    } else {
+        const lgs_grid* grid = grids[0];
+        const OneGrid g{GridRef{grids[0]->origin(), grid->nx, grid->ny, grid->pitch, grid->min_x, grid->min_y, grid->res}};
+        integ_sensor_kernel<<<(n + 127) / 128, 128, 0, cs0>>>(w.sensor.p, w.begin.p, n, g, dMeta);
+        LGS_LAUNCH_CHECK(c);
+        if (maxBeams > 0) {
+            dim3 gb((maxBeams + 127) / 128, n);
+            integ_beam_kernel<<<gb, 128, 0, cs0>>>(w.hit.p, g, dMeta, w.rel.p, nullptr);
+            LGS_LAUNCH_CHECK(c);
+        }
     }
     LGS_CUDA(c, cudaMemcpyAsync(hMeta, dMeta, (size_t)n * sizeof(ScanMeta), cudaMemcpyDeviceToHost, cs0));
     LGS_CUDA(c, cudaStreamSynchronize(cs0));
     tPre = msSince(tStart);
-    for (int s = 0; s < n; ++s)
-        if (hMeta[s].bad)
-            return lgs_fail(c, LGS_ERR_INVALID, "integrate: scan %d touches cells outside the %dx%d grid "
-                            "(expand the map first, as GridMap::Expand does)", s, grid->nx, grid->ny);
+    for (int i = 0; i < nMaps; ++i)
+        for (int s = scanBase[i]; s < scanBase[i + 1]; ++s)
+            if (hMeta[s].bad) {
+                if (many)
+                    return lgs_fail(c, LGS_ERR_INVALID, "integrate_many: map %d, scan %d touches cells outside the "
+                                    "%dx%d grid (expand the map first, as GridMap::Expand does)", i, s - scanBase[i],
+                                    grids[i]->nx, grids[i]->ny);
+                return lgs_fail(c, LGS_ERR_INVALID, "integrate: scan %d touches cells outside the %dx%d grid "
+                                "(expand the map first, as GridMap::Expand does)", s, grids[i]->nx, grids[i]->ny);
+            }
 
     // ValueToOdds(prob) for the two observations (binary_bayes_grid_cell.hpp:104-113), host IEEE.
     auto clampP = [](double v) { const double lo = 1e-3, hi = 1.0 - 1e-3; return v < lo ? lo : (hi < v ? hi : v); };
@@ -691,12 +837,13 @@ int integ_submit(lgs_ctx* c, lgs_grid* grid, const lgs_hit_batch* scans, double 
     if (c->opt.integSideWords > 0) sideCap = (size_t)std::max<long long>(8, c->opt.integSideWords);
     // tiles of scan s's reach: the square of half side maxLen around the sensor cell
     auto tileSpan = [](int lo, int hi) { return (hi >> kTileShift) - (lo >> kTileShift) + 1; };
+
     // LGS_INTEG_TIMING=1 (diagnostic): CUDA-event time of every pass, summed over the call, to stderr.
     const bool timing = c->opt.integTiming != 0;
     const bool diag = timing && c->opt.integDiag != 0;   // + per-cell update counts (slows the fold)
     std::vector<cudaEvent_t> evs;
     auto stamp = [&]() { if (timing) { cudaEvent_t e; cudaEventCreate(&e); cudaEventRecord(e, c->stream); evs.push_back(e); } };
-    // The fold pass runs on a second stream so that it overlaps the next chunk's touch passes
+    // The fold pass runs on a second stream so that it overlaps the next round's touch passes
     // (LGS_INTEG_TIMING serialises everything on the context stream to time the passes).
     const bool overlap = !timing;
     if (!w.foldStream) {
@@ -706,35 +853,24 @@ int integ_submit(lgs_ctx* c, lgs_grid* grid, const lgs_hit_batch* scans, double 
             LGS_CUDA(c, cudaEventCreateWithFlags(&w.evFold[b], cudaEventDisableTiming));
         }
     }
+    // Rounds: consecutive chunks (below) share one launch of each pass while the round holds at most one chunk
+    // per map (the fold owns the map's cells), and its records, tile index space and mark-pass rows stay within
+    // the limits of one chunk.  A round is launched as soon as it is closed; one with several chunks takes its
+    // regions from a table at its own place in manyRegions (a one-chunk round needs none).
+    struct Round { int first, count, rows, beams, len; size_t tiles, pairBound; };
+    std::vector<Region> regions;
+    if (many) LGS_CUDA(c, ws.manyRegions.reserve((size_t)n * sizeof(Region)));   // a chunk holds >= 1 scan
     int lastBuf = -1;
-    int s0 = 0;
-    while (s0 < n) {
-        // grow the chunk while it stays within 64 scans and the record budget
-        int x0 = grid->nx, y0 = grid->ny, x1 = -1, y1 = -1, subBeams = 0, subLen = 0, ns = 0;
-        size_t pairBound = 0;
-        while (s0 + ns < n && ns < kChunk) {
-            const ScanMeta& m = hMeta[s0 + ns];
-            if (m.n > 0) {
-                const int lx = std::max(m.sx - m.maxLen, 0), hx = std::min(m.sx + m.maxLen, grid->nx - 1);
-                const int ly = std::max(m.sy - m.maxLen, 0), hy = std::min(m.sy + m.maxLen, grid->ny - 1);
-                const size_t pb = (size_t)tileSpan(lx, hx) * tileSpan(ly, hy);
-                if (ns > 0 && (pairBound + pb) * kTileCells * sizeof(unsigned) > kRecordBudget) break;
-                pairBound += pb;
-                x0 = std::min(x0, lx); x1 = std::max(x1, hx);
-                y0 = std::min(y0, ly); y1 = std::max(y1, hy);
-                subBeams = std::max(subBeams, m.n);
-                subLen = std::max(subLen, m.maxLen);
-            }
-            ++ns;
+    auto launchRound = [&](const Round& rd) -> int {
+        const size_t nTiles = rd.tiles, pairBound = rd.pairBound;
+        const OneRegion one{regions[rd.first]};
+        RegionTable table{nullptr, rd.count};
+        if (rd.count > 1) {
+            Region* dst = reinterpret_cast<Region*>(ws.manyRegions.p) + rd.first;
+            LGS_CUDA(c, cudaMemcpyAsync(dst, regions.data() + rd.first, (size_t)rd.count * sizeof(Region),
+                                        cudaMemcpyHostToDevice, c->stream));
+            table.r = dst;
         }
-        const int cs = s0;
-        s0 += ns;
-        if (subBeams == 0 || x1 < x0 || y1 < y0) continue;
-        x0 &= ~(kTile - 1); y0 &= ~(kTile - 1);                       // tile-aligned region origin
-        const int tw = tileSpan(x0, x1), th = tileSpan(y0, y1);
-        const size_t nTiles = (size_t)tw * th;
-        if (nTiles * kChunk >= ((size_t)1 << 31)) return lgs_fail(c, LGS_ERR_INVALID, "integrate: region of %dx%d tiles is too large", tw, th);
-        pairBound = std::min(pairBound, nTiles * ns);
 
         // mark buffers: kept in their reset state by the pair pass; (re)initialise what is new
         if (w.dirty) { w.cleanTiles = 0; w.dirty = false; }
@@ -743,7 +879,7 @@ int integ_submit(lgs_ctx* c, lgs_grid* grid, const lgs_hit_batch* scans, double 
         LGS_CUDA(c, w.kmax.reserve(nTiles * kChunk));
         const int buf = (int)(ws.chunks & 1);
         ++ws.chunks;
-        // this buffer's previous fold (chunk k - 2, possibly of the previous call) must be done before it is
+        // this buffer's previous fold (round k - 2, possibly of the previous call) must be done before it is
         // overwritten: the context stream waits for it; only a buffer that has to grow makes the host wait
         // (reallocation frees)
         if (ws.usedBuf[buf]) {
@@ -767,13 +903,19 @@ int integ_submit(lgs_ctx* c, lgs_grid* grid, const lgs_hit_batch* scans, double 
 
         w.dirty = true;
         stamp();
-        const int beamsPad = (subBeams + 31) & ~31, pieces = subLen / kTile + 1;
-        dim3 gm((unsigned)(((size_t)beamsPad * pieces + 127) / 128), ns);
-        integ_mark_kernel<<<gm, 128, 0, c->stream>>>(dMeta + cs, w.rel.p, x0, y0, tw, beamsPad, w.kmin.p, w.kmax.p);
+        const int beamsPad = (rd.beams + 31) & ~31, pieces = rd.len / kTile + 1;
+        dim3 gm((unsigned)(((size_t)beamsPad * pieces + 127) / 128), rd.rows);
+        if (rd.count == 1) integ_mark_kernel<<<gm, 128, 0, c->stream>>>(dMeta, w.rel.p, one, beamsPad, w.kmin.p, w.kmax.p);
+        else integ_mark_kernel<<<gm, 128, 0, c->stream>>>(dMeta, w.rel.p, table, beamsPad, w.kmin.p, w.kmax.p);
         LGS_LAUNCH_CHECK(c);
         stamp();
-        integ_pairs_kernel<<<(unsigned)((nTiles * 32 + 127) / 128), 128, 0, c->stream>>>((int)nTiles, dMeta + cs, x0, y0, tw, w.kmin.p, w.kmax.p,
-                                                                                       w.tileInfo[buf].p, w.pairs[buf].p, nPairs);
+        const unsigned pairBlocks = (unsigned)((nTiles * 32 + 127) / 128);
+        if (rd.count == 1)
+            integ_pairs_kernel<<<pairBlocks, 128, 0, c->stream>>>((int)nTiles, dMeta, one, w.kmin.p, w.kmax.p,
+                                                                  w.tileInfo[buf].p, w.pairs[buf].p, nPairs);
+        else
+            integ_pairs_kernel<<<pairBlocks, 128, 0, c->stream>>>((int)nTiles, dMeta, table, w.kmin.p, w.kmax.p,
+                                                                  w.tileInfo[buf].p, w.pairs[buf].p, nPairs);
         LGS_LAUNCH_CHECK(c);
         stamp();
         w.dirty = false;
@@ -783,18 +925,82 @@ int integ_submit(lgs_ctx* c, lgs_grid* grid, const lgs_hit_batch* scans, double 
                                                                       w.counters.p);
         LGS_LAUNCH_CHECK(c);
         stamp();
-        // fold on its own stream: it only has to follow this chunk's touch pass and the previous fold
+        // fold on its own stream: it only has to follow this round's touch pass and the previous fold
         LGS_CUDA(c, cudaEventRecord(w.evTouch[buf], c->stream));
         cudaStream_t fs = overlap ? w.foldStream : c->stream;
         if (overlap) LGS_CUDA(c, cudaStreamWaitEvent(fs, w.evTouch[buf], 0));
         FoldArgs a{w.rel.p, w.tileInfo[buf].p, w.pairs[buf].p, w.records[buf].p, w.side[buf].p,
                    diag ? w.counters.p : nullptr, pHit, pMiss, oddsHit, oddsMiss};
-        integ_fold_kernel<<<(unsigned)nTiles, kTileCells, 0, fs>>>(a, g, x0, y0, tw);
+        if (rd.count == 1) integ_fold_kernel<<<(unsigned)nTiles, kTileCells, 0, fs>>>(a, one);
+        else integ_fold_kernel<<<(unsigned)nTiles, kTileCells, 0, fs>>>(a, table);
         LGS_LAUNCH_CHECK(c);
         LGS_CUDA(c, cudaEventRecord(w.evFold[buf], fs));
         ws.usedBuf[buf] = true;
         lastBuf = buf;
         stamp();
+        return LGS_OK;
+    };
+
+    // Chunks: each map's scans in order, a chunk grows while it stays within 64 scans and the record budget;
+    // chunks without hits are dropped.  Pass p takes chunk p of every map that has one.
+    Round rd{0, 0, 0, 0, 0, 0, 0};
+    std::vector<int> next(scanBase.begin(), scanBase.end() - 1), inRound(nMaps, -1);
+    int nRounds = 0;
+    for (bool more = true; more;) {
+        more = false;
+        for (int i = 0; i < nMaps; ++i) {
+            const int end = scanBase[i + 1];
+            if (next[i] >= end) continue;
+            more = true;
+            const lgs_grid* grid = grids[i];
+            int x0 = grid->nx, y0 = grid->ny, x1 = -1, y1 = -1, subBeams = 0, subLen = 0, ns = 0;
+            size_t pairBound = 0;
+            while (next[i] + ns < end && ns < kChunk) {
+                const ScanMeta& m = hMeta[next[i] + ns];
+                if (m.n > 0) {
+                    const int lx = std::max(m.sx - m.maxLen, 0), hx = std::min(m.sx + m.maxLen, grid->nx - 1);
+                    const int ly = std::max(m.sy - m.maxLen, 0), hy = std::min(m.sy + m.maxLen, grid->ny - 1);
+                    const size_t pb = (size_t)tileSpan(lx, hx) * tileSpan(ly, hy);
+                    if (ns > 0 && (pairBound + pb) * kTileCells * sizeof(unsigned) > kRecordBudget) break;
+                    pairBound += pb;
+                    x0 = std::min(x0, lx); x1 = std::max(x1, hx);
+                    y0 = std::min(y0, ly); y1 = std::max(y1, hy);
+                    subBeams = std::max(subBeams, m.n);
+                    subLen = std::max(subLen, m.maxLen);
+                }
+                ++ns;
+            }
+            const int cs = next[i];
+            next[i] += ns;
+            if (subBeams == 0 || x1 < x0 || y1 < y0) continue;
+            x0 &= ~(kTile - 1); y0 &= ~(kTile - 1);                   // tile-aligned region origin
+            const int tw = tileSpan(x0, x1), th = tileSpan(y0, y1);
+            const size_t nTiles = (size_t)tw * th;
+            if (nTiles * kChunk >= ((size_t)1 << 31)) return lgs_fail(c, LGS_ERR_INVALID, "integrate: region of %dx%d tiles is too large", tw, th);
+            pairBound = std::min(pairBound, nTiles * ns);
+            if (rd.count > 0 && (inRound[i] == nRounds || (rd.pairBound + pairBound) * kTileCells * sizeof(unsigned) > kRecordBudget ||
+                                 (rd.tiles + nTiles) * kChunk >= ((size_t)1 << 31) || rd.rows + ns > 65535)) {
+                const int rc = launchRound(rd);
+                if (rc != LGS_OK) return rc;
+                rd = Round{(int)regions.size(), 0, 0, 0, 0, 0, 0};
+                ++nRounds;
+            }
+            regions.push_back(Region{GridRef{const_cast<lgs_grid*>(grid)->origin(), grid->nx, grid->ny, grid->pitch,
+                                             grid->min_x, grid->min_y, grid->res},
+                                     x0, y0, tw, (int)rd.tiles, cs, rd.rows});
+            ++rd.count;
+            rd.rows += ns;
+            rd.beams = std::max(rd.beams, subBeams);
+            rd.len = std::max(rd.len, subLen);
+            rd.tiles += nTiles;
+            rd.pairBound += pairBound;
+            inRound[i] = nRounds;
+        }
+    }
+    if (rd.count > 0) {
+        const int rc = launchRound(rd);
+        if (rc != LGS_OK) return rc;
+        ++nRounds;
     }
     tLoop = msSince(tStart);
     // The call is complete when its counters are back AND its last fold is done.  The context stream does
@@ -812,13 +1018,24 @@ int integ_submit(lgs_ctx* c, lgs_grid* grid, const lgs_hit_batch* scans, double 
     w0.pending = true;
     ++ws.calls;
     ++ws.nPending;
-    if (hostTiming && msSince(tStart) > c->opt.integHostTimingMinMs)
-        fprintf(stderr, "[lgs integrate host] %d scans into %dx%d: staged %.3f ms, pre-pass synced %.3f ms, chunks queued "
-                "%.3f ms\n", n, grid->nx, grid->ny, tStage, tPre, tLoop);
+    if (many && perMap)
+        for (int i = 0; i < nMaps; ++i) {
+            unsigned long long u = 0;
+            for (int s = scanBase[i]; s < scanBase[i + 1]; ++s) u += ws.hManyTouches.p[s];
+            perMap[i] = (long long)u;
+        }
+    if (hostTiming && msSince(tStart) > c->opt.integHostTimingMinMs) {
+        if (many)
+            fprintf(stderr, "[lgs integrate host] %d scans into %d maps, %d rounds: staged %.3f ms, pre-pass synced "
+                    "%.3f ms, rounds queued %.3f ms\n", n, nMaps, nRounds, tStage, tPre, tLoop);
+        else
+            fprintf(stderr, "[lgs integrate host] %d scans into %dx%d: staged %.3f ms, pre-pass synced %.3f ms, chunks "
+                    "queued %.3f ms\n", n, grids[0]->nx, grids[0]->ny, tStage, tPre, tLoop);
+    }
     if (timing) {
         LGS_CUDA(c, cudaStreamSynchronize(c->stream));
         float t[4] = {0, 0, 0, 0};
-        for (size_t k = 0; k + 5 <= evs.size(); k += 5)      // 5 stamps per chunk
+        for (size_t k = 0; k + 5 <= evs.size(); k += 5)      // 5 stamps per round
             for (int j = 0; j < 4; ++j) { float ms = 0; cudaEventElapsedTime(&ms, evs[k + j], evs[k + j + 1]); t[j] += ms; }
         fprintf(stderr, "[lgs integrate] %d scans: mark %.3f ms, pairs %.3f ms, touch %.3f ms, fold %.3f ms; computed updates: "
                 "max per cell and call %llu, total %llu of %llu touches\n", n, t[0], t[1], t[2], t[3],
@@ -839,19 +1056,52 @@ int lgs_grid_integrate_scans(lgs_ctx* c, lgs_grid* grid, const lgs_hit_batch* sc
     // calls submitted asynchronously before this one finish first (their counts are dropped)
     while (c->integ && c->integ->nPending > 0) { const int rc = integ_wait(c, nullptr); if (rc != LGS_OK) return rc; }
     if (scans->n_scans == 0) return LGS_OK;
-    const int rc = integ_submit(c, grid, scans, pHit, pMiss);
+    const int rc = integ_submit(c, 1, &grid, scans, pHit, pMiss, false, nullptr);
     if (rc != LGS_OK) return rc;
     return integ_wait(c, nUpdatesOut);
 }
 
 int lgs_grid_integrate_submit(lgs_ctx* c, lgs_grid* grid, const lgs_hit_batch* scans, double pHit, double pMiss) {
     if (!c || !grid || !scans) return LGS_ERR_INVALID;
-    return integ_submit(c, grid, scans, pHit, pMiss);
+    return integ_submit(c, 1, &grid, scans, pHit, pMiss, false, nullptr);
 }
 
 int lgs_grid_integrate_wait(lgs_ctx* c, long long* nUpdatesOut) {
     if (!c) return LGS_ERR_INVALID;
     return integ_wait(c, nUpdatesOut);
+}
+
+int lgs_grid_integrate_many(lgs_ctx* c, int nMaps, lgs_grid* const* grids, const lgs_hit_batch* scans,
+                            double pHit, double pMiss, long long* nUpdates) {
+    if (!c) return LGS_ERR_INVALID;
+    if (nMaps < 0 || (nMaps > 0 && (!grids || !scans)))
+        return lgs_fail(c, LGS_ERR_INVALID, "integrate_many: %d maps, grids %p, scans %p", nMaps, (const void*)grids,
+                        (const void*)scans);
+    if (nUpdates) std::fill(nUpdates, nUpdates + nMaps, 0LL);
+    if (c->integ && c->integ->nPending > 0)
+        return lgs_fail(c, LGS_ERR_INVALID, "integrate_many: an lgs_grid_integrate_submit call is in flight, wait for it first");
+    // every argument is checked before anything is staged: a refused call leaves every grid as it was
+    for (int i = 0; i < nMaps; ++i) {
+        const lgs_grid* g = grids[i];
+        const lgs_hit_batch& b = scans[i];
+        if (!g) return lgs_fail(c, LGS_ERR_INVALID, "integrate_many: grid %d is NULL", i);
+        if (g->off_x || g->off_y)
+            return lgs_fail(c, LGS_ERR_INVALID, "integrate_many: grid %d is windowed (lgs_grid_set_window), not supported", i);
+        if (g->ctx->device != c->device)
+            return lgs_fail(c, LGS_ERR_INVALID, "integrate_many: grid %d lives on device %d, the context on %d", i,
+                            g->ctx->device, c->device);
+        if (b.n_scans < 0 || (b.n_scans > 0 && (!b.sensor_xy || !b.hit_begin)))
+            return lgs_fail(c, LGS_ERR_INVALID, "integrate_many: bad scan batch of map %d", i);
+        if (b.n_scans > 0 && b.hit_begin[b.n_scans] > 0 && !b.hit_xy)
+            return lgs_fail(c, LGS_ERR_INVALID, "integrate_many: hit_xy of map %d is NULL", i);
+    }
+    std::vector<const lgs_grid*> sorted(grids, grids + nMaps);
+    std::sort(sorted.begin(), sorted.end());
+    if (std::adjacent_find(sorted.begin(), sorted.end()) != sorted.end())
+        return lgs_fail(c, LGS_ERR_INVALID, "integrate_many: the same grid appears twice");
+    const int rc = integ_submit(c, nMaps, grids, scans, pHit, pMiss, true, nUpdates);
+    if (rc != LGS_OK) return rc;
+    return integ_wait(c, nullptr);
 }
 
 long long lgs_ctx_integrate_fallback_cells(const lgs_ctx* c) { return (c && c->integ) ? c->integ->fallbackCells : 0; }

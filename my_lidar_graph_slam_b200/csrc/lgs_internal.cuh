@@ -128,9 +128,15 @@ struct lgs_integ_ws {
     size_t cleanTiles = 0;                   // kmin / kmax are in their reset state up to here
     bool dirty = false;                      // a call failed between the mark and the pair pass
     long long fallbackCells = 0;
+    // lgs_grid_integrate_many only (synchronous): grid table + per-scan map index, per-scan update counts,
+    // the regions of every round
+    DevBuf<char> manyTab, manyRegions;
+    DevBuf<unsigned long long> manyTouches;
+    PinBuf<unsigned long long> hManyTouches;
     void release() {
         stage[0].release(); stage[1].release();
         kmin.release(); kmax.release();
+        manyTab.release(); manyRegions.release(); manyTouches.release(); hManyTouches.release();
         for (int b = 0; b < 2; ++b) {
             tileInfo[b].release(); pairs[b].release(); records[b].release(); side[b].release();
             if (evTouch[b]) cudaEventDestroy(evTouch[b]);

@@ -55,16 +55,14 @@ winmax_x_kernel(const double* __restrict__ in, double* __restrict__ out, int nx,
 // store is coalesced and CELLS * 4 independent loads are in flight per thread.  The output level is
 // larger than L2 on big maps and is next read by a later launch: streaming stores.
 template <int CELLS>
-__global__ void __launch_bounds__(256)
-winmax_double_kernel(const double* __restrict__ in, double* __restrict__ out, int nx, int ny,
-                     int pitch, int w) {
-    const int y = blockIdx.y;
+__device__ __forceinline__ void winmaxDoubleRow(const double* __restrict__ in, double* __restrict__ out, int nx,
+                                                int ny, int pitch, int w, int y, int xBlock) {
     int y0, y1;
     if (ny >= 2 * w) { y0 = min(y, ny - 2 * w); y1 = y0 + w; } else { y0 = 0; y1 = ny - 1; }
     const double* r0 = in + (size_t)y0 * pitch;
     const double* r1 = in + (size_t)y1 * pitch;
     double* o = out + (size_t)y * pitch;
-    const int xb = blockIdx.x * (CELLS * 256) + threadIdx.x;
+    const int xb = xBlock * (CELLS * 256) + threadIdx.x;
     double m[CELLS];
 #pragma unroll
     for (int k = 0; k < CELLS; ++k) {
@@ -80,15 +78,21 @@ winmax_double_kernel(const double* __restrict__ in, double* __restrict__ out, in
     }
 }
 
+template <int CELLS>
+__global__ void __launch_bounds__(256)
+winmax_double_kernel(const double* __restrict__ in, double* __restrict__ out, int nx, int ny,
+                     int pitch, int w) {
+    winmaxDoubleRow<CELLS>(in, out, nx, ny, pitch, w, blockIdx.y, blockIdx.x);
+}
+
 // Zero the apron of every level of a pyramid slab (the interior is fully written by the level
 // kernels, so clearing the whole slab would double the write traffic of a build).
-__global__ void __launch_bounds__(256)
-zero_apron_kernel(double* __restrict__ slab, size_t levelCells, int nLevels, int pitch, int rows, int apron) {
+// Work item r < (H + 1) * per of a slab's apron clear, per = apron cells of one level.
+__device__ __forceinline__ void zeroApronItem(double* __restrict__ slab, size_t levelCells, long long t, int pitch,
+                                              int rows, int apron) {
     const long long band = (long long)apron * pitch;                       // full rows at the bottom / top
     const long long side = (long long)(rows - 2 * apron) * (2 * apron);     // left + right columns
     const long long per = 2 * band + side;
-    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= per * nLevels) return;
     const int lvl = (int)(t / per);
     const long long r = t - (long long)lvl * per;
     size_t cell;
@@ -100,6 +104,64 @@ zero_apron_kernel(double* __restrict__ slab, size_t levelCells, int nLevels, int
         cell = (size_t)row * pitch + (k < apron ? k : pitch - 2 * apron + k);
     }
     slab[levelCells * lvl + cell] = 0.0;
+}
+
+__global__ void __launch_bounds__(256)
+zero_apron_kernel(double* __restrict__ slab, size_t levelCells, int nLevels, int pitch, int rows, int apron) {
+    const long long per = 2LL * apron * pitch + (long long)(rows - 2 * apron) * (2 * apron);
+    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= per * nLevels) return;
+    zeroApronItem(slab, levelCells, t, pitch, rows, apron);
+}
+
+// ---- lgs_pyramid_create_many: every pass is one launch over all pyramids ------------------------------
+// One entry per pyramid; a launch's flat index (thread of the apron clear, block of the row passes) finds
+// its pyramid by the base of its range.
+struct PyrJob {
+    const double* src;        // the grid's cell (0, 0)
+    double* slab;             // level h's cell (0, 0) is at level0 + h * levelCells
+    double* level0;
+    size_t levelCells;
+    int nx, ny, pitch, rows, apron, xBlocks;
+    long long apronBase;      // first apron work item
+    long long blockBase;      // first block of the row passes: ny * xBlocks blocks of kPyrCells * 256 cells
+};
+constexpr int kPyrCells = 4;
+
+template <long long PyrJob::*Base>
+__device__ __forceinline__ const PyrJob& findJob(const PyrJob* __restrict__ jobs, int n, long long v) {
+    int lo = 0, hi = n - 1;
+    while (lo < hi) { const int mid = (lo + hi + 1) >> 1; if (jobs[mid].*Base <= v) lo = mid; else hi = mid - 1; }
+    return jobs[lo];
+}
+
+__global__ void __launch_bounds__(256)
+zero_apron_many_kernel(const PyrJob* __restrict__ jobs, int n, long long items) {
+    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= items) return;
+    const PyrJob& j = findJob<&PyrJob::apronBase>(jobs, n, t);
+    zeroApronItem(j.slab, j.levelCells, t - j.apronBase, j.pitch, j.rows, j.apron);
+}
+
+// level 0 = the grid itself (the copy lgs_pyramid_create makes with cudaMemcpy2DAsync)
+__global__ void __launch_bounds__(256)
+pyr_copy_many_kernel(const PyrJob* __restrict__ jobs, int n) {
+    const PyrJob& j = findJob<&PyrJob::blockBase>(jobs, n, blockIdx.x);
+    const long long b = (long long)blockIdx.x - j.blockBase;
+    const int y = (int)(b / j.xBlocks), xb = (int)(b % j.xBlocks) * (kPyrCells * 256) + threadIdx.x;
+    const double* in = j.src + (size_t)y * j.pitch;
+    double* o = j.level0 + (size_t)y * j.pitch;
+#pragma unroll
+    for (int k = 0; k < kPyrCells; ++k)
+        if (xb + k * 256 < j.nx) o[xb + k * 256] = __ldg(in + xb + k * 256);
+}
+
+__global__ void __launch_bounds__(256)
+winmax_double_many_kernel(const PyrJob* __restrict__ jobs, int n, int h) {
+    const PyrJob& j = findJob<&PyrJob::blockBase>(jobs, n, blockIdx.x);
+    const long long b = (long long)blockIdx.x - j.blockBase;
+    winmaxDoubleRow<kPyrCells>(j.level0 + j.levelCells * (h - 1), j.level0 + j.levelCells * h, j.nx, j.ny, j.pitch,
+                               1 << (h - 1), (int)(b / j.xBlocks), (int)(b % j.xBlocks));
 }
 
 bool same_geometry(const lgs_grid* a, const lgs_grid* b) {
@@ -217,6 +279,93 @@ int lgs_pyramid_create(lgs_ctx* c, const lgs_grid* in, int heightMax, lgs_pyrami
         }
     }
     *outp = p;
+    return LGS_OK;
+}
+
+int lgs_pyramid_create_many(lgs_ctx* c, int n, const lgs_grid* const* grids, int heightMax, lgs_pyramid** out) {
+    if (!c) return LGS_ERR_INVALID;
+    if (n < 0 || (n > 0 && (!grids || !out)))
+        return lgs_fail(c, LGS_ERR_INVALID, "pyramid_create_many: %d grids, grids %p, out %p", n, (const void*)grids,
+                        (const void*)out);
+    std::fill(out, out + n, nullptr);
+    if (heightMax < 0 || heightMax > 20) return lgs_fail(c, LGS_ERR_INVALID, "pyramid: height %d", heightMax);
+    for (int i = 0; i < n; ++i) {
+        if (!grids[i]) return lgs_fail(c, LGS_ERR_INVALID, "pyramid_create_many: grid %d is NULL", i);
+        if (grids[i]->ctx->device != c->device)
+            return lgs_fail(c, LGS_ERR_INVALID, "pyramid_create_many: grid %d lives on device %d, the context on %d", i,
+                            grids[i]->ctx->device, c->device);
+    }
+    if (n == 0) return LGS_OK;
+    LGS_CUDA(c, cudaSetDevice(c->device));
+    for (int i = 0; i < n; ++i) LGS_CUDA(c, lgs_grid_acquire(c, grids[i]));   // pending work of other contexts
+    // every pyramid keeps a slab of its own (lgs_pyramid_destroy frees them one by one)
+    std::vector<PyrJob> jobs(n);
+    long long items = 0, blocks = 0;
+    auto release = [&]() {
+        for (int i = 0; i < n; ++i) if (out[i]) { lgs_pyramid_destroy(out[i]); out[i] = nullptr; }
+    };
+    for (int i = 0; i < n; ++i) {
+        const lgs_grid* in = grids[i];
+        lgs_pyramid* p = new lgs_pyramid();
+        p->ctx = c;
+        const size_t levelCells = (size_t)in->pitch * in->rows;
+        const size_t bytes = levelCells * (size_t)(heightMax + 1) * sizeof(double);
+        const cudaError_t me = lgs_alloc_async(c, &p->slab, std::max<size_t>(bytes, 8));
+        if (me != cudaSuccess) {
+            delete p;
+            release();
+            return lgs_fail(c, LGS_ERR_NOMEM, "pyramid_create_many: grid %d: cudaMallocAsync(%zu) -> %s", i, bytes,
+                            cudaGetErrorString(me));
+        }
+        for (int h = 0; h <= heightMax; ++h) {
+            lgs_grid* g = new lgs_grid(*in);
+            g->ctx = c;
+            g->d = p->slab + levelCells * h;
+            g->owns = false;
+            p->levels.push_back(g);
+        }
+        out[i] = p;
+        PyrJob& j = jobs[i];
+        const int xBlocks = (in->nx + kPyrCells * 256 - 1) / (kPyrCells * 256);
+        j = PyrJob{in->origin(), p->slab, p->levels[0]->origin(), levelCells, in->nx, in->ny, in->pitch, in->rows,
+                   in->apron, xBlocks, items, blocks};
+        // the apron of every level, the whole slab when the grid is empty (all of it is apron then)
+        if (in->apron > 0)
+            items += (2LL * in->apron * in->pitch + (long long)(in->rows - 2 * in->apron) * 2 * in->apron) * (heightMax + 1);
+        if (in->nx > 0 && in->ny > 0) blocks += (long long)in->ny * xBlocks;
+    }
+    if (blocks > 0x7fffffffLL) {
+        release();
+        return lgs_fail(c, LGS_ERR_INVALID, "pyramid_create_many: %lld row blocks in one launch", blocks);
+    }
+    PyrJob* dJobs = nullptr;
+    cudaError_t e = lgs_alloc_async(c, &dJobs, (size_t)n * sizeof(PyrJob));
+    if (e != cudaSuccess) {
+        release();
+        return lgs_fail(c, LGS_ERR_NOMEM, "pyramid_create_many: job table -> %s", cudaGetErrorString(e));
+    }
+    // pageable source: the copy has taken it when cudaMemcpyAsync returns
+    e = cudaMemcpyAsync(dJobs, jobs.data(), (size_t)n * sizeof(PyrJob), cudaMemcpyHostToDevice, c->stream);
+    if (e == cudaSuccess && items > 0) {
+        zero_apron_many_kernel<<<(unsigned)((items + 255) / 256), 256, 0, c->stream>>>(dJobs, n, items);
+        c->launches++;
+        e = cudaGetLastError();
+    }
+    if (e == cudaSuccess && blocks > 0) {
+        pyr_copy_many_kernel<<<(unsigned)blocks, 256, 0, c->stream>>>(dJobs, n);
+        c->launches++;
+        e = cudaGetLastError();
+        for (int h = 1; e == cudaSuccess && h <= heightMax; ++h) {
+            winmax_double_many_kernel<<<(unsigned)blocks, 256, 0, c->stream>>>(dJobs, n, h);
+            c->launches++;
+            e = cudaGetLastError();
+        }
+    }
+    cudaFreeAsync(dJobs, c->stream);
+    if (e != cudaSuccess) {
+        release();
+        return lgs_fail(c, LGS_ERR_CUDA, "pyramid_create_many: %s", cudaGetErrorString(e));
+    }
     return LGS_OK;
 }
 
