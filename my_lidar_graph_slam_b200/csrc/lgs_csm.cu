@@ -10,10 +10,10 @@
 //    operation order (IEEE add/mul/div intrinsics, never fused).  Only sin/cos can differ from
 //    glibc by an ulp, which can change floor() only within the edge guard band of a cell edge; such
 //    points are flagged and re-derived on the host with glibc before the result is accepted.
-//  * the sweep (csm_sweep_rows_kernel: lanes = the x offsets of one window row, 4-5 rows per
-//    thread; csm_sweep_kernel: one thread per hypothesis, for small windows) sums the gathered
-//    cells of every hypothesis in beam order in double: the score is bit-identical to the CPU loop
-//    by construction, so no epsilon logic is needed anywhere.
+//  * the sweep (csm_sweep_rows_kernel: lanes = the x offsets of one window row, 4-5 rows of
+//    kThetaGroup theta slices per thread; csm_sweep_kernel: one thread per hypothesis, for small
+//    windows) sums the gathered cells of every hypothesis in beam order in double: the score is
+//    bit-identical to the CPU loop by construction, so no epsilon logic is needed anywhere.
 //  * csm_select_kernel computes each coarse block's fine maximum with first-visit argmax and
 //    then reproduces the CPU's pruned visit sequence: a parallel (score desc, visit asc)
 //    reduction when every coarse score bounds its block, otherwise a sequential replay of
@@ -21,7 +21,8 @@
 //
 // Data layout: projected points are stored per (match, theta) as int32 offsets into the
 // apron-padded grid, clamped so that every out-of-map read lands in the zero apron; the sweep
-// stages one theta's offsets in shared memory and each thread gathers grid[base + off[i]].
+// stages the offsets of its theta slice(s) in shared memory and each thread gathers
+// grid[base + off[i]].
 #include <cfloat>
 #include <cmath>
 
@@ -31,6 +32,8 @@ namespace {
 
 constexpr int kBeamPad = 8;          // kept-beam count is padded to a multiple of this
 constexpr int kFlagCap = 1 << 16;    // initial capacity of the near-edge fix-up list (grown on demand)
+constexpr int kThetaGroup = 2;       // row-mapped sweep: theta slices per thread (profiles/r3_csm_theta_reuse.md)
+constexpr int kRowsUnroll = 4;       // row-mapped sweep: beams per loop iteration
 
 struct CsmDesc {
     double sx, sy, st;       // sensor pose
@@ -201,47 +204,96 @@ csm_sweep_kernel(const CsmDesc* __restrict__ descs, const double* __restrict__ f
     }
 }
 
-// ---- K2b: the sweep, row mapped --------------------------------------------------------------------
+// ---- K2b: the sweep, row mapped and theta grouped ----------------------------------------------------
 // Same arithmetic as csm_sweep_kernel, different ownership: a warp's lanes are the x offsets of ONE
-// window row (25 of 32 lanes for config C2) and a thread owns ROWS consecutive rows.  A 32-lane
-// request then touches the 2-3 cache lines of a single 25-cell row (2.5 L1 wavefronts on average)
-// instead of the 3.8 lines of 1.28 rows of the flattened mapping: ~15 % fewer L1 wavefronts for the
-// same gathers, and the L1 data pipe is what bounds this kernel (profiles/r1_kernels_v2.md).
-template <int UNROLL, int ROWS>
+// window row (25 of 32 lanes for config C2) and a thread owns ROWS consecutive rows of TG consecutive
+// theta slices.  A 32-lane request touches the 2-3 cache lines of a single 25-cell row (2.5 L1
+// wavefronts on average) instead of the 3.8 lines of 1.28 rows of the flattened mapping, and the L1
+// data pipe is what bounds this kernel (profiles/r1_kernels_v2.md).
+//
+// Theta grouping gathers fewer bytes for the same sums.  Slices t and t + 1 differ by one angular step,
+// so a beam usually projects to the same cell in both, or to the cell directly above or below.  The
+// rows a thread gathered for slice t are then exactly the rows slice t + 1 needs, or the same rows
+// shifted by one, and only the missing row is loaded (on C2: 0.67 of the loads at TG = 2, 0.50 at TG = 4).
+// TG = 2 is the fastest measured: larger groups need more accumulator registers and lose more occupancy
+// than they save in loads (profiles/r3_csm_theta_reuse.md).  Each decision compares two staged offsets of
+// the same beam, which every lane of the block shares: the branches never diverge, and an equal address
+// cannot give a different value.
+// The adds stay acc[t][k] += v[k] in beam order, so every score is the one the CPU loop computes.
+//
+// Shared memory holds the group's offsets interleaved [beam][t]: one broadcast load per beam feeds all
+// TG slices.  A slice past the match's nT (last group; matches of one batch can differ in nT) repeats
+// the last valid slice's offsets, so it takes the equal-offset branch, loads nothing and is not stored.
+template <int TG>
+__device__ __forceinline__ void load_theta_group(const int* s, int (&o)[TG]) {
+    if constexpr (TG % 4 == 0) {
+#pragma unroll
+        for (int q = 0; q < TG / 4; ++q) {
+            const int4 v = reinterpret_cast<const int4*>(s)[q];
+            o[4 * q] = v.x; o[4 * q + 1] = v.y; o[4 * q + 2] = v.z; o[4 * q + 3] = v.w;
+        }
+    } else if constexpr (TG == 2) {
+        const int2 v = *reinterpret_cast<const int2*>(s);
+        o[0] = v.x; o[1] = v.y;
+    } else {
+#pragma unroll
+        for (int t = 0; t < TG; ++t) o[t] = s[t];
+    }
+}
+
+template <int UNROLL, int ROWS, int TG>
 __global__ void __launch_bounds__(256)
 csm_sweep_rows_kernel(const CsmDesc* __restrict__ descs, const double* __restrict__ fineGrid,
                       const double* __restrict__ coarseGrid, int pitch, CsmWindow w,
                       const int* __restrict__ offs, double* __restrict__ fineTab,
                       double* __restrict__ coarseTab) {
-    extern __shared__ int sOff[];
+    extern __shared__ int sOff[];   // [beam][TG]
     const CsmDesc d = descs[blockIdx.z];
-    const int t = blockIdx.y;
-    if (t >= d.nT) return;
-    {   // stage this theta's offsets (nKeptPad is a multiple of 4 ints = 16 B)
-        const int4* src = reinterpret_cast<const int4*>(offs + d.offBegin + (long long)t * d.nKeptPad);
-        int4* dst = reinterpret_cast<int4*>(sOff);
-        for (int k = threadIdx.x; k < d.nKeptPad / 4; k += blockDim.x) dst[k] = src[k];
+    const int t0 = blockIdx.y * TG;
+    if (t0 >= d.nT) return;
+    const int nTg = min(TG, d.nT - t0);   // valid slices of this group
+    {   // stage the group's offsets (nKeptPad is a multiple of 4 ints = 16 B)
+        const int n4 = d.nKeptPad / 4;
+        const int* src = offs + d.offBegin + (long long)t0 * d.nKeptPad;
+        for (int k = threadIdx.x; k < TG * n4; k += blockDim.x) {
+            const int t = k / n4, q = k - t * n4;
+            const int4 v = reinterpret_cast<const int4*>(src + (long long)min(t, nTg - 1) * d.nKeptPad)[q];
+            int* dst = sOff + 4 * q * TG + t;
+            dst[0] = v.x; dst[TG] = v.y; dst[2 * TG] = v.z; dst[3 * TG] = v.w;
+        }
     }
     __syncthreads();
     const int n = d.nKeptPad;   // multiple of kBeamPad >= UNROLL
 
     if (blockIdx.x >= (unsigned)w.tilesFine) {
-        // Coarse hypotheses (stride lowRes on the win-max map), one per thread.
+        // Coarse hypotheses (stride lowRes on the win-max map), one per thread, TG slices each.
+        // Only the equal-offset reuse applies: a thread holds a single row.
         const int h = (blockIdx.x - w.tilesFine) * blockDim.x + threadIdx.x;
         if (h >= w.nbx * w.nby) return;
         const int oy = h / w.nbx, ox = h - oy * w.nbx;
         const double* __restrict__ gp =
             coarseGrid + (-w.winY + oy * w.lowRes) * pitch + (-w.winX + ox * w.lowRes);
-        double acc = 0.0;
+        double acc[TG];
+#pragma unroll
+        for (int t = 0; t < TG; ++t) acc[t] = 0.0;
 #pragma unroll 1
         for (int i = 0; i < n; i += UNROLL) {
-            double v[UNROLL];
 #pragma unroll
-            for (int u = 0; u < UNROLL; ++u) v[u] = __ldg(gp + sOff[i + u]);
+            for (int u = 0; u < UNROLL; ++u) {
+                int o[TG];
+                load_theta_group<TG>(sOff + (i + u) * TG, o);
+                double v = __ldg(gp + o[0]);
+                acc[0] = __dadd_rn(acc[0], v);
 #pragma unroll
-            for (int u = 0; u < UNROLL; ++u) acc = __dadd_rn(acc, v[u]);
+                for (int t = 1; t < TG; ++t) {
+                    if (o[t] != o[t - 1]) v = __ldg(gp + o[t]);
+                    acc[t] = __dadd_rn(acc[t], v);
+                }
+            }
         }
-        coarseTab[d.coarseBegin + ((long long)t * w.nbx + ox) * w.nby + oy] = acc;
+#pragma unroll
+        for (int t = 0; t < TG; ++t)
+            if (t < nTg) coarseTab[d.coarseBegin + ((long long)(t0 + t) * w.nbx + ox) * w.nby + oy] = acc[t];
         return;
     }
 
@@ -251,37 +303,67 @@ csm_sweep_rows_kernel(const CsmDesc* __restrict__ descs, const double* __restric
     if (rg >= w.rowGroups || ox >= w.nxw) return;
     const int oy0 = rg * ROWS;
     const double* __restrict__ gp = fineGrid + (-w.winY + oy0) * pitch + (-w.winX + ox);
-    double acc[ROWS];
+    double acc[TG][ROWS];
 #pragma unroll
-    for (int k = 0; k < ROWS; ++k) acc[k] = 0.0;
+    for (int t = 0; t < TG; ++t)
+#pragma unroll
+        for (int k = 0; k < ROWS; ++k) acc[t][k] = 0.0;
     const int nRows = min(ROWS, w.nyw - oy0);
     if (nRows == ROWS) {
+        // the thread's ROWS window rows; row k of slice t is row[k] + o[t]
+        const double* __restrict__ row[ROWS];
+#pragma unroll
+        for (int k = 0; k < ROWS; ++k) row[k] = gp + k * pitch;
 #pragma unroll 1
         for (int i = 0; i < n; i += UNROLL) {
-            double v[UNROLL][ROWS];
 #pragma unroll
             for (int u = 0; u < UNROLL; ++u) {
-                const double* __restrict__ q = gp + sOff[i + u];
+                int o[TG];
+                load_theta_group<TG>(sOff + (i + u) * TG, o);
+                double v[ROWS];   // rows o[t] + k * pitch, k < ROWS, of the current slice
 #pragma unroll
-                for (int k = 0; k < ROWS; ++k) v[u][k] = __ldg(q + k * pitch);
+                for (int k = 0; k < ROWS; ++k) v[k] = __ldg(row[k] + o[0]);
+#pragma unroll
+                for (int k = 0; k < ROWS; ++k) acc[0][k] = __dadd_rn(acc[0][k], v[k]);   // beam order, like the CPU
+#pragma unroll
+                for (int t = 1; t < TG; ++t) {
+                    if (o[t] == o[t - 1]) {
+                        // same cell: all ROWS rows are already held
+                    } else if (o[t] == o[t - 1] + pitch) {        // one row up the map: shift, load the top row
+#pragma unroll
+                        for (int k = 0; k < ROWS - 1; ++k) v[k] = v[k + 1];
+                        v[ROWS - 1] = __ldg(row[ROWS - 1] + o[t]);
+                    } else if (o[t] == o[t - 1] - pitch) {        // one row down: shift, load the bottom row
+#pragma unroll
+                        for (int k = ROWS - 1; k > 0; --k) v[k] = v[k - 1];
+                        v[0] = __ldg(row[0] + o[t]);
+                    } else {
+#pragma unroll
+                        for (int k = 0; k < ROWS; ++k) v[k] = __ldg(row[k] + o[t]);
+                    }
+#pragma unroll
+                    for (int k = 0; k < ROWS; ++k) acc[t][k] = __dadd_rn(acc[t][k], v[k]);
+                }
             }
-#pragma unroll
-            for (int u = 0; u < UNROLL; ++u)
-#pragma unroll
-                for (int k = 0; k < ROWS; ++k) acc[k] = __dadd_rn(acc[k], v[u][k]);   // beam order, like the CPU
         }
     } else {                                   // last row group of a window whose height is no multiple of ROWS
 #pragma unroll 1
         for (int i = 0; i < n; ++i) {
-            const double* __restrict__ q = gp + sOff[i];
 #pragma unroll
-            for (int k = 0; k < ROWS; ++k)
-                if (k < nRows) acc[k] = __dadd_rn(acc[k], __ldg(q + k * pitch));
+            for (int t = 0; t < TG; ++t) {
+                const double* __restrict__ q = gp + sOff[i * TG + t];
+#pragma unroll
+                for (int k = 0; k < ROWS; ++k)
+                    if (k < nRows) acc[t][k] = __dadd_rn(acc[t][k], __ldg(q + k * pitch));
+            }
         }
     }
 #pragma unroll
-    for (int k = 0; k < ROWS; ++k)
-        if (k < nRows) fineTab[d.fineBegin + ((long long)t * w.nyw + oy0 + k) * w.nxw + ox] = acc[k];
+    for (int t = 0; t < TG; ++t)
+#pragma unroll
+        for (int k = 0; k < ROWS; ++k)
+            if (t < nTg && k < nRows)
+                fineTab[d.fineBegin + ((long long)(t0 + t) * w.nyw + oy0 + k) * w.nxw + ox] = acc[t][k];
 }
 
 // ---- K3: block maxima + CPU-order selection -----------------------------------------------------
@@ -412,6 +494,7 @@ struct lgs_rtcsm_batch {
     lgs_rtcsm_params params{};
     int nMatch = 0;
     int maxNT = 0, maxKeptPad = 0;
+    size_t sweepSmem = 0;                        // dynamic shared memory of the sweep launch
     CsmWindow win{};
     GridGeom geom{};
     std::vector<CsmDesc> descs;
@@ -443,14 +526,16 @@ static int csm_launch_sweep(lgs_rtcsm_batch* b, const lgs_grid* grid, const lgs_
     const CsmWindow& w = b->win;
     for (int m0 = 0; m0 < b->nMatch; m0 += 65535) {
         const int nm = std::min(65535, b->nMatch - m0);
-        dim3 gridDim(w.tilesFine + w.tilesCoarse, b->maxNT, nm);
-        const size_t smem = (size_t)b->maxKeptPad * sizeof(int);
+        // the row-mapped sweep takes kThetaGroup slices per block row
+        const int tiles = w.rows ? (b->maxNT + kThetaGroup - 1) / kThetaGroup : b->maxNT;
+        dim3 gridDim(w.tilesFine + w.tilesCoarse, tiles, nm);
+        const size_t smem = b->sweepSmem;
         if (w.rows == 5)
-            csm_sweep_rows_kernel<4, 5><<<gridDim, w.block, smem, c->stream>>>(
+            csm_sweep_rows_kernel<kRowsUnroll, 5, kThetaGroup><<<gridDim, w.block, smem, c->stream>>>(
                 b->dDescs.p + m0, grid->origin(), coarse->origin(), grid->pitch, w, b->dOffs.p,
                 b->dFine.p, b->dCoarse.p);
         else if (w.rows == 4)
-            csm_sweep_rows_kernel<4, 4><<<gridDim, w.block, smem, c->stream>>>(
+            csm_sweep_rows_kernel<kRowsUnroll, 4, kThetaGroup><<<gridDim, w.block, smem, c->stream>>>(
                 b->dDescs.p + m0, grid->origin(), coarse->origin(), grid->pitch, w, b->dOffs.p,
                 b->dFine.p, b->dCoarse.p);
         else if (w.hpt == 4)
@@ -606,7 +691,9 @@ int lgs_rtcsm_batch_upload(lgs_rtcsm_batch* b, const lgs_grid* grid, const lgs_s
     }
     if (b->maxNT > 65535)
         return lgs_fail(c, LGS_ERR_INVALID, "rtcsm: %d theta slices exceed the launch grid", b->maxNT);
-    if ((size_t)b->maxKeptPad * sizeof(int) > 200 * 1024)
+    // the row-mapped sweep stages the offsets of kThetaGroup slices, the flattened one of one slice
+    b->sweepSmem = (size_t)(w.rows ? kThetaGroup : 1) * b->maxKeptPad * sizeof(int);
+    if (b->sweepSmem > 200 * 1024)
         return lgs_fail(c, LGS_ERR_INVALID, "rtcsm: %d beams exceed shared memory", b->maxKeptPad);
     b->nOff = nOff; b->nCell = nCell; b->nFine = nFine; b->nCoarse = nCoarse;
     if (n == 0) { b->uploaded = true; return LGS_OK; }
@@ -640,20 +727,20 @@ int lgs_rtcsm_batch_upload(lgs_rtcsm_batch* b, const lgs_grid* grid, const lgs_s
         LGS_CUDA(c, cudaMemcpyAsync(b->dRanges.p, b->hStage.p + nk, nk * sizeof(double),
                                     cudaMemcpyHostToDevice, c->stream));
     }
-    if ((size_t)b->maxKeptPad * sizeof(int) > 48 * 1024)
+    if (b->sweepSmem > 48 * 1024)
     {
-        LGS_CUDA(c, cudaFuncSetAttribute(csm_sweep_kernel<kBeamPad, 1>,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         b->maxKeptPad * (int)sizeof(int)));
-        LGS_CUDA(c, cudaFuncSetAttribute(csm_sweep_kernel<4, 4>,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         b->maxKeptPad * (int)sizeof(int)));
-        LGS_CUDA(c, cudaFuncSetAttribute(csm_sweep_rows_kernel<4, 5>,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         b->maxKeptPad * (int)sizeof(int)));
-        LGS_CUDA(c, cudaFuncSetAttribute(csm_sweep_rows_kernel<4, 4>,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         b->maxKeptPad * (int)sizeof(int)));
+        const int smem = (int)b->sweepSmem;
+        if (w.rows) {
+            LGS_CUDA(c, cudaFuncSetAttribute(csm_sweep_rows_kernel<kRowsUnroll, 5, kThetaGroup>,
+                                             cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+            LGS_CUDA(c, cudaFuncSetAttribute(csm_sweep_rows_kernel<kRowsUnroll, 4, kThetaGroup>,
+                                             cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+        } else {
+            LGS_CUDA(c, cudaFuncSetAttribute(csm_sweep_kernel<kBeamPad, 1>,
+                                             cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+            LGS_CUDA(c, cudaFuncSetAttribute(csm_sweep_kernel<4, 4>,
+                                             cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+        }
     }
     b->uploaded = true;
     return LGS_OK;
