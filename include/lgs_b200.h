@@ -150,7 +150,9 @@ int lgs_grid_clear(lgs_grid* g);                             /* GridMap::Reset *
  * beam order, exactly as ComputeBoundingBoxAndScanPoints / ConstructMapFromScans produce them
  * (grid_map_builder.cpp:335-380, :240-277).  Scans are applied in order; every touched cell
  * must already be inside the grid (expand first).  n_updates (optional) receives the number of
- * BinaryBayesGridCell::Update calls the CPU would have made. */
+ * BinaryBayesGridCell::Update calls the CPU would have made.  The one-map calls (integrate_scans,
+ * _submit) are lgs_grid_integrate_many's code with one map; they refuse (LGS_ERR_INVALID) a windowed
+ * grid and a grid on another device, and a call without scans returns LGS_OK before any grid check. */
 typedef struct lgs_hit_batch {
     int n_scans;
     const double* sensor_xy;    /* [n_scans][2]           */
@@ -209,14 +211,16 @@ int lgs_geometry_expand(const lgs_geometry* cur, double min_x, double min_y, dou
  * out(x,y) = max grid[xs..xs+w) x [ys..ys+w), xs = min(x, max(nx-w, 0)) (the reference repeats
  * the last full window at the upper edges).  `out` must have the geometry of `in`. */
 int lgs_precompute(lgs_ctx* ctx, const lgs_grid* in, int win, lgs_grid* out);
-/* Levels 0..height_max with windows 1, 2, ..., 2^height_max (PrecomputeGridMaps). */
+/* Levels 0..height_max with windows 1, 2, ..., 2^height_max (PrecomputeGridMaps):
+ * lgs_pyramid_create_many with one grid. */
 int lgs_pyramid_create(lgs_ctx* ctx, const lgs_grid* in, int height_max, lgs_pyramid** out);
 /* The pyramids of n grids at once: out[i] is an ordinary pyramid of grids[i] (its own slab, freed by
- * lgs_pyramid_destroy), level by level identical to lgs_pyramid_create's.  The apron clear, the level-0
- * copy and each doubling level are one launch over all grids, so the launch count depends on height_max
- * only.  The loop detector's pyramid cache, refilled after every loop closure, is the intended caller.
- * Grids may belong to other contexts of the same device.  If an allocation fails, everything made so
- * far is released, out[] is all NULL and the call returns LGS_ERR_NOMEM. */
+ * lgs_pyramid_destroy), level by level identical to a build of grids[i] alone.  The apron clear, the
+ * level-0 copy and each doubling level are one launch over all grids, so the launch count (height_max + 2)
+ * does not depend on n.  The loop detector's pyramid cache, refilled after every loop closure, is the
+ * intended caller.  Grids may belong to other contexts of the same device; a grid on another device is
+ * refused (LGS_ERR_INVALID).  If an allocation fails, everything made so far is released, out[] is all
+ * NULL and the call returns LGS_ERR_NOMEM. */
 int lgs_pyramid_create_many(lgs_ctx* ctx, int n, const lgs_grid* const* grids, int height_max,
                             lgs_pyramid** out);
 int lgs_pyramid_destroy(lgs_pyramid* p);

@@ -65,17 +65,7 @@ struct GridRef {
     double minX, minY, res;
 };
 
-// Grid of each scan in the pre-pass: one grid for the one-map entry points, a per-scan map index into a
-// device table of grids for lgs_grid_integrate_many.
-struct OneGrid {
-    GridRef g;
-    __device__ __forceinline__ GridRef of(int) const { return g; }
-};
-struct GridTable {
-    const GridRef* __restrict__ g;
-    const int* __restrict__ mapOf;
-    __device__ __forceinline__ GridRef of(int s) const { return g[mapOf[s]]; }
-};
+GridRef gridRef(lgs_grid* g) { return GridRef{g->origin(), g->nx, g->ny, g->pitch, g->min_x, g->min_y, g->res}; }
 
 // A chunk's tile region (x0, y0, tw) inside a ROUND, the set of chunks -- of different maps -- that one
 // launch of each pass covers: the round's regions share one tile index space and one mark-pass grid.
@@ -87,7 +77,7 @@ struct Region {
     int rowBase;         // first mark-pass row (blockIdx.y) of the chunk
 };
 
-// Region source of a round with one chunk (every round of the one-map entry points): nothing to look up.
+// Region source of a round with one chunk (every round of a one-map call): nothing to look up.
 struct OneRegion {
     Region r;            // tileBase == rowBase == 0
     __device__ __forceinline__ Region byTile(int) const { return r; }
@@ -158,12 +148,13 @@ __device__ __forceinline__ int minorAt(int amin, int amaj, int k) {
 }
 
 // ---- pre-pass A: sensor cells ---------------------------------------------------------------------
-template <class Grids>
+// Scan s belongs to grids[mapOf[s]].
 __global__ void integ_sensor_kernel(const double* __restrict__ sensorXY, const int* __restrict__ hitBegin,
-                                    int nScans, Grids grids, ScanMeta* __restrict__ meta) {
+                                    int nScans, const GridRef* __restrict__ grids, const int* __restrict__ mapOf,
+                                    ScanMeta* __restrict__ meta) {
     const int s = blockIdx.x * blockDim.x + threadIdx.x;
     if (s >= nScans) return;
-    const GridRef g = grids.of(s);
+    const GridRef g = grids[mapOf[s]];
     ScanMeta m;
     // WorldCoordinateToGridCellIndex (grid_map.hpp:779-790)
     m.sx = __double2int_rd(__ddiv_rn(__dsub_rn(sensorXY[2 * s], g.minX), g.res));
@@ -177,11 +168,11 @@ __global__ void integ_sensor_kernel(const double* __restrict__ sensorXY, const i
 
 // ---- pre-pass B: per beam end cell relative to the sensor cell ---------------------------------------
 // touches (NULL = not wanted): per scan, the Update calls of the CPU, one per cell of each ray.
-template <class Grids>
-__global__ void integ_beam_kernel(const double* __restrict__ hitXY, Grids grids, ScanMeta* __restrict__ meta,
+__global__ void integ_beam_kernel(const double* __restrict__ hitXY, const GridRef* __restrict__ grids,
+                                  const int* __restrict__ mapOf, ScanMeta* __restrict__ meta,
                                   int2* __restrict__ rel, unsigned long long* __restrict__ touches) {
     const int s = blockIdx.y;
-    const GridRef g = grids.of(s);
+    const GridRef g = grids[mapOf[s]];
     const int n = meta[s].n, beamBegin = meta[s].beamBegin, sx = meta[s].sx, sy = meta[s].sy;
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     int len = 0;
@@ -664,23 +655,27 @@ int integ_wait(lgs_ctx* c, long long* nUpdatesOut) {
     return LGS_OK;
 }
 
+// The checks of one (grid, scan batch) pair of a call; map = its index in the call.
+int integ_check(lgs_ctx* c, int map, const lgs_grid* g, const lgs_hit_batch* b) {
+    if (!g) return lgs_fail(c, LGS_ERR_INVALID, "integrate: grid of map %d is NULL", map);
+    if (b->n_scans < 0 || (b->n_scans > 0 && (!b->sensor_xy || !b->hit_begin)))
+        return lgs_fail(c, LGS_ERR_INVALID, "integrate: bad scan batch of map %d", map);
+    if (b->n_scans > 0 && b->hit_begin[b->n_scans] > 0 && !b->hit_xy)
+        return lgs_fail(c, LGS_ERR_INVALID, "integrate: hit_xy of map %d is NULL", map);
+    if (g->off_x || g->off_y)
+        return lgs_fail(c, LGS_ERR_INVALID, "integrate: grid of map %d is windowed (lgs_grid_set_window), not supported", map);
+    if (g->ctx->device != c->device)
+        return lgs_fail(c, LGS_ERR_INVALID, "integrate: grid of map %d lives on device %d, the context on %d", map,
+                        g->ctx->device, c->device);
+    return LGS_OK;
+}
+
 // Everything of a call up to the last enqueue; the host waits only for the pre-pass (scan bounds).
-// A call integrates batches[i] into grids[i], i < nMaps.  The one-map entry points pass one map; `many`
-// (lgs_grid_integrate_many, arguments checked by the caller) stages every map into one blob behind a
-// device table of grids, returns each map's update count in perMap, and packs the next chunk of every
-// map into one round of launches.
+// A call integrates batches[i] into grids[i], i < nMaps (checked by the caller): every map is staged into
+// one blob behind a device table of grids, and the next chunk of every map goes into one round of
+// launches.  perMap (NULL = not wanted) receives each map's update count.
 int integ_submit(lgs_ctx* c, int nMaps, lgs_grid* const* grids, const lgs_hit_batch* batches, double pHit,
-                 double pMiss, bool many, long long* perMap) {
-    if (!many) {
-        const lgs_hit_batch* scans = batches;
-        const int n = scans->n_scans;
-        if (n < 0 || (n > 0 && (!scans->sensor_xy || !scans->hit_begin)))
-            return lgs_fail(c, LGS_ERR_INVALID, "integrate: bad scan batch");
-        if (n == 0) return LGS_OK;                   // nothing in flight: the matching wait reports 0 updates
-        if (grids[0]->off_x || grids[0]->off_y)
-            return lgs_fail(c, LGS_ERR_INVALID, "integrate: windowed grids (lgs_grid_set_window) are not supported");
-        if (scans->hit_begin[n] > 0 && !scans->hit_xy) return lgs_fail(c, LGS_ERR_INVALID, "integrate: hit_xy is NULL");
-    }
+                 double pMiss, long long* perMap) {
     // scans of map i are scans [scanBase[i], scanBase[i + 1]) of the call, their hits start at hitBase[i]
     std::vector<int> scanBase(nMaps + 1, 0);
     std::vector<long long> hitBase(nMaps + 1, 0);
@@ -706,13 +701,13 @@ int integ_submit(lgs_ctx* c, int nMaps, lgs_grid* const* grids, const lgs_hit_ba
     }
     // `w` = the shared workspace with this call's staging set in front of it
     struct View {
-        DevBuf<double>& sensor; DevBuf<double>& hit; DevBuf<int>& begin; DevBuf<char>& meta; DevBuf<int2>& rel;
+        DevBuf<double>& sensor; DevBuf<double>& hit; DevBuf<char>& tab; DevBuf<char>& meta; DevBuf<int2>& rel;
         DevBuf<unsigned long long>& counters; PinBuf<char>& hMeta; PinBuf<unsigned long long>& hCounters;
         DevBuf<unsigned>& kmin; DevBuf<unsigned>& kmax;
         DevBuf<uint2>* tileInfo; DevBuf<int4>* pairs; DevBuf<unsigned>* records; DevBuf<unsigned>* side;
         cudaStream_t& foldStream; cudaEvent_t* evTouch; cudaEvent_t* evFold;
         size_t& cleanTiles; bool& dirty;
-    } w{w0.sensor, w0.hit, w0.begin, w0.meta, w0.rel, w0.counters, w0.hMeta, w0.hCounters, ws.kmin, ws.kmax,
+    } w{w0.sensor, w0.hit, w0.tab, w0.meta, w0.rel, w0.counters, w0.hMeta, w0.hCounters, ws.kmin, ws.kmax,
         ws.tileInfo, ws.pairs, ws.records, ws.side, ws.foldStream, ws.evTouch, ws.evFold, ws.cleanTiles, ws.dirty};
     cudaStream_t cs0 = ws.copyStream;
     // LGS_INTEG_HOSTTIMING=1 (diagnostic): host wall time of the call's phases to stderr when a call
@@ -724,61 +719,51 @@ int integ_submit(lgs_ctx* c, int nMaps, lgs_grid* const* grids, const lgs_hit_ba
     double tStage = 0.0, tPre = 0.0, tLoop = 0.0;
 
     // Stage the whole batch once, on the copy stream (under the chunks of an earlier call that is still
-    // running); the passes then run over chunks of <= 64 scans (one mask bit each).
+    // running); the passes then run over chunks of <= 64 scans (one mask bit each).  The pre-pass finds the
+    // grid of scan s as grids[mapOf[s]]: the grid table, the hit offsets rebased into the blob and mapOf
+    // go in one copy (pageable host vector: the copy has taken it when cudaMemcpyAsync returns).
+    const size_t tabBytes = (size_t)nMaps * sizeof(GridRef) + (size_t)(2 * n + 1) * sizeof(int);
     LGS_CUDA(c, w.sensor.reserve((size_t)n * 2));
     LGS_CUDA(c, w.hit.reserve(std::max<size_t>((size_t)total, 1) * 2));
-    LGS_CUDA(c, w.begin.reserve((size_t)n + 1));
+    LGS_CUDA(c, w.tab.reserve(tabBytes));
     LGS_CUDA(c, w.meta.reserve((size_t)n * sizeof(ScanMeta)));
     LGS_CUDA(c, w.rel.reserve(std::max<size_t>((size_t)total, 1)));
     LGS_CUDA(c, w.counters.reserve(8));
     LGS_CUDA(c, w.hMeta.reserve((size_t)n * sizeof(ScanMeta)));
     LGS_CUDA(c, w.hCounters.reserve(8));
-    // lgs_grid_integrate_many: hit offsets rebased into the blob, per-scan map index, grid table (pageable
-    // host vectors: the copies have taken them when cudaMemcpyAsync returns)
-    std::vector<int> hBegin;
-    std::vector<char> hTab;
-    const GridRef* dGrids = nullptr;
-    const int* dMapOf = nullptr;
+    std::vector<char> hTab(tabBytes);
+    GridRef* tg = reinterpret_cast<GridRef*>(hTab.data());
+    int* hBegin = reinterpret_cast<int*>(tg + nMaps);
+    int* hMapOf = hBegin + n + 1;
+    for (int i = 0; i < nMaps; ++i) {
+        tg[i] = gridRef(grids[i]);
+        for (int s = 0; s < batches[i].n_scans; ++s) {
+            hBegin[scanBase[i] + s] = (int)(hitBase[i] + batches[i].hit_begin[s]);
+            hMapOf[scanBase[i] + s] = i;
+        }
+    }
+    hBegin[n] = (int)total;
+    for (int i = 0; i < nMaps; ++i) {
+        const lgs_hit_batch& b = batches[i];
+        if (b.n_scans == 0) continue;
+        LGS_CUDA(c, cudaMemcpyAsync(w.sensor.p + 2 * (size_t)scanBase[i], b.sensor_xy,
+                                    (size_t)b.n_scans * 2 * sizeof(double), cudaMemcpyHostToDevice, cs0));
+        if (hitBase[i + 1] > hitBase[i])
+            LGS_CUDA(c, cudaMemcpyAsync(w.hit.p + 2 * (size_t)hitBase[i], b.hit_xy,
+                                        (size_t)(hitBase[i + 1] - hitBase[i]) * 2 * sizeof(double),
+                                        cudaMemcpyHostToDevice, cs0));
+    }
+    LGS_CUDA(c, cudaMemcpyAsync(w.tab.p, hTab.data(), tabBytes, cudaMemcpyHostToDevice, cs0));
+    const GridRef* dGrids = reinterpret_cast<const GridRef*>(w.tab.p);
+    const int* dBegin = reinterpret_cast<const int*>(dGrids + nMaps);
+    const int* dMapOf = dBegin + n + 1;
+    // per-scan update counts, only for perMap (the call's total is counters[0] of the touch pass)
     unsigned long long* dTouches = nullptr;
-    if (many) {
-        hBegin.resize((size_t)n + 1);
-        hTab.resize((size_t)nMaps * sizeof(GridRef) + (size_t)n * sizeof(int));
-        GridRef* tg = reinterpret_cast<GridRef*>(hTab.data());
-        int* mapOf = reinterpret_cast<int*>(hTab.data() + (size_t)nMaps * sizeof(GridRef));
-        for (int i = 0; i < nMaps; ++i) {
-            const lgs_grid* gr = grids[i];
-            tg[i] = GridRef{const_cast<lgs_grid*>(gr)->origin(), gr->nx, gr->ny, gr->pitch, gr->min_x, gr->min_y, gr->res};
-            for (int s = 0; s < batches[i].n_scans; ++s) {
-                hBegin[scanBase[i] + s] = (int)(hitBase[i] + batches[i].hit_begin[s]);
-                mapOf[scanBase[i] + s] = i;
-            }
-        }
-        hBegin[n] = (int)total;
-        LGS_CUDA(c, ws.manyTab.reserve(hTab.size()));
-        LGS_CUDA(c, ws.manyTouches.reserve((size_t)n));
-        LGS_CUDA(c, ws.hManyTouches.reserve((size_t)n));
-        dGrids = reinterpret_cast<const GridRef*>(ws.manyTab.p);
-        dMapOf = reinterpret_cast<const int*>(ws.manyTab.p + (size_t)nMaps * sizeof(GridRef));
-        dTouches = ws.manyTouches.p;
-        for (int i = 0; i < nMaps; ++i) {
-            const lgs_hit_batch& b = batches[i];
-            if (b.n_scans == 0) continue;
-            LGS_CUDA(c, cudaMemcpyAsync(w.sensor.p + 2 * (size_t)scanBase[i], b.sensor_xy,
-                                        (size_t)b.n_scans * 2 * sizeof(double), cudaMemcpyHostToDevice, cs0));
-            if (hitBase[i + 1] > hitBase[i])
-                LGS_CUDA(c, cudaMemcpyAsync(w.hit.p + 2 * (size_t)hitBase[i], b.hit_xy,
-                                            (size_t)(hitBase[i + 1] - hitBase[i]) * 2 * sizeof(double),
-                                            cudaMemcpyHostToDevice, cs0));
-        }
-        LGS_CUDA(c, cudaMemcpyAsync(w.begin.p, hBegin.data(), (size_t)(n + 1) * sizeof(int), cudaMemcpyHostToDevice, cs0));
-        LGS_CUDA(c, cudaMemcpyAsync(ws.manyTab.p, hTab.data(), hTab.size(), cudaMemcpyHostToDevice, cs0));
+    if (perMap) {
+        LGS_CUDA(c, ws.touches.reserve((size_t)n));
+        LGS_CUDA(c, ws.hTouches.reserve((size_t)n));
+        dTouches = ws.touches.p;
         LGS_CUDA(c, cudaMemsetAsync(dTouches, 0, (size_t)n * sizeof(unsigned long long), cs0));
-    } else {
-        const lgs_hit_batch* scans = batches;
-        LGS_CUDA(c, cudaMemcpyAsync(w.sensor.p, scans->sensor_xy, (size_t)n * 2 * sizeof(double), cudaMemcpyHostToDevice, cs0));
-        if (total)
-            LGS_CUDA(c, cudaMemcpyAsync(w.hit.p, scans->hit_xy, (size_t)total * 2 * sizeof(double), cudaMemcpyHostToDevice, cs0));
-        LGS_CUDA(c, cudaMemcpyAsync(w.begin.p, scans->hit_begin, (size_t)(n + 1) * sizeof(int), cudaMemcpyHostToDevice, cs0));
     }
     LGS_CUDA(c, cudaMemsetAsync(w.counters.p, 0, 8 * sizeof(unsigned long long), cs0));
     tStage = msSince(tStart);
@@ -790,41 +775,26 @@ int integ_submit(lgs_ctx* c, int nMaps, lgs_grid* const* grids, const lgs_hit_ba
     ScanMeta* dMeta = reinterpret_cast<ScanMeta*>(w.meta.p);
     ScanMeta* hMeta = reinterpret_cast<ScanMeta*>(w.hMeta.p);
     // Pre-pass over the whole batch: sensor cells, relative end cells, ray lengths, bounds check.
-    if (many) {
-        integ_sensor_kernel<<<(n + 127) / 128, 128, 0, cs0>>>(w.sensor.p, w.begin.p, n, GridTable{dGrids, dMapOf}, dMeta);
+    integ_sensor_kernel<<<(n + 127) / 128, 128, 0, cs0>>>(w.sensor.p, dBegin, n, dGrids, dMapOf, dMeta);
+    LGS_LAUNCH_CHECK(c);
+    for (int s0 = 0; maxBeams > 0 && s0 < n; s0 += 65535) {       // grid rows: at most 65535 scans a launch
+        dim3 gb((maxBeams + 127) / 128, std::min(n - s0, 65535));
+        integ_beam_kernel<<<gb, 128, 0, cs0>>>(w.hit.p, dGrids, dMapOf + s0, dMeta + s0, w.rel.p,
+                                               dTouches ? dTouches + s0 : nullptr);
         LGS_LAUNCH_CHECK(c);
-        for (int s0 = 0; maxBeams > 0 && s0 < n; s0 += 65535) {       // grid rows: at most 65535 scans a launch
-            dim3 gb((maxBeams + 127) / 128, std::min(n - s0, 65535));
-            integ_beam_kernel<<<gb, 128, 0, cs0>>>(w.hit.p, GridTable{dGrids, dMapOf + s0}, dMeta + s0, w.rel.p,
-                                                   dTouches + s0);
-            LGS_LAUNCH_CHECK(c);
-        }
-        LGS_CUDA(c, cudaMemcpyAsync(ws.hManyTouches.p, dTouches, (size_t)n * sizeof(unsigned long long),
-                                    cudaMemcpyDeviceToHost, cs0));
-    } else {
-        const lgs_grid* grid = grids[0];
-        const OneGrid g{GridRef{grids[0]->origin(), grid->nx, grid->ny, grid->pitch, grid->min_x, grid->min_y, grid->res}};
-        integ_sensor_kernel<<<(n + 127) / 128, 128, 0, cs0>>>(w.sensor.p, w.begin.p, n, g, dMeta);
-        LGS_LAUNCH_CHECK(c);
-        if (maxBeams > 0) {
-            dim3 gb((maxBeams + 127) / 128, n);
-            integ_beam_kernel<<<gb, 128, 0, cs0>>>(w.hit.p, g, dMeta, w.rel.p, nullptr);
-            LGS_LAUNCH_CHECK(c);
-        }
     }
+    if (dTouches)
+        LGS_CUDA(c, cudaMemcpyAsync(ws.hTouches.p, dTouches, (size_t)n * sizeof(unsigned long long),
+                                    cudaMemcpyDeviceToHost, cs0));
     LGS_CUDA(c, cudaMemcpyAsync(hMeta, dMeta, (size_t)n * sizeof(ScanMeta), cudaMemcpyDeviceToHost, cs0));
     LGS_CUDA(c, cudaStreamSynchronize(cs0));
     tPre = msSince(tStart);
     for (int i = 0; i < nMaps; ++i)
         for (int s = scanBase[i]; s < scanBase[i + 1]; ++s)
-            if (hMeta[s].bad) {
-                if (many)
-                    return lgs_fail(c, LGS_ERR_INVALID, "integrate_many: map %d, scan %d touches cells outside the "
-                                    "%dx%d grid (expand the map first, as GridMap::Expand does)", i, s - scanBase[i],
-                                    grids[i]->nx, grids[i]->ny);
-                return lgs_fail(c, LGS_ERR_INVALID, "integrate: scan %d touches cells outside the %dx%d grid "
-                                "(expand the map first, as GridMap::Expand does)", s, grids[i]->nx, grids[i]->ny);
-            }
+            if (hMeta[s].bad)
+                return lgs_fail(c, LGS_ERR_INVALID, "integrate: map %d, scan %d touches cells outside the %dx%d grid "
+                                "(expand the map first, as GridMap::Expand does)", i, s - scanBase[i],
+                                grids[i]->nx, grids[i]->ny);
 
     // ValueToOdds(prob) for the two observations (binary_bayes_grid_cell.hpp:104-113), host IEEE.
     auto clampP = [](double v) { const double lo = 1e-3, hi = 1.0 - 1e-3; return v < lo ? lo : (hi < v ? hi : v); };
@@ -856,17 +826,19 @@ int integ_submit(lgs_ctx* c, int nMaps, lgs_grid* const* grids, const lgs_hit_ba
     // Rounds: consecutive chunks (below) share one launch of each pass while the round holds at most one chunk
     // per map (the fold owns the map's cells), and its records, tile index space and mark-pass rows stay within
     // the limits of one chunk.  A round is launched as soon as it is closed; one with several chunks takes its
-    // regions from a table at its own place in manyRegions (a one-chunk round needs none).
+    // regions from a table at its own place in ws.regions.  A one-chunk round (every round of a one-map call)
+    // copies no table: that copy would run on the context stream while the fold of a call submitted before
+    // this one may still be reading the table on the fold stream.
     struct Round { int first, count, rows, beams, len; size_t tiles, pairBound; };
     std::vector<Region> regions;
-    if (many) LGS_CUDA(c, ws.manyRegions.reserve((size_t)n * sizeof(Region)));   // a chunk holds >= 1 scan
+    LGS_CUDA(c, ws.regions.reserve((size_t)n * sizeof(Region)));   // a chunk holds >= 1 scan
     int lastBuf = -1;
     auto launchRound = [&](const Round& rd) -> int {
         const size_t nTiles = rd.tiles, pairBound = rd.pairBound;
         const OneRegion one{regions[rd.first]};
         RegionTable table{nullptr, rd.count};
         if (rd.count > 1) {
-            Region* dst = reinterpret_cast<Region*>(ws.manyRegions.p) + rd.first;
+            Region* dst = reinterpret_cast<Region*>(ws.regions.p) + rd.first;
             LGS_CUDA(c, cudaMemcpyAsync(dst, regions.data() + rd.first, (size_t)rd.count * sizeof(Region),
                                         cudaMemcpyHostToDevice, c->stream));
             table.r = dst;
@@ -985,9 +957,7 @@ int integ_submit(lgs_ctx* c, int nMaps, lgs_grid* const* grids, const lgs_hit_ba
                 rd = Round{(int)regions.size(), 0, 0, 0, 0, 0, 0};
                 ++nRounds;
             }
-            regions.push_back(Region{GridRef{const_cast<lgs_grid*>(grid)->origin(), grid->nx, grid->ny, grid->pitch,
-                                             grid->min_x, grid->min_y, grid->res},
-                                     x0, y0, tw, (int)rd.tiles, cs, rd.rows});
+            regions.push_back(Region{gridRef(grids[i]), x0, y0, tw, (int)rd.tiles, cs, rd.rows});
             ++rd.count;
             rd.rows += ns;
             rd.beams = std::max(rd.beams, subBeams);
@@ -1018,20 +988,15 @@ int integ_submit(lgs_ctx* c, int nMaps, lgs_grid* const* grids, const lgs_hit_ba
     w0.pending = true;
     ++ws.calls;
     ++ws.nPending;
-    if (many && perMap)
+    if (perMap)
         for (int i = 0; i < nMaps; ++i) {
             unsigned long long u = 0;
-            for (int s = scanBase[i]; s < scanBase[i + 1]; ++s) u += ws.hManyTouches.p[s];
+            for (int s = scanBase[i]; s < scanBase[i + 1]; ++s) u += ws.hTouches.p[s];
             perMap[i] = (long long)u;
         }
-    if (hostTiming && msSince(tStart) > c->opt.integHostTimingMinMs) {
-        if (many)
-            fprintf(stderr, "[lgs integrate host] %d scans into %d maps, %d rounds: staged %.3f ms, pre-pass synced "
-                    "%.3f ms, rounds queued %.3f ms\n", n, nMaps, nRounds, tStage, tPre, tLoop);
-        else
-            fprintf(stderr, "[lgs integrate host] %d scans into %dx%d: staged %.3f ms, pre-pass synced %.3f ms, chunks "
-                    "queued %.3f ms\n", n, grids[0]->nx, grids[0]->ny, tStage, tPre, tLoop);
-    }
+    if (hostTiming && msSince(tStart) > c->opt.integHostTimingMinMs)
+        fprintf(stderr, "[lgs integrate host] %d scans into %d maps, %d rounds: staged %.3f ms, pre-pass synced "
+                "%.3f ms, rounds queued %.3f ms\n", n, nMaps, nRounds, tStage, tPre, tLoop);
     if (timing) {
         LGS_CUDA(c, cudaStreamSynchronize(c->stream));
         float t[4] = {0, 0, 0, 0};
@@ -1055,15 +1020,17 @@ int lgs_grid_integrate_scans(lgs_ctx* c, lgs_grid* grid, const lgs_hit_batch* sc
     if (nUpdatesOut) *nUpdatesOut = 0;
     // calls submitted asynchronously before this one finish first (their counts are dropped)
     while (c->integ && c->integ->nPending > 0) { const int rc = integ_wait(c, nullptr); if (rc != LGS_OK) return rc; }
-    if (scans->n_scans == 0) return LGS_OK;
-    const int rc = integ_submit(c, 1, &grid, scans, pHit, pMiss, false, nullptr);
+    const int rc = lgs_grid_integrate_submit(c, grid, scans, pHit, pMiss);
     if (rc != LGS_OK) return rc;
     return integ_wait(c, nUpdatesOut);
 }
 
 int lgs_grid_integrate_submit(lgs_ctx* c, lgs_grid* grid, const lgs_hit_batch* scans, double pHit, double pMiss) {
     if (!c || !grid || !scans) return LGS_ERR_INVALID;
-    return integ_submit(c, 1, &grid, scans, pHit, pMiss, false, nullptr);
+    if (scans->n_scans == 0) return LGS_OK;          // nothing in flight: the matching wait reports 0 updates
+    const int rc = integ_check(c, 0, grid, scans);
+    if (rc != LGS_OK) return rc;
+    return integ_submit(c, 1, &grid, scans, pHit, pMiss, nullptr);
 }
 
 int lgs_grid_integrate_wait(lgs_ctx* c, long long* nUpdatesOut) {
@@ -1082,24 +1049,14 @@ int lgs_grid_integrate_many(lgs_ctx* c, int nMaps, lgs_grid* const* grids, const
         return lgs_fail(c, LGS_ERR_INVALID, "integrate_many: an lgs_grid_integrate_submit call is in flight, wait for it first");
     // every argument is checked before anything is staged: a refused call leaves every grid as it was
     for (int i = 0; i < nMaps; ++i) {
-        const lgs_grid* g = grids[i];
-        const lgs_hit_batch& b = scans[i];
-        if (!g) return lgs_fail(c, LGS_ERR_INVALID, "integrate_many: grid %d is NULL", i);
-        if (g->off_x || g->off_y)
-            return lgs_fail(c, LGS_ERR_INVALID, "integrate_many: grid %d is windowed (lgs_grid_set_window), not supported", i);
-        if (g->ctx->device != c->device)
-            return lgs_fail(c, LGS_ERR_INVALID, "integrate_many: grid %d lives on device %d, the context on %d", i,
-                            g->ctx->device, c->device);
-        if (b.n_scans < 0 || (b.n_scans > 0 && (!b.sensor_xy || !b.hit_begin)))
-            return lgs_fail(c, LGS_ERR_INVALID, "integrate_many: bad scan batch of map %d", i);
-        if (b.n_scans > 0 && b.hit_begin[b.n_scans] > 0 && !b.hit_xy)
-            return lgs_fail(c, LGS_ERR_INVALID, "integrate_many: hit_xy of map %d is NULL", i);
+        const int rc = integ_check(c, i, grids[i], &scans[i]);
+        if (rc != LGS_OK) return rc;
     }
     std::vector<const lgs_grid*> sorted(grids, grids + nMaps);
     std::sort(sorted.begin(), sorted.end());
     if (std::adjacent_find(sorted.begin(), sorted.end()) != sorted.end())
         return lgs_fail(c, LGS_ERR_INVALID, "integrate_many: the same grid appears twice");
-    const int rc = integ_submit(c, nMaps, grids, scans, pHit, pMiss, true, nUpdates);
+    const int rc = integ_submit(c, nMaps, grids, scans, pHit, pMiss, nUpdates);
     if (rc != LGS_OK) return rc;
     return integ_wait(c, nullptr);
 }

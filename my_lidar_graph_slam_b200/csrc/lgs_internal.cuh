@@ -94,7 +94,7 @@ struct lgs_integ_ws {
     // still read set k.
     struct Stage {
         DevBuf<double> sensor, hit;
-        DevBuf<int> begin;
+        DevBuf<char> tab;                    // GridRef per map, hit offset per scan (+ end), map index per scan
         DevBuf<char> meta;                   // ScanMeta per scan
         DevBuf<int2> rel;                    // per beam: hit cell - sensor cell
         DevBuf<unsigned long long> counters;
@@ -104,7 +104,7 @@ struct lgs_integ_ws {
         cudaEvent_t evCounters = nullptr;
         bool pending = false;                // submitted, not yet waited for
         void release() {
-            sensor.release(); hit.release(); begin.release(); meta.release(); rel.release();
+            sensor.release(); hit.release(); tab.release(); meta.release(); rel.release();
             counters.release(); hMeta.release(); hCounters.release();
             if (evDone) cudaEventDestroy(evDone);
             if (evCounters) cudaEventDestroy(evCounters);
@@ -128,15 +128,14 @@ struct lgs_integ_ws {
     size_t cleanTiles = 0;                   // kmin / kmax are in their reset state up to here
     bool dirty = false;                      // a call failed between the mark and the pair pass
     long long fallbackCells = 0;
-    // lgs_grid_integrate_many only (synchronous): grid table + per-scan map index, per-scan update counts,
-    // the regions of every round
-    DevBuf<char> manyTab, manyRegions;
-    DevBuf<unsigned long long> manyTouches;
-    PinBuf<unsigned long long> hManyTouches;
+    DevBuf<char> regions;                    // region tables of the rounds with several chunks
+    // per-scan update counts of a call that asks for each map's count (lgs_grid_integrate_many, synchronous)
+    DevBuf<unsigned long long> touches;
+    PinBuf<unsigned long long> hTouches;
     void release() {
         stage[0].release(); stage[1].release();
         kmin.release(); kmax.release();
-        manyTab.release(); manyRegions.release(); manyTouches.release(); hManyTouches.release();
+        regions.release(); touches.release(); hTouches.release();
         for (int b = 0; b < 2; ++b) {
             tileInfo[b].release(); pairs[b].release(); records[b].release(); side[b].release();
             if (evTouch[b]) cudaEventDestroy(evTouch[b]);

@@ -221,6 +221,28 @@ def test_rejections(ctx):
         assert np.array_equal(_bits(a.download()), _bits(b.download()))
 
 
+@pytest.mark.skipif(capi.device_count() < 2, reason="needs a second GPU")
+def test_grids_on_another_device_are_refused(ctx):
+    """The one-map and the batched calls, integration and pyramids alike, refuse a grid of another device."""
+    maps = _random_maps(25, [3])
+    sensors, hits = maps[0]["sensors"], maps[0]["hits"]
+    other = capi.Context(1)
+    try:
+        g = capi.Grid(other, *maps[0]["geo"], apron=1)
+        calls = [lambda: capi.integrate_scans(ctx, g, sensors, hits),
+                 lambda: capi.integrate_submit(ctx, g, capi.PackedHits(sensors, hits)),
+                 lambda: capi.integrate_many(ctx, [g], [sensors], [hits]),
+                 lambda: capi.Pyramid(ctx, g, 3),
+                 lambda: capi.Pyramid.create_many(ctx, [g], 3)]
+        for call in calls:
+            with pytest.raises(capi.LgsError, match="lives on device 1"):
+                call()
+        assert capi.integrate_wait(ctx) == 0
+        assert not g.download().any()
+    finally:
+        other.close()
+
+
 def test_grids_of_another_context(ctx):
     """Grids owned by a second context of the same device (e.g. the builder's), ordered like lgs_grid_copy:
     the owner's pending uploads come first."""
