@@ -105,6 +105,8 @@ int lgs_measure_gather_peak(lgs_ctx* ctx, int nx, int ny, int row_lanes, int ali
  *                       of the persistent kernel's warp mappings
  *   "bb_host_timing", "integ_host_timing", "integ_timing", "integ_diag"   timing reports on stderr
  *   "integ_side_words"  integration side-buffer size in words (tests shrink it)    (LGS_INTEG_SIDE_WORDS)
+ *   "integ_resolve_ulps" lgs_grid_construct_many: half width, in ulps of cos / sin, of the interval around the
+ *                       device's value (default 8; huge values send every hit and every bbox side to the host)
  *   "gs_tables"         grid search through the index tables instead of the fused kernel (LGS_GS_TABLES) */
 int lgs_ctx_set_option(lgs_ctx* ctx, const char* name, double value);
 int lgs_ctx_get_option(const lgs_ctx* ctx, const char* name, double* value);
@@ -198,6 +200,32 @@ typedef struct lgs_geometry {
     double min_x, min_y, res;
     int patch;                  /* cells per patch side       */
 } lgs_geometry;
+
+/* GridMapBuilder::ConstructMapFromScans (grid_map_builder.cpp:227-332) for many maps in one synchronous call,
+ * from raw scans.  Map i: scans[i] holds its nodes' scans in node order, sensor_pose[k] = Compound(node pose,
+ * RelativeSensorPose()), range_min[k] / range_max[k] = max(UsableRangeMin, MinRange()) / min(UsableRangeMax,
+ * MaxRange()) (both arrays required).  A beam is used unless r >= range_max or r <= range_min (:365-366); its hit
+ * is HitPoint's.  The bbox covers every hit and sensor position, from min = DBL_MAX and max = DBL_MIN (:236-237);
+ * the new geometry is lgs_geometry_resize(cur[i], bbox) -- cur[i] is the map's current geometry, whose origin
+ * anchors the patch lattice (a fresh map: 0 x 0 cells at its anchor) -- and grids[i] takes it with every cell
+ * unknown (Resize + Reset) before every hit is integrated as lgs_grid_integrate_many would.  geometry_out[i],
+ * bbox_out[i] = {min_x, min_y, max_x, max_y} (optional) and n_updates[i] (optional) return what was used.
+ * Every cell, geometry and bbox is bit-identical to lgs_scan_hit_points per scan, then the bbox, then
+ * lgs_geometry_resize, then lgs_grid_integrate_many: beams are projected on the device with an interval that
+ * contains glibc's cos / sin ("integ_resolve_ulps"), and the few hits that interval cannot settle -- near a
+ * cell edge, or possibly a bbox extreme -- are re-derived on the host (lgs_ctx_construct_host_points).  The
+ * extra launches do not depend on n_maps.  Intended callers: GridMapBuilderCuda::AfterLoopClosure (every local
+ * map plus the latest map in one call), UpdateLatestMap and ConstructGlobalMap.  Refused (LGS_ERR_INVALID)
+ * before any grid changes: the refusals of lgs_grid_integrate_many, a map without scans, NULL range arrays,
+ * a non-finite sensor pose or range window, and a non-finite angle or range on a beam that is used. */
+struct lgs_scan_batch;          /* defined with the scans below */
+int lgs_grid_construct_many(lgs_ctx* ctx, int n_maps, lgs_grid* const* grids,
+                            const struct lgs_scan_batch* scans, const lgs_geometry* cur,
+                            double p_hit, double p_miss, lgs_geometry* geometry_out,
+                            double* bbox_out, long long* n_updates);
+/* Points lgs_grid_construct_many re-derived on the host (cumulative over this context): bbox candidates
+ * and near-edge hits. */
+int lgs_ctx_construct_host_points(const lgs_ctx* ctx, long long* bbox_points, long long* edge_points);
 int lgs_scan_hit_points(const double* sensor_pose, int n, const double* angles,
                         const double* ranges, double range_min, double range_max,
                         double* hit_xy, int* n_hit, double* bbox);

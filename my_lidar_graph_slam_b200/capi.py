@@ -735,6 +735,10 @@ SIGNATURES.update({
                             [C.POINTER(Geometry), c_ip, c_ip]),
     "lgs_geometry_expand": (C.c_int, [C.POINTER(Geometry)] + [C.c_double] * 5 +
                             [C.POINTER(Geometry), c_ip, c_ip, c_ip]),
+    "lgs_grid_construct_many": (C.c_int, [vp, C.c_int, C.POINTER(vp), C.POINTER(ScanBatch), C.POINTER(Geometry),
+                                          C.c_double, C.c_double, C.POINTER(Geometry), c_dp,
+                                          C.POINTER(C.c_longlong)]),
+    "lgs_ctx_construct_host_points": (C.c_int, [vp, C.POINTER(C.c_longlong), C.POINTER(C.c_longlong)]),
 })
 
 
@@ -849,6 +853,34 @@ def integrate_many(ctx: Context, grids, sensor_xy_list, hits_lists, p_hit=0.6, p
     ctx.check(lib().lgs_grid_integrate_many(ctx.h, n, handles, batches, p_hit, p_miss,
                                             out.ctypes.data_as(C.POINTER(C.c_longlong))))
     return out[:n]
+
+
+def construct_many(ctx: Context, grids, scans_list, cur_geometries, p_hit=0.6, p_miss=0.45):
+    """lgs_grid_construct_many: ConstructMapFromScans of every map from raw scans (scans_list[i], a Scans with
+    range_min / range_max) in one call; grids[i] is resized from cur_geometries[i] and rebuilt.
+    -> (geometries [Geometry], bboxes [n][4] float64, updates [n] int64).  Each Grid's nx / ny / min_x / min_y
+    follow its new geometry."""
+    n = len(grids)
+    assert len(scans_list) == n and len(cur_geometries) == n
+    batches = (ScanBatch * max(n, 1))(*[s.c for s in scans_list])
+    handles = (vp * max(n, 1))(*[g.h for g in grids])
+    cur = (Geometry * max(n, 1))(*cur_geometries)
+    geo = (Geometry * max(n, 1))()
+    bbox = np.zeros((max(n, 1), 4), dtype=np.float64)
+    out = np.zeros(max(n, 1), dtype=np.int64)
+    ctx.check(lib().lgs_grid_construct_many(ctx.h, n, handles, batches, cur, p_hit, p_miss, geo, _dptr(bbox),
+                                            out.ctypes.data_as(C.POINTER(C.c_longlong))))
+    geos = [geo[i] for i in range(n)]
+    for g, r in zip(grids, geos):
+        g.nx, g.ny, g.min_x, g.min_y, g.res = r.nx, r.ny, r.min_x, r.min_y, r.res
+    return geos, bbox[:n], out[:n]
+
+
+def construct_host_points(ctx: Context):
+    """(bbox candidates, near-edge hits) lgs_grid_construct_many re-derived on the host so far."""
+    b, e = C.c_longlong(), C.c_longlong()
+    ctx.check(lib().lgs_ctx_construct_host_points(ctx.h, C.byref(b), C.byref(e)))
+    return b.value, e.value
 
 
 def measure_gather_peak(ctx: Context, nx=960, ny=640, row_lanes=25, aligned=False, local=True) -> float:

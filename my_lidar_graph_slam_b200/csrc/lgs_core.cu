@@ -51,6 +51,7 @@ const OptField kOptFields[] = {
     LGS_OPT("integ_timing", "LGS_INTEG_TIMING", 0, integTiming),
     LGS_OPT("integ_diag", "LGS_INTEG_DIAG", 0, integDiag),
     LGS_OPT("integ_side_words", "LGS_INTEG_SIDE_WORDS", 2, integSideWords),
+    LGS_OPT("integ_resolve_ulps", nullptr, 1, integResolveUlps),
     LGS_OPT("gs_tables", "LGS_GS_TABLES", 0, gsTables),
 };
 #undef LGS_OPT

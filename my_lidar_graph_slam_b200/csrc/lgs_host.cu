@@ -21,6 +21,13 @@ inline int worldToCell(double p, double minP, double res) {
 
 }  // namespace
 
+void lgs_hit_point_host(const double* sensorPose, double angle, double r, double* hx, double* hy) {
+    const double cosT = std::cos(sensorPose[2] + angle);              // sensor_data.hpp:168-169
+    const double sinT = std::sin(sensorPose[2] + angle);
+    *hx = sensorPose[0] + r * cosT;
+    *hy = sensorPose[1] + r * sinT;
+}
+
 extern "C" {
 
 int lgs_scan_hit_points(const double* sensorPose, int n, const double* angles, const double* ranges,
@@ -31,9 +38,8 @@ int lgs_scan_hit_points(const double* sensorPose, int n, const double* angles, c
     for (int i = 0; i < n; ++i) {
         const double r = ranges[i];
         if (r >= rangeMax || r <= rangeMin) continue;                 // grid_map_builder.cpp:365-366
-        const double cosT = std::cos(sensorPose[2] + angles[i]);      // sensor_data.hpp:168-169
-        const double sinT = std::sin(sensorPose[2] + angles[i]);
-        const double hx = sensorPose[0] + r * cosT, hy = sensorPose[1] + r * sinT;
+        double hx, hy;
+        lgs_hit_point_host(sensorPose, angles[i], r, &hx, &hy);
         hitXY[2 * k] = hx; hitXY[2 * k + 1] = hy; ++k;
         minX = std::min(minX, hx); minY = std::min(minY, hy);         // :373-377
         maxX = std::max(maxX, hx); maxY = std::max(maxY, hy);

@@ -632,6 +632,189 @@ __global__ void grid_shift_copy_kernel(const double* __restrict__ src, int srcNx
     dst[(size_t)y * dstPitch + x] = v;
 }
 
+// ---- lgs_grid_construct_many: projection of raw scans ------------------------------------------------
+// ConstructMapFromScans (grid_map_builder.cpp:227-332) projects every beam with glibc cos / sin.  The device's
+// sincos may differ from glibc in the last ulps, so every hit is carried as an interval [lo, hi] that contains
+// glibc's value: the CPU's expression sx + r * cos(st + a) evaluated, in its operation order, at cos +- U ulps
+// (every operation is monotone; r may have either sign, so lo / hi are the smaller / larger end).  A cell whose
+// floor is equal at both ends is the CPU's cell; the bbox extremes and the near-edge hits are settled on the host
+// with glibc (DESIGN.md section 3.4).
+struct ConScan {
+    double sx, sy, st;          // sensor pose
+    double rmin, rmax;          // usable range window: a beam is used unless r >= rmax || r <= rmin
+    int beamBegin, n;           // beams [beamBegin, beamBegin + n) of the call
+    int map;
+};
+constexpr int kConThreads = 256;                 // one block per scan
+enum { kConBad = 0, kConCand = 1, kConEdge = 2 };   // ConFlags: first bad scan, bbox candidates, near-edge hits
+
+// Unsigned keys that order like the doubles they encode (no NaN): per-map bbox bounds by integer atomics.
+__host__ __device__ inline unsigned long long conKey(unsigned long long bits) {
+    return (bits >> 63) ? ~bits : (bits | 0x8000000000000000ull);
+}
+
+__device__ __forceinline__ bool conUsed(double r, const ConScan& q) { return !(r >= q.rmax || r <= q.rmin); }   // :365-366
+
+// Sum over the block of one int per thread.
+__device__ __forceinline__ int conBlockSum(int v, int* sh) {
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    if ((threadIdx.x & 31) == 0) sh[threadIdx.x >> 5] = v;
+    __syncthreads();
+    int t = 0;
+    for (int w = 0; w < kConThreads / 32; ++w) t += sh[w];
+    __syncthreads();
+    return t;
+}
+
+// Used beams per scan; the first scan with a non-finite angle or range on a used beam.
+__global__ void __launch_bounds__(kConThreads)
+con_count_kernel(const ConScan* __restrict__ scans, const double* __restrict__ angles, const double* __restrict__ ranges,
+                 int* __restrict__ count, int* __restrict__ flags) {
+    __shared__ int sh[kConThreads / 32];
+    const int s = blockIdx.x;
+    const ConScan q = scans[s];
+    int k = 0;
+    bool bad = false;
+    for (int i = threadIdx.x; i < q.n; i += kConThreads) {
+        const double r = ranges[q.beamBegin + i];
+        if (!conUsed(r, q)) continue;
+        ++k;
+        bad |= !isfinite(r) || !isfinite(angles[q.beamBegin + i]);
+    }
+    if (bad) atomicMin(flags + kConBad, s);
+    k = conBlockSum(k, sh);
+    if (threadIdx.x == 0) count[s] = k;
+}
+
+// begin[s] = hits of the scans before s (one block; begin[n] = all hits).
+__global__ void __launch_bounds__(1024) con_offsets_kernel(const int* __restrict__ count, int n, int* __restrict__ begin) {
+    __shared__ int sh[1024];
+    const int per = (n + 1023) / 1024, s0 = min(n, (int)threadIdx.x * per), s1 = min(n, s0 + per);
+    int sum = 0;
+    for (int s = s0; s < s1; ++s) sum += count[s];
+    sh[threadIdx.x] = sum;
+    __syncthreads();
+    for (int o = 1; o < 1024; o <<= 1) {                 // inclusive scan of the segment sums
+        const int v = threadIdx.x >= (unsigned)o ? sh[threadIdx.x - o] : 0;
+        __syncthreads();
+        sh[threadIdx.x] += v;
+        __syncthreads();
+    }
+    int run = sh[threadIdx.x] - sum;
+    for (int s = s0; s < s1; ++s) { begin[s] = run; run += count[s]; }
+    if (threadIdx.x == 1023) begin[n] = sh[1023];
+}
+
+// Hits of scan s in beam order at begin[s]: lo -> hit (the staging buffer of the integration), hi -> hi, the
+// call's beam index -> beam.  A non-finite end makes the interval (-inf, inf).  Per map, keys[4 m + ..] take
+// the bbox bounds the device can prove: [0] / [1] min over hits of hi.x / hi.y (min sides), [2] / [3] max of
+// lo.x / lo.y (max sides); the host seeds them with the sensor positions and the reference's initial values.
+__global__ void __launch_bounds__(kConThreads)
+con_project_kernel(const ConScan* __restrict__ scans, const double* __restrict__ angles,
+                   const double* __restrict__ ranges, const int* __restrict__ begin, double ulps,
+                   double2* __restrict__ lo, double2* __restrict__ hi, int* __restrict__ beam,
+                   unsigned long long* __restrict__ keys) {
+    __shared__ int sh[kConThreads / 32];
+    __shared__ double sr[4][kConThreads / 32];
+    const int s = blockIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const ConScan q = scans[s];
+    const double k = ulps * 2.220446049250313e-16, inf = __longlong_as_double(0x7ff0000000000000ll);
+    double bnd[4] = {inf, inf, -inf, -inf};
+    int base = begin[s];
+    for (int c0 = 0; c0 < q.n; c0 += kConThreads) {
+        const int i = c0 + threadIdx.x;
+        const double r = i < q.n ? ranges[q.beamBegin + i] : 0.0;
+        const bool used = i < q.n && conUsed(r, q);
+        const unsigned m = __ballot_sync(0xffffffffu, used);
+        if (lane == 0) sh[warp] = __popc(m);
+        __syncthreads();
+        int off = base, tot = 0;
+        for (int w = 0; w < kConThreads / 32; ++w) { off += w < warp ? sh[w] : 0; tot += sh[w]; }
+        __syncthreads();
+        base += tot;
+        if (!used) continue;
+        off += __popc(m & ((1u << lane) - 1u));
+        double sn, cs;
+        sincos(__dadd_rn(q.st, angles[q.beamBegin + i]), &sn, &cs);            // sensor_data.hpp:168-169
+        const double wc = __dadd_rn(__dmul_rn(fabs(cs), k), 4.9406564584124654e-324);
+        const double ws = __dadd_rn(__dmul_rn(fabs(sn), k), 4.9406564584124654e-324);
+        const double x0 = __dadd_rn(q.sx, __dmul_rn(r, __dsub_rn(cs, wc))), x1 = __dadd_rn(q.sx, __dmul_rn(r, __dadd_rn(cs, wc)));
+        const double y0 = __dadd_rn(q.sy, __dmul_rn(r, __dsub_rn(sn, ws))), y1 = __dadd_rn(q.sy, __dmul_rn(r, __dadd_rn(sn, ws)));
+        const bool fx = isfinite(x0) && isfinite(x1), fy = isfinite(y0) && isfinite(y1);
+        const double2 l = make_double2(fx ? fmin(x0, x1) : -inf, fy ? fmin(y0, y1) : -inf);
+        const double2 h = make_double2(fx ? fmax(x0, x1) : inf, fy ? fmax(y0, y1) : inf);
+        lo[off] = l;
+        hi[off] = h;
+        beam[off] = q.beamBegin + i;
+        bnd[0] = fmin(bnd[0], h.x); bnd[1] = fmin(bnd[1], h.y);
+        bnd[2] = fmax(bnd[2], l.x); bnd[3] = fmax(bnd[3], l.y);
+    }
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+        double v = bnd[j];
+        for (int o = 16; o > 0; o >>= 1) {
+            const double u = __shfl_xor_sync(0xffffffffu, v, o);
+            v = j < 2 ? fmin(v, u) : fmax(v, u);
+        }
+        if (lane == 0) sr[j][warp] = v;
+    }
+    __syncthreads();
+    if (threadIdx.x < 4) {
+        const int j = threadIdx.x;
+        double v = sr[j][0];
+        for (int w = 1; w < kConThreads / 32; ++w) v = j < 2 ? fmin(v, sr[j][w]) : fmax(v, sr[j][w]);
+        const unsigned long long key = conKey((unsigned long long)__double_as_longlong(v));
+        if (j < 2) atomicMin(keys + 4 * q.map + j, key); else atomicMax(keys + 4 * q.map + j, key);
+    }
+}
+
+// Hits that may hold a bbox extreme (hi >= the max side's bound, lo <= the min side's): {call beam, sides}
+// into cand[0 .. cap), every one counted in flags[kConCand].
+__global__ void __launch_bounds__(kConThreads)
+con_candidates_kernel(const ConScan* __restrict__ scans, const int* __restrict__ begin, const double2* __restrict__ lo,
+                      const double2* __restrict__ hi, const int* __restrict__ beam,
+                      const unsigned long long* __restrict__ keys, int2* __restrict__ cand, int cap, int* __restrict__ flags) {
+    const int s = blockIdx.x;
+    const unsigned long long* K = keys + 4 * scans[s].map;
+    const unsigned long long k0 = K[0], k1 = K[1], k2 = K[2], k3 = K[3];
+    for (int b = begin[s] + threadIdx.x; b < begin[s + 1]; b += kConThreads) {
+        const double2 l = lo[b], h = hi[b];
+        const int sides = (conKey((unsigned long long)__double_as_longlong(l.x)) <= k0 ? 1 : 0) |
+                          (conKey((unsigned long long)__double_as_longlong(l.y)) <= k1 ? 2 : 0) |
+                          (conKey((unsigned long long)__double_as_longlong(h.x)) >= k2 ? 4 : 0) |
+                          (conKey((unsigned long long)__double_as_longlong(h.y)) >= k3 ? 8 : 0);
+        if (!sides) continue;
+        const int slot = atomicAdd(flags + kConCand, 1);
+        if (slot < cap) cand[slot] = make_int2(beam[b], sides);
+    }
+}
+
+// Hits whose interval ends fall into different cells of their map's new geometry (geo[3 m ..] = min_x, min_y,
+// res): {hit, call beam} into edge[0 .. cap), every one counted in flags[kConEdge].  The cells are the
+// integration's (integ_beam_kernel), so a hit that is not listed keeps lo, which lies in the CPU's cell.
+__global__ void __launch_bounds__(kConThreads)
+con_edge_kernel(const ConScan* __restrict__ scans, const int* __restrict__ begin, const double2* __restrict__ lo,
+                const double2* __restrict__ hi, const int* __restrict__ beam, const double* __restrict__ geo,
+                int2* __restrict__ edge, int cap, int* __restrict__ flags) {
+    const int s = blockIdx.x;
+    const double* G = geo + 3 * scans[s].map;
+    const double minX = G[0], minY = G[1], res = G[2];
+    auto cell = [&](double p, double mn) { return __double2int_rd(__ddiv_rn(__dsub_rn(p, mn), res)); };
+    for (int b = begin[s] + threadIdx.x; b < begin[s + 1]; b += kConThreads) {
+        const double2 l = lo[b], h = hi[b];
+        if (cell(l.x, minX) == cell(h.x, minX) && cell(l.y, minY) == cell(h.y, minY)) continue;
+        const int slot = atomicAdd(flags + kConEdge, 1);
+        if (slot < cap) edge[slot] = make_int2(b, beam[b]);
+    }
+}
+
+// The host's glibc hit of every near-edge hit, in the order of the edge list.
+__global__ void con_patch_kernel(const int2* __restrict__ edge, const double2* __restrict__ val, int n,
+                                 double2* __restrict__ hit) {
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k < n) hit[edge[k].x] = val[k];
+}
+
 }  // namespace
 
 extern "C" {
@@ -639,6 +822,10 @@ extern "C" {
 }  // extern "C"
 
 namespace {
+
+// The grid takes nx x ny cells at (minX, minY) in a fresh buffer, on its own context's stream; with `copy`, new
+// cell (x, y) takes old cell (x + shiftX, y + shiftY) (one launch), otherwise every cell is unknown.
+int grid_replace(lgs_grid* g, int nx, int ny, double minX, double minY, bool copy, int shiftX, int shiftY);
 
 // Completion of the OLDEST submitted call: its update count, the fallback statistics, its staging set.
 int integ_wait(lgs_ctx* c, long long* nUpdatesOut) {
@@ -655,12 +842,13 @@ int integ_wait(lgs_ctx* c, long long* nUpdatesOut) {
     return LGS_OK;
 }
 
-// The checks of one (grid, scan batch) pair of a call; map = its index in the call.
+// The checks of one (grid, scan batch) pair of a call; map = its index in the call.  b == NULL: the grid only
+// (lgs_grid_construct_many checks its raw scans itself).
 int integ_check(lgs_ctx* c, int map, const lgs_grid* g, const lgs_hit_batch* b) {
     if (!g) return lgs_fail(c, LGS_ERR_INVALID, "integrate: grid of map %d is NULL", map);
-    if (b->n_scans < 0 || (b->n_scans > 0 && (!b->sensor_xy || !b->hit_begin)))
+    if (b && (b->n_scans < 0 || (b->n_scans > 0 && (!b->sensor_xy || !b->hit_begin))))
         return lgs_fail(c, LGS_ERR_INVALID, "integrate: bad scan batch of map %d", map);
-    if (b->n_scans > 0 && b->hit_begin[b->n_scans] > 0 && !b->hit_xy)
+    if (b && b->n_scans > 0 && b->hit_begin[b->n_scans] > 0 && !b->hit_xy)
         return lgs_fail(c, LGS_ERR_INVALID, "integrate: hit_xy of map %d is NULL", map);
     if (g->off_x || g->off_y)
         return lgs_fail(c, LGS_ERR_INVALID, "integrate: grid of map %d is windowed (lgs_grid_set_window), not supported", map);
@@ -670,12 +858,37 @@ int integ_check(lgs_ctx* c, int map, const lgs_grid* g, const lgs_hit_batch* b) 
     return LGS_OK;
 }
 
+// The checks of a synchronous many-map call (`who` names it in the messages): nothing submitted in flight,
+// every (grid, batch) pair, no grid twice.  batches == NULL: grids only.
+int integ_check_many(lgs_ctx* c, const char* who, int nMaps, lgs_grid* const* grids, const lgs_hit_batch* batches) {
+    if (c->integ && c->integ->nPending > 0)
+        return lgs_fail(c, LGS_ERR_INVALID, "%s: an lgs_grid_integrate_submit call is in flight, wait for it first", who);
+    for (int i = 0; i < nMaps; ++i) {
+        const int rc = integ_check(c, i, grids[i], batches ? &batches[i] : nullptr);
+        if (rc != LGS_OK) return rc;
+    }
+    std::vector<const lgs_grid*> sorted(grids, grids + nMaps);
+    std::sort(sorted.begin(), sorted.end());
+    if (std::adjacent_find(sorted.begin(), sorted.end()) != sorted.end())
+        return lgs_fail(c, LGS_ERR_INVALID, "%s: the same grid appears twice", who);
+    return LGS_OK;
+}
+
+// The integration workspace of a context, with its copy stream.
+int integ_workspace(lgs_ctx* c) {
+    if (!c->integ) c->integ = new lgs_integ_ws();
+    if (!c->integ->copyStream) LGS_CUDA(c, cudaStreamCreateWithFlags(&c->integ->copyStream, cudaStreamNonBlocking));
+    return LGS_OK;
+}
+
 // Everything of a call up to the last enqueue; the host waits only for the pre-pass (scan bounds).
 // A call integrates batches[i] into grids[i], i < nMaps (checked by the caller): every map is staged into
 // one blob behind a device table of grids, and the next chunk of every map goes into one round of
-// launches.  perMap (NULL = not wanted) receives each map's update count.
+// launches.  perMap (NULL = not wanted) receives each map's update count.  hitsOnDevice: the hits are
+// already in the staging set's hit buffer, at the call's hit offsets (lgs_grid_construct_many's device
+// projection, queued on the copy stream), and batches[].hit_xy is not read.
 int integ_submit(lgs_ctx* c, int nMaps, lgs_grid* const* grids, const lgs_hit_batch* batches, double pHit,
-                 double pMiss, long long* perMap) {
+                 double pMiss, long long* perMap, bool hitsOnDevice = false) {
     // scans of map i are scans [scanBase[i], scanBase[i + 1]) of the call, their hits start at hitBase[i]
     std::vector<int> scanBase(nMaps + 1, 0);
     std::vector<long long> hitBase(nMaps + 1, 0);
@@ -689,12 +902,12 @@ int integ_submit(lgs_ctx* c, int nMaps, lgs_grid* const* grids, const lgs_hit_ba
     if (total > 0x7fffffffLL) return lgs_fail(c, LGS_ERR_INVALID, "integrate: %lld hits in one call (at most 2^31 - 1)", total);
     LGS_CUDA(c, cudaSetDevice(c->device));
     for (int i = 0; i < nMaps; ++i) LGS_CUDA(c, lgs_grid_acquire(c, grids[i]));
-    if (!c->integ) c->integ = new lgs_integ_ws();
+    const int rcWs = integ_workspace(c);
+    if (rcWs != LGS_OK) return rcWs;
     lgs_integ_ws& ws = *c->integ;
     if (ws.nPending >= 2 || ws.stage[ws.calls & 1].pending)
         return lgs_fail(c, LGS_ERR_INVALID, "integrate: two calls are in flight, wait for the older one first");
     lgs_integ_ws::Stage& w0 = ws.stage[ws.calls & 1];
-    if (!ws.copyStream) LGS_CUDA(c, cudaStreamCreateWithFlags(&ws.copyStream, cudaStreamNonBlocking));
     if (!w0.evDone) {
         LGS_CUDA(c, cudaEventCreateWithFlags(&w0.evDone, cudaEventDisableTiming));
         LGS_CUDA(c, cudaEventCreateWithFlags(&w0.evCounters, cudaEventDisableTiming));
@@ -748,7 +961,7 @@ int integ_submit(lgs_ctx* c, int nMaps, lgs_grid* const* grids, const lgs_hit_ba
         if (b.n_scans == 0) continue;
         LGS_CUDA(c, cudaMemcpyAsync(w.sensor.p + 2 * (size_t)scanBase[i], b.sensor_xy,
                                     (size_t)b.n_scans * 2 * sizeof(double), cudaMemcpyHostToDevice, cs0));
-        if (hitBase[i + 1] > hitBase[i])
+        if (!hitsOnDevice && hitBase[i + 1] > hitBase[i])
             LGS_CUDA(c, cudaMemcpyAsync(w.hit.p + 2 * (size_t)hitBase[i], b.hit_xy,
                                         (size_t)(hitBase[i + 1] - hitBase[i]) * 2 * sizeof(double),
                                         cudaMemcpyHostToDevice, cs0));
@@ -1045,26 +1258,270 @@ int lgs_grid_integrate_many(lgs_ctx* c, int nMaps, lgs_grid* const* grids, const
         return lgs_fail(c, LGS_ERR_INVALID, "integrate_many: %d maps, grids %p, scans %p", nMaps, (const void*)grids,
                         (const void*)scans);
     if (nUpdates) std::fill(nUpdates, nUpdates + nMaps, 0LL);
-    if (c->integ && c->integ->nPending > 0)
-        return lgs_fail(c, LGS_ERR_INVALID, "integrate_many: an lgs_grid_integrate_submit call is in flight, wait for it first");
     // every argument is checked before anything is staged: a refused call leaves every grid as it was
-    for (int i = 0; i < nMaps; ++i) {
-        const int rc = integ_check(c, i, grids[i], &scans[i]);
-        if (rc != LGS_OK) return rc;
-    }
-    std::vector<const lgs_grid*> sorted(grids, grids + nMaps);
-    std::sort(sorted.begin(), sorted.end());
-    if (std::adjacent_find(sorted.begin(), sorted.end()) != sorted.end())
-        return lgs_fail(c, LGS_ERR_INVALID, "integrate_many: the same grid appears twice");
-    const int rc = integ_submit(c, nMaps, grids, scans, pHit, pMiss, nUpdates);
+    int rc = integ_check_many(c, "integrate_many", nMaps, grids, scans);
+    if (rc != LGS_OK) return rc;
+    rc = integ_submit(c, nMaps, grids, scans, pHit, pMiss, nUpdates);
     if (rc != LGS_OK) return rc;
     return integ_wait(c, nullptr);
+}
+
+int lgs_grid_construct_many(lgs_ctx* c, int nMaps, lgs_grid* const* grids, const lgs_scan_batch* scans,
+                            const lgs_geometry* cur, double pHit, double pMiss, lgs_geometry* geoOut,
+                            double* bboxOut, long long* nUpdates) {
+    if (!c) return LGS_ERR_INVALID;
+    if (nMaps < 0 || (nMaps > 0 && (!grids || !scans || !cur || !geoOut)))
+        return lgs_fail(c, LGS_ERR_INVALID, "construct_many: %d maps, grids %p, scans %p, cur %p, geometry_out %p", nMaps,
+                        (const void*)grids, (const void*)scans, (const void*)cur, (const void*)geoOut);
+    if (nUpdates) std::fill(nUpdates, nUpdates + nMaps, 0LL);
+    // every argument is checked before any grid changes: a refused call leaves every grid as it was
+    int rc = integ_check_many(c, "construct_many", nMaps, grids, nullptr);
+    if (rc != LGS_OK) return rc;
+    std::vector<ConScan> hs;
+    std::vector<int> scanBase(nMaps + 1, 0);
+    std::vector<long long> beamBase(nMaps + 1, 0);
+    for (int i = 0; i < nMaps; ++i) {
+        const lgs_scan_batch& b = scans[i];
+        if (b.n_scans < 1) return lgs_fail(c, LGS_ERR_INVALID, "construct_many: map %d has no scans", i);
+        if (!b.beam_begin || !b.sensor_pose || !b.range_min || !b.range_max)
+            return lgs_fail(c, LGS_ERR_INVALID, "construct_many: map %d: beam_begin, sensor_pose, range_min and range_max "
+                            "are required", i);
+        const lgs_geometry& g = cur[i];
+        if (g.patch <= 0 || !(g.res > 0.0) || !std::isfinite(g.res) || !std::isfinite(g.min_x) || !std::isfinite(g.min_y))
+            return lgs_fail(c, LGS_ERR_INVALID, "construct_many: bad current geometry of map %d", i);
+        for (int s = 0; s < b.n_scans; ++s) {
+            const double* p = b.sensor_pose + 3 * s;
+            if (b.beam_begin[s + 1] < b.beam_begin[s])
+                return lgs_fail(c, LGS_ERR_INVALID, "construct_many: map %d, scan %d: beam_begin decreases", i, s);
+            if (!std::isfinite(p[0]) || !std::isfinite(p[1]) || !std::isfinite(p[2]) ||
+                !std::isfinite(b.range_min[s]) || !std::isfinite(b.range_max[s]))
+                return lgs_fail(c, LGS_ERR_INVALID, "construct_many: map %d, scan %d: non-finite sensor pose or range window", i, s);
+            hs.push_back(ConScan{p[0], p[1], p[2], b.range_min[s], b.range_max[s],
+                                 (int)(beamBase[i] + b.beam_begin[s] - b.beam_begin[0]), b.beam_begin[s + 1] - b.beam_begin[s], i});
+        }
+        const long long nb = b.beam_begin[b.n_scans] - b.beam_begin[0];
+        if (nb > 0 && (!b.angles || !b.ranges)) return lgs_fail(c, LGS_ERR_INVALID, "construct_many: map %d: angles / ranges NULL", i);
+        scanBase[i + 1] = scanBase[i] + b.n_scans;
+        beamBase[i + 1] = beamBase[i] + nb;
+        if (beamBase[i + 1] > 0x7fffffffLL)
+            return lgs_fail(c, LGS_ERR_INVALID, "construct_many: more than 2^31 - 1 beams in one call");
+    }
+    if (nMaps == 0) return LGS_OK;
+    const int n = scanBase[nMaps];
+    const long long beams = beamBase[nMaps];
+    LGS_CUDA(c, cudaSetDevice(c->device));
+    rc = integ_workspace(c);
+    if (rc != LGS_OK) return rc;
+    lgs_integ_ws& ws = *c->integ;
+    lgs_integ_ws::Construct& w = ws.con;
+    DevBuf<double>& hit = ws.stage[ws.calls & 1].hit;          // the staging set integ_submit uses next
+    cudaStream_t cs = ws.copyStream;                            // integ_submit's pre-pass follows on it
+
+    // Stage: raw beams, the scan table, the bbox seeds (DBL_MAX / DBL_MIN as ConstructMapFromScans starts them,
+    // :236-237, and every sensor position), the flags.
+    const double kTiny = 2.2250738585072014e-308, kMax = 1.7976931348623157e308;
+    std::vector<unsigned long long> keys(4 * (size_t)nMaps);
+    auto key = [](double v) { unsigned long long u; memcpy(&u, &v, 8); return conKey(u); };
+    for (int i = 0; i < nMaps; ++i) {
+        double bx0 = kMax, by0 = kMax, bx1 = kTiny, by1 = kTiny;
+        for (int s = scanBase[i]; s < scanBase[i + 1]; ++s) {
+            bx0 = std::min(bx0, hs[s].sx); by0 = std::min(by0, hs[s].sy);
+            bx1 = std::max(bx1, hs[s].sx); by1 = std::max(by1, hs[s].sy);
+        }
+        keys[4 * i] = key(bx0); keys[4 * i + 1] = key(by0); keys[4 * i + 2] = key(bx1); keys[4 * i + 3] = key(by1);
+    }
+    const size_t nbAlloc = std::max<size_t>((size_t)beams, 1);
+    LGS_CUDA(c, w.angles.reserve(nbAlloc));
+    LGS_CUDA(c, w.ranges.reserve(nbAlloc));
+    LGS_CUDA(c, hit.reserve(2 * nbAlloc));
+    LGS_CUDA(c, w.hi.reserve(2 * nbAlloc));
+    LGS_CUDA(c, w.beam.reserve(nbAlloc));
+    LGS_CUDA(c, w.scans.reserve((size_t)n * sizeof(ConScan)));
+    LGS_CUDA(c, w.count.reserve((size_t)n));
+    LGS_CUDA(c, w.begin.reserve((size_t)n + 1));
+    LGS_CUDA(c, w.keys.reserve(4 * (size_t)nMaps));
+    LGS_CUDA(c, w.geo.reserve(3 * (size_t)nMaps));
+    LGS_CUDA(c, w.flags.reserve(4));
+    LGS_CUDA(c, w.hFlags.reserve(4));
+    LGS_CUDA(c, w.hCount.reserve((size_t)n));
+    if (w.cand.cap == 0) LGS_CUDA(c, w.cand.reserve(4096));
+    if (w.edge.cap == 0) LGS_CUDA(c, w.edge.reserve(4096));
+    for (int i = 0; i < nMaps; ++i) {
+        const lgs_scan_batch& b = scans[i];
+        const size_t nb = (size_t)(beamBase[i + 1] - beamBase[i]);
+        if (nb == 0) continue;
+        LGS_CUDA(c, cudaMemcpyAsync(w.angles.p + beamBase[i], b.angles + b.beam_begin[0], nb * sizeof(double),
+                                    cudaMemcpyHostToDevice, cs));
+        LGS_CUDA(c, cudaMemcpyAsync(w.ranges.p + beamBase[i], b.ranges + b.beam_begin[0], nb * sizeof(double),
+                                    cudaMemcpyHostToDevice, cs));
+    }
+    LGS_CUDA(c, cudaMemcpyAsync(w.scans.p, hs.data(), (size_t)n * sizeof(ConScan), cudaMemcpyHostToDevice, cs));
+    LGS_CUDA(c, cudaMemcpyAsync(w.keys.p, keys.data(), keys.size() * sizeof(unsigned long long), cudaMemcpyHostToDevice, cs));
+    const int flags0[4] = {0x7fffffff, 0, 0, 0};
+    LGS_CUDA(c, cudaMemcpyAsync(w.flags.p, flags0, sizeof(flags0), cudaMemcpyHostToDevice, cs));
+    const ConScan* dScans = reinterpret_cast<const ConScan*>(w.scans.p);
+    double2* lo = reinterpret_cast<double2*>(hit.p);
+    const double2* hi = reinterpret_cast<const double2*>(w.hi.p);
+
+    // Projection, bbox bounds and candidates; the host reads the hit counts and the candidates back.
+    con_count_kernel<<<n, kConThreads, 0, cs>>>(dScans, w.angles.p, w.ranges.p, w.count.p, w.flags.p);
+    LGS_LAUNCH_CHECK(c);
+    con_offsets_kernel<<<1, 1024, 0, cs>>>(w.count.p, n, w.begin.p);
+    LGS_LAUNCH_CHECK(c);
+    con_project_kernel<<<n, kConThreads, 0, cs>>>(dScans, w.angles.p, w.ranges.p, w.begin.p,
+                                                  std::max(c->opt.integResolveUlps, 0.0), lo,
+                                                  reinterpret_cast<double2*>(w.hi.p), w.beam.p, w.keys.p);
+    LGS_LAUNCH_CHECK(c);
+    // A fix-up list comes back with its count; a list longer than its buffer is listed again into a grown one.
+    auto fetchList = [&](DevBuf<int2>& list, int which, auto launch) -> int {
+        LGS_CUDA(c, cudaMemsetAsync(w.flags.p + which, 0, sizeof(int), cs));
+        launch();
+        LGS_LAUNCH_CHECK(c);
+        LGS_CUDA(c, cudaMemcpyAsync(w.hFlags.p, w.flags.p, 4 * sizeof(int), cudaMemcpyDeviceToHost, cs));
+        LGS_CUDA(c, cudaStreamSynchronize(cs));
+        const int cnt = w.hFlags.p[which];
+        if ((size_t)cnt > list.cap) {
+            LGS_CUDA(c, list.reserve((size_t)cnt));
+            LGS_CUDA(c, cudaMemsetAsync(w.flags.p + which, 0, sizeof(int), cs));
+            launch();
+            LGS_LAUNCH_CHECK(c);
+        }
+        LGS_CUDA(c, w.hList.reserve(std::max(cnt, 1)));
+        LGS_CUDA(c, cudaMemcpyAsync(w.hList.p, list.p, (size_t)cnt * sizeof(int2), cudaMemcpyDeviceToHost, cs));
+        LGS_CUDA(c, cudaStreamSynchronize(cs));
+        return LGS_OK;
+    };
+    LGS_CUDA(c, cudaMemcpyAsync(w.hCount.p, w.count.p, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, cs));
+    rc = fetchList(w.cand, kConCand, [&]() {
+        con_candidates_kernel<<<n, kConThreads, 0, cs>>>(dScans, w.begin.p, lo, hi, w.beam.p, w.keys.p, w.cand.p,
+                                                         (int)std::min<size_t>(w.cand.cap, 0x7fffffff), w.flags.p);
+    });
+    if (rc != LGS_OK) return rc;
+    if (w.hFlags.p[kConBad] != 0x7fffffff) {
+        const int s = w.hFlags.p[kConBad];
+        const int i = (int)(std::upper_bound(scanBase.begin(), scanBase.end(), s) - scanBase.begin()) - 1;
+        return lgs_fail(c, LGS_ERR_INVALID, "construct_many: map %d, scan %d: a beam that passes the range filter has a "
+                        "non-finite angle or range", i, s - scanBase[i]);
+    }
+    const int nCand = w.hFlags.p[kConCand];
+    ws.conBboxPoints += nCand;
+
+    // The scan and beam of a call beam, and glibc's hit of it.
+    auto hostHit = [&](int callBeam, double* hx, double* hy) {
+        const int i = (int)(std::upper_bound(beamBase.begin(), beamBase.end(), (long long)callBeam) - beamBase.begin()) - 1;
+        const lgs_scan_batch& b = scans[i];
+        const int j = b.beam_begin[0] + (int)(callBeam - beamBase[i]);                 // beam of the batch
+        const int s = (int)(std::upper_bound(b.beam_begin, b.beam_begin + b.n_scans + 1, j) - b.beam_begin) - 1;
+        lgs_hit_point_host(b.sensor_pose + 3 * s, b.angles[j], b.ranges[j], hx, hy);
+    };
+    // Exact bbox: the seeds, every sensor position and the candidates' glibc hits, in (scan, beam) order like
+    // the reference (no other hit can be an extreme).  Then GridMap::Resize's geometry and the size check.
+    std::vector<int2> cands(w.hList.p, w.hList.p + nCand);
+    std::vector<int> order(nCand);
+    for (int k = 0; k < nCand; ++k) order[k] = k;
+    std::sort(order.begin(), order.end(), [&](int a, int b) { return cands[a].x < cands[b].x; });
+    std::vector<lgs_geometry> geo(nMaps);
+    std::vector<double> bbox(4 * (size_t)nMaps), geoTab(3 * (size_t)nMaps);
+    for (int i = 0, k = 0; i < nMaps; ++i) {
+        double bx0 = kMax, by0 = kMax, bx1 = kTiny, by1 = kTiny;
+        for (int s = scanBase[i]; s < scanBase[i + 1]; ++s) {
+            bx0 = std::min(bx0, hs[s].sx); by0 = std::min(by0, hs[s].sy);
+            bx1 = std::max(bx1, hs[s].sx); by1 = std::max(by1, hs[s].sy);
+            for (; k < nCand && cands[order[k]].x < hs[s].beamBegin + hs[s].n; ++k) {
+                double hx, hy;
+                hostHit(cands[order[k]].x, &hx, &hy);
+                bx0 = std::min(bx0, hx); by0 = std::min(by0, hy);
+                bx1 = std::max(bx1, hx); by1 = std::max(by1, hy);
+            }
+        }
+        bbox[4 * i] = bx0; bbox[4 * i + 1] = by0; bbox[4 * i + 2] = bx1; bbox[4 * i + 3] = by1;
+        if (lgs_geometry_resize(&cur[i], bx0, by0, bx1, by1, &geo[i], nullptr, nullptr) != LGS_OK)
+            return lgs_fail(c, LGS_ERR_INVALID, "construct_many: map %d: no geometry for bbox [%g, %g] x [%g, %g]", i, bx0, bx1, by0, by1);
+        const long long a = grids[i]->apron;
+        if (((long long)geo[i].nx + 2 * a) * ((long long)geo[i].ny + 2 * a) >= (1LL << 31))
+            return lgs_fail(c, LGS_ERR_INVALID, "construct_many: map %d: %dx%d cells are too many", i, geo[i].nx, geo[i].ny);
+        geoTab[3 * i] = geo[i].min_x; geoTab[3 * i + 1] = geo[i].min_y; geoTab[3 * i + 2] = geo[i].res;
+    }
+
+    // GridMap::Resize + Reset: every grid takes its new geometry with every cell unknown, on its own stream.
+    for (int i = 0; i < nMaps; ++i) {
+        lgs_grid* g = grids[i];
+        g->res = geo[i].res;
+        if (g->nx == geo[i].nx && g->ny == geo[i].ny) {
+            g->min_x = geo[i].min_x; g->min_y = geo[i].min_y;
+            rc = lgs_grid_clear(g);
+        } else {
+            rc = grid_replace(g, geo[i].nx, geo[i].ny, geo[i].min_x, geo[i].min_y, false, 0, 0);
+        }
+        if (rc != LGS_OK) {
+            const std::string why = g->ctx->err;
+            return lgs_fail(c, rc, "construct_many: map %d: %s", i, why.c_str());
+        }
+        geoOut[i] = geo[i];
+        if (bboxOut) std::copy(&bbox[4 * i], &bbox[4 * i + 4], bboxOut + 4 * i);
+    }
+
+    // Near-edge hits: glibc's hit replaces the interval end in the staging buffer.
+    LGS_CUDA(c, cudaMemcpyAsync(w.geo.p, geoTab.data(), geoTab.size() * sizeof(double), cudaMemcpyHostToDevice, cs));
+    rc = fetchList(w.edge, kConEdge, [&]() {
+        con_edge_kernel<<<n, kConThreads, 0, cs>>>(dScans, w.begin.p, lo, hi, w.beam.p, w.geo.p, w.edge.p,
+                                                   (int)std::min<size_t>(w.edge.cap, 0x7fffffff), w.flags.p);
+    });
+    if (rc != LGS_OK) return rc;
+    const int nEdge = w.hFlags.p[kConEdge];
+    ws.conEdgePoints += nEdge;
+    std::vector<double> patch(2 * (size_t)std::max(nEdge, 1));
+    for (int k = 0; k < nEdge; ++k) hostHit(w.hList.p[k].y, &patch[2 * k], &patch[2 * k + 1]);
+    LGS_CUDA(c, w.patch.reserve(patch.size()));
+    LGS_CUDA(c, cudaMemcpyAsync(w.patch.p, patch.data(), patch.size() * sizeof(double), cudaMemcpyHostToDevice, cs));
+    con_patch_kernel<<<std::max((nEdge + 255) / 256, 1), 256, 0, cs>>>(w.edge.p, reinterpret_cast<const double2*>(w.patch.p),
+                                                                      nEdge, lo);
+    LGS_LAUNCH_CHECK(c);
+
+    // From here on the integration of lgs_grid_integrate_many, its hits already staged.
+    std::vector<double> sensorXY(2 * (size_t)n);
+    std::vector<int> hitBegin((size_t)n + nMaps);
+    std::vector<lgs_hit_batch> batches(nMaps);
+    for (int i = 0; i < nMaps; ++i) {
+        int* hb = hitBegin.data() + scanBase[i] + i;
+        hb[0] = 0;
+        for (int s = scanBase[i]; s < scanBase[i + 1]; ++s) {
+            sensorXY[2 * s] = hs[s].sx; sensorXY[2 * s + 1] = hs[s].sy;
+            hb[s - scanBase[i] + 1] = hb[s - scanBase[i]] + w.hCount.p[s];
+        }
+        batches[i] = lgs_hit_batch{scans[i].n_scans, sensorXY.data() + 2 * scanBase[i], hb, nullptr};
+    }
+    rc = integ_submit(c, nMaps, grids, batches.data(), pHit, pMiss, nUpdates, true);
+    if (rc != LGS_OK) return rc;
+    return integ_wait(c, nullptr);
+}
+
+int lgs_ctx_construct_host_points(const lgs_ctx* c, long long* bboxPoints, long long* edgePoints) {
+    if (!c) return LGS_ERR_INVALID;
+    if (bboxPoints) *bboxPoints = c->integ ? c->integ->conBboxPoints : 0;
+    if (edgePoints) *edgePoints = c->integ ? c->integ->conEdgePoints : 0;
+    return LGS_OK;
 }
 
 long long lgs_ctx_integrate_fallback_cells(const lgs_ctx* c) { return (c && c->integ) ? c->integ->fallbackCells : 0; }
 
 int lgs_grid_resize(lgs_grid* g, int nx, int ny, double minX, double minY, int shiftX, int shiftY) {
+    return g ? grid_replace(g, nx, ny, minX, minY, true, shiftX, shiftY) : LGS_ERR_INVALID;
+}
+
+int lgs_grid_clear(lgs_grid* g) {
     if (!g) return LGS_ERR_INVALID;
+    lgs_ctx* c = g->ctx;
+    LGS_CUDA(c, cudaSetDevice(c->device));
+    LGS_CUDA(c, cudaMemsetAsync(g->d, 0, (size_t)g->pitch * g->rows * sizeof(double), c->stream));
+    return LGS_OK;
+}
+
+}  // extern "C"
+
+namespace {
+
+int grid_replace(lgs_grid* g, int nx, int ny, double minX, double minY, bool copy, int shiftX, int shiftY) {
     lgs_ctx* c = g->ctx;
     if (nx < 0 || ny < 0) return lgs_fail(c, LGS_ERR_INVALID, "grid_resize: %dx%d", nx, ny);
     const long long pitch = (long long)nx + 2LL * g->apron, rows = (long long)ny + 2LL * g->apron;
@@ -1077,7 +1534,7 @@ int lgs_grid_resize(lgs_grid* g, int nx, int ny, double minX, double minY, int s
     cudaError_t e = lgs_alloc_async(c, &nd, std::max<size_t>(bytes, 8));
     if (e != cudaSuccess) return lgs_fail(c, LGS_ERR_NOMEM, "grid_resize: cudaMallocAsync(%zu) -> %s", bytes, cudaGetErrorString(e));
     LGS_CUDA(c, cudaMemsetAsync(nd, 0, bytes, c->stream));
-    if (nx > 0 && ny > 0) {
+    if (copy && nx > 0 && ny > 0) {
         dim3 gridDim((nx + 255) / 256, ny);
         grid_shift_copy_kernel<<<gridDim, 256, 0, c->stream>>>(g->origin(), g->nx, g->ny, g->pitch,
                                                                nd + (size_t)g->apron * pitch + g->apron,
@@ -1090,12 +1547,4 @@ int lgs_grid_resize(lgs_grid* g, int nx, int ny, double minX, double minY, int s
     return LGS_OK;
 }
 
-int lgs_grid_clear(lgs_grid* g) {
-    if (!g) return LGS_ERR_INVALID;
-    lgs_ctx* c = g->ctx;
-    LGS_CUDA(c, cudaSetDevice(c->device));
-    LGS_CUDA(c, cudaMemsetAsync(g->d, 0, (size_t)g->pitch * g->rows * sizeof(double), c->stream));
-    return LGS_OK;
-}
-
-}  // extern "C"
+}  // namespace

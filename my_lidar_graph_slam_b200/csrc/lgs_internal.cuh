@@ -132,10 +132,29 @@ struct lgs_integ_ws {
     // per-scan update counts of a call that asks for each map's count (lgs_grid_integrate_many, synchronous)
     DevBuf<unsigned long long> touches;
     PinBuf<unsigned long long> hTouches;
+    // Device projection of lgs_grid_construct_many (the projected hits themselves go into stage[].hit):
+    // raw beams, per-scan inputs and hit counts / offsets, the upper interval ends and the beam of every hit,
+    // per-map bbox keys and geometry, and the host fix-up lists (bbox candidates, near-edge hits).
+    struct Construct {
+        DevBuf<double> angles, ranges, hi, geo;
+        DevBuf<char> scans;
+        DevBuf<int> count, begin, beam, flags;
+        DevBuf<unsigned long long> keys;
+        DevBuf<int2> cand, edge;
+        DevBuf<double> patch;
+        PinBuf<int> hCount, hFlags;
+        PinBuf<int2> hList;
+        void release() {
+            angles.release(); ranges.release(); hi.release(); geo.release(); scans.release(); count.release();
+            begin.release(); beam.release(); flags.release(); keys.release(); cand.release(); edge.release();
+            patch.release(); hCount.release(); hFlags.release(); hList.release();
+        }
+    } con;
+    long long conBboxPoints = 0, conEdgePoints = 0;   // points re-derived on the host (lgs_ctx_construct_host_points)
     void release() {
         stage[0].release(); stage[1].release();
         kmin.release(); kmax.release();
-        regions.release(); touches.release(); hTouches.release();
+        regions.release(); touches.release(); hTouches.release(); con.release();
         for (int b = 0; b < 2; ++b) {
             tileInfo[b].release(); pairs[b].release(); records[b].release(); side[b].release();
             if (evTouch[b]) cudaEventDestroy(evTouch[b]);
@@ -174,6 +193,7 @@ struct lgs_opts {
     int integTiming = 0;        // "integ_timing"    LGS_INTEG_TIMING
     int integDiag = 0;          // "integ_diag"      LGS_INTEG_DIAG
     long long integSideWords = 0; // "integ_side_words" LGS_INTEG_SIDE_WORDS (0 = default size)
+    double integResolveUlps = 8.0;  // "integ_resolve_ulps" half width (ulps of cos / sin) of lgs_grid_construct_many's intervals
     int gsTables = 0;           // "gs_tables"       LGS_GS_TABLES: grid search through the index tables
 };
 
@@ -198,6 +218,10 @@ struct lgs_ctx {
 // differ from glibc's in the last ulp (SURVEY.md H5).  Device-vs-host differences are
 // below 1e-11 cells for |coordinates| < 1e4 m, so 1e-9 leaves two orders of magnitude.
 #define LGS_EDGE_EPS_DEFAULT 1e-9
+
+// ScanData::HitPoint with glibc cos / sin in the reference's operation order (lgs_host.cu): the host
+// arithmetic every device projection is checked against.
+void lgs_hit_point_host(const double* sensorPose, double angle, double r, double* hx, double* hy);
 
 // Stream-ordered allocation from the context's private pool (freed with cudaFreeAsync).
 inline cudaError_t lgs_alloc_async(lgs_ctx* c, void** p, size_t bytes) {
