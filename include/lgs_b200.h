@@ -296,19 +296,32 @@ int lgs_rtcsm_batch_destroy(lgs_rtcsm_batch* b);
 int lgs_rtcsm_batch_upload(lgs_rtcsm_batch* b, const lgs_grid* grid, const lgs_scan_batch* scans,
                            const double* norm_threshold);
 int lgs_rtcsm_batch_run(lgs_rtcsm_batch* b, const lgs_grid* grid, const lgs_grid* coarse);
-/* Same as run, but brackets the three kernels with CUDA events and waits:
- * ms[0] = projection, ms[1] = sweep (the hot kernel), ms[2] = selection. */
+/* Windows of >= 512 hypotheses are scored exactly but not exhaustively: every coarse hypothesis, then only
+ * the fine tiles whose coarse scores can still reach the match's best fine score (the reference scores a
+ * fine block only when its coarse score beats the running best).  This needs `coarse` to be
+ * lgs_precompute(grid, low_res) of `grid`, as the reference's precomputed map is.
+ * Same as run, but brackets the stages with CUDA events and waits:
+ * ms[0] = projection, ms[1] = scoring (coarse scores, bound, work list, fine scores), ms[2] = selection. */
 int lgs_rtcsm_batch_run_timed(lgs_rtcsm_batch* b, const lgs_grid* grid, const lgs_grid* coarse,
                               float* ms);
 int lgs_rtcsm_batch_results(lgs_rtcsm_batch* b, const lgs_grid* grid, const lgs_grid* coarse,
                             lgs_match_result* out);
 /* Test/diagnostic access to the per-match scratch of scan `m` after a run:
  * fine[nT][nyw][nxw], coarse[nT][nbx][nby], cells[nT][nKept][2] (projected cell indices,
- * un-clamped), dims = {nT, nxw, nyw, nbx, nby, nKept}.  Any pointer may be NULL. */
+ * un-clamped), dims = {nT, nxw, nyw, nbx, nby, nKept}.  Any pointer may be NULL.
+ * After a pruned run, the first call that asks for `fine` or `coarse` scores the whole batch again with
+ * the exhaustive sweep against the grids of that run, which must still exist unchanged, and waits for it
+ * (about the time of a run without pruning); later calls only copy. */
 int lgs_rtcsm_batch_debug(lgs_rtcsm_batch* b, int m, int* dims, double* fine, double* coarse,
                           int* cells);
-/* Algorithmic work of the last upload: hypotheses (fine + coarse) and gathered cells. */
+/* Algorithmic work of the last upload: hypotheses (fine + coarse) and gathered cells.  These count
+ * every hypothesis of each window, the window the result is exact over, also where the run prunes. */
 int lgs_rtcsm_batch_work(const lgs_rtcsm_batch* b, long long* hypotheses, long long* gathers);
+/* Diagnostic: fine tiles the last scoring pass of run (or of results' re-scoring) summed, and the tiles
+ * of the exhaustive sweep.  A tile is one warp's share of the row sweep: up to 32 x offsets, 4-5 window
+ * rows, 2 theta slices.  Windows of the flattened sweep (< 512 hypotheses) are never pruned; for them
+ * both counts are that sweep's warps.  Waits for the stream. */
+int lgs_rtcsm_batch_fine_tiles(lgs_rtcsm_batch* b, long long* scored, long long* total);
 /* Convenience: upload + run + results. */
 int lgs_rtcsm_match(lgs_ctx* ctx, const lgs_grid* grid, const lgs_grid* coarse,
                     const lgs_rtcsm_params* params, const lgs_scan_batch* scans,

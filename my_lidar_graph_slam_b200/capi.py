@@ -112,6 +112,7 @@ SIGNATURES = {
     "lgs_rtcsm_batch_results": (C.c_int, [vp, vp, vp, C.POINTER(MatchResult)]),
     "lgs_rtcsm_batch_debug": (C.c_int, [vp, C.c_int, c_ip, c_dp, c_dp, c_ip]),
     "lgs_rtcsm_batch_work": (C.c_int, [vp, C.POINTER(C.c_longlong), C.POINTER(C.c_longlong)]),
+    "lgs_rtcsm_batch_fine_tiles": (C.c_int, [vp, C.POINTER(C.c_longlong), C.POINTER(C.c_longlong)]),
     "lgs_rtcsm_match": (C.c_int, [vp, vp, vp, C.POINTER(RtcsmParams), C.POINTER(ScanBatch), c_dp,
                                   C.POINTER(MatchResult)]),
     "lgs_bb_batch_create": (C.c_int, [vp, C.POINTER(BbParams), C.POINTER(vp)]),
@@ -410,6 +411,12 @@ class RtcsmBatch:
         h, g = C.c_longlong(), C.c_longlong()
         self.ctx.check(lib().lgs_rtcsm_batch_work(self.h, C.byref(h), C.byref(g)))
         return h.value, g.value
+
+    def fine_tiles(self):
+        """-> (fine tiles the last scoring pass summed, tiles of the exhaustive sweep)."""
+        n, total = C.c_longlong(), C.c_longlong()
+        self.ctx.check(lib().lgs_rtcsm_batch_fine_tiles(self.h, C.byref(n), C.byref(total)))
+        return n.value, total.value
 
     def debug(self, m: int):
         dims = (C.c_int * 6)()

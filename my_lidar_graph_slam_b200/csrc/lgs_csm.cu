@@ -70,7 +70,8 @@ struct GridGeom {
 struct DevResult {
     double score;
     int found, ix, iy, it;
-    int exactReplay, pad;
+    int exactReplay;
+    int needFull;            // pruned select found a coarse score below its block: score every tile again
 };
 
 struct FlagEntry { int m, t, i; };
@@ -84,7 +85,8 @@ __global__ void csm_project_kernel(const CsmDesc* __restrict__ descs,
                                    const double* __restrict__ angles,
                                    const double* __restrict__ ranges, GridGeom g, CsmWindow w, double eps,
                                    int* __restrict__ offs, int2* __restrict__ cells,
-                                   FlagEntry* __restrict__ flags, int flagCap, int* __restrict__ flagCount) {
+                                   FlagEntry* __restrict__ flags, int flagCap, int* __restrict__ flagCount,
+                                   int* __restrict__ noBound) {
     const CsmDesc d = descs[blockIdx.y];
     const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= (long long)d.nT * d.nKeptPad) return;
@@ -118,6 +120,20 @@ __global__ void csm_project_kernel(const CsmDesc* __restrict__ descs,
     const int ccx = clampi(cx, -xHi - 1, g.nx - xLo);
     const int ccy = clampi(cy, -yHi - 1, g.ny - yLo);
     offs[d.offBegin + idx] = ccy * g.pitch + ccx;
+    // "coarse may not bound" (K2c): a coarse read of this point in (-lowRes, 0) on either axis
+    const int e = edge ? 1 : 0;
+    bool band = false;
+    for (int c = -e; c <= e; ++c) {
+        for (int bx = 0; bx < w.nbx; ++bx) {
+            const int rx = ccx + c - w.winX + bx * w.lowRes;
+            band |= rx > -w.lowRes && rx < 0;
+        }
+        for (int by = 0; by < w.nby; ++by) {
+            const int ry = ccy + c - w.winY + by * w.lowRes;
+            band |= ry > -w.lowRes && ry < 0;
+        }
+    }
+    if (band) noBound[blockIdx.y] = 1;
 }
 
 // ---- K2: the sweep (hot kernel) -------------------------------------------------------------------
@@ -241,65 +257,61 @@ __device__ __forceinline__ void load_theta_group(const int* s, int (&o)[TG]) {
     }
 }
 
-template <int UNROLL, int ROWS, int TG>
-__global__ void __launch_bounds__(256)
-csm_sweep_rows_kernel(const CsmDesc* __restrict__ descs, const double* __restrict__ fineGrid,
-                      const double* __restrict__ coarseGrid, int pitch, CsmWindow w,
-                      const int* __restrict__ offs, double* __restrict__ fineTab,
-                      double* __restrict__ coarseTab) {
-    extern __shared__ int sOff[];   // [beam][TG]
-    const CsmDesc d = descs[blockIdx.z];
-    const int t0 = blockIdx.y * TG;
-    if (t0 >= d.nT) return;
-    const int nTg = min(TG, d.nT - t0);   // valid slices of this group
-    {   // stage the group's offsets (nKeptPad is a multiple of 4 ints = 16 B)
-        const int n4 = d.nKeptPad / 4;
-        const int* src = offs + d.offBegin + (long long)t0 * d.nKeptPad;
-        for (int k = threadIdx.x; k < TG * n4; k += blockDim.x) {
-            const int t = k / n4, q = k - t * n4;
-            const int4 v = reinterpret_cast<const int4*>(src + (long long)min(t, nTg - 1) * d.nKeptPad)[q];
-            int* dst = sOff + 4 * q * TG + t;
-            dst[0] = v.x; dst[TG] = v.y; dst[2 * TG] = v.z; dst[3 * TG] = v.w;
-        }
+// Stages the offsets of slices t0 .. t0 + TG of match d into s ([beam][TG]); threads tid of nthr take part.
+template <int TG>
+__device__ __forceinline__ void stage_theta_group(const CsmDesc& d, const int* __restrict__ offs, int t0, int nTg,
+                                                  int* s, int tid, int nthr) {
+    const int n4 = d.nKeptPad / 4;   // nKeptPad is a multiple of 4 ints = 16 B
+    const int* src = offs + d.offBegin + (long long)t0 * d.nKeptPad;
+    for (int k = tid; k < TG * n4; k += nthr) {
+        const int t = k / n4, q = k - t * n4;
+        const int4 v = reinterpret_cast<const int4*>(src + (long long)min(t, nTg - 1) * d.nKeptPad)[q];
+        int* dst = s + 4 * q * TG + t;
+        dst[0] = v.x; dst[TG] = v.y; dst[2 * TG] = v.z; dst[3 * TG] = v.w;
     }
-    __syncthreads();
-    const int n = d.nKeptPad;   // multiple of kBeamPad >= UNROLL
+}
 
-    if (blockIdx.x >= (unsigned)w.tilesFine) {
-        // Coarse hypotheses (stride lowRes on the win-max map), one per thread, TG slices each.
-        // Only the equal-offset reuse applies: a thread holds a single row.
-        const int h = (blockIdx.x - w.tilesFine) * blockDim.x + threadIdx.x;
-        if (h >= w.nbx * w.nby) return;
-        const int oy = h / w.nbx, ox = h - oy * w.nbx;
-        const double* __restrict__ gp =
-            coarseGrid + (-w.winY + oy * w.lowRes) * pitch + (-w.winX + ox * w.lowRes);
-        double acc[TG];
+// Coarse hypothesis h (stride lowRes on the win-max map) of TG slices, beams in order.  Only the equal-offset
+// reuse applies: a thread holds a single row.
+template <int UNROLL, int TG>
+__device__ __forceinline__ void coarse_theta_group(const CsmDesc& d, const CsmWindow& w, const int* sOff,
+                                                   const double* __restrict__ coarseGrid, int pitch, int h, int t0,
+                                                   int nTg, double* __restrict__ coarseTab) {
+    const int n = d.nKeptPad;   // multiple of kBeamPad >= UNROLL
+    const int oy = h / w.nbx, ox = h - oy * w.nbx;
+    const double* __restrict__ gp =
+        coarseGrid + (-w.winY + oy * w.lowRes) * pitch + (-w.winX + ox * w.lowRes);
+    double acc[TG];
 #pragma unroll
-        for (int t = 0; t < TG; ++t) acc[t] = 0.0;
+    for (int t = 0; t < TG; ++t) acc[t] = 0.0;
 #pragma unroll 1
-        for (int i = 0; i < n; i += UNROLL) {
+    for (int i = 0; i < n; i += UNROLL) {
 #pragma unroll
-            for (int u = 0; u < UNROLL; ++u) {
-                int o[TG];
-                load_theta_group<TG>(sOff + (i + u) * TG, o);
-                double v = __ldg(gp + o[0]);
-                acc[0] = __dadd_rn(acc[0], v);
+        for (int u = 0; u < UNROLL; ++u) {
+            int o[TG];
+            load_theta_group<TG>(sOff + (i + u) * TG, o);
+            double v = __ldg(gp + o[0]);
+            acc[0] = __dadd_rn(acc[0], v);
 #pragma unroll
-                for (int t = 1; t < TG; ++t) {
-                    if (o[t] != o[t - 1]) v = __ldg(gp + o[t]);
-                    acc[t] = __dadd_rn(acc[t], v);
-                }
+            for (int t = 1; t < TG; ++t) {
+                if (o[t] != o[t - 1]) v = __ldg(gp + o[t]);
+                acc[t] = __dadd_rn(acc[t], v);
             }
         }
-#pragma unroll
-        for (int t = 0; t < TG; ++t)
-            if (t < nTg) coarseTab[d.coarseBegin + ((long long)(t0 + t) * w.nbx + ox) * w.nby + oy] = acc[t];
-        return;
     }
+#pragma unroll
+    for (int t = 0; t < TG; ++t)
+        if (t < nTg) coarseTab[d.coarseBegin + ((long long)(t0 + t) * w.nbx + ox) * w.nby + oy] = acc[t];
+}
 
-    const int wg = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+// Fine rows of warp wg (x chunk wg % xChunks, row group wg / xChunks) of one theta group; lane = x in the chunk.
+template <int UNROLL, int ROWS, int TG>
+__device__ __forceinline__ void fine_theta_group(const CsmDesc& d, const CsmWindow& w, const int* sOff,
+                                                 const double* __restrict__ fineGrid, int pitch, int wg, int lane,
+                                                 int t0, int nTg, double* __restrict__ fineTab) {
+    const int n = d.nKeptPad;   // multiple of kBeamPad >= UNROLL
     const int xc = wg % w.xChunks, rg = wg / w.xChunks;
-    const int ox = xc * 32 + (threadIdx.x & 31);
+    const int ox = xc * 32 + lane;
     if (rg >= w.rowGroups || ox >= w.nxw) return;
     const int oy0 = rg * ROWS;
     const double* __restrict__ gp = fineGrid + (-w.winY + oy0) * pitch + (-w.winX + ox);
@@ -366,12 +378,197 @@ csm_sweep_rows_kernel(const CsmDesc* __restrict__ descs, const double* __restric
                 fineTab[d.fineBegin + ((long long)(t0 + t) * w.nyw + oy0 + k) * w.nxw + ox] = acc[t][k];
 }
 
+// The exhaustive row sweep: grid = (tilesFine + tilesCoarse, theta groups, matches).  It fills the whole fine
+// and coarse tables; lgs_rtcsm_batch_debug runs it to return them after a pruned run.
+template <int UNROLL, int ROWS, int TG>
+__global__ void __launch_bounds__(256)
+csm_sweep_rows_kernel(const CsmDesc* __restrict__ descs, const double* __restrict__ fineGrid,
+                      const double* __restrict__ coarseGrid, int pitch, CsmWindow w,
+                      const int* __restrict__ offs, double* __restrict__ fineTab,
+                      double* __restrict__ coarseTab) {
+    extern __shared__ int sOff[];   // [beam][TG]
+    const CsmDesc d = descs[blockIdx.z];
+    const int t0 = blockIdx.y * TG;
+    if (t0 >= d.nT) return;
+    const int nTg = min(TG, d.nT - t0);   // valid slices of this group
+    stage_theta_group<TG>(d, offs, t0, nTg, sOff, threadIdx.x, blockDim.x);
+    __syncthreads();
+    if (blockIdx.x >= (unsigned)w.tilesFine) {
+        const int h = (blockIdx.x - w.tilesFine) * blockDim.x + threadIdx.x;
+        if (h < w.nbx * w.nby) coarse_theta_group<UNROLL, TG>(d, w, sOff, coarseGrid, pitch, h, t0, nTg, coarseTab);
+        return;
+    }
+    fine_theta_group<UNROLL, ROWS, TG>(d, w, sOff, fineGrid, pitch, blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5),
+                                       threadIdx.x & 31, t0, nTg, fineTab);
+}
+
+// ---- K2c: the pruned sweep of row-mapped windows ------------------------------------------------------
+// The reference scores a fine block only when its coarse score beats the running best, so its answer depends
+// only on blocks with C[b] >= F* (F* = the match's best fine score) whenever every coarse score bounds its
+// block.  The device therefore scores every coarse hypothesis (csm_coarse_kernel), takes a lower bound L <= F*
+// from the fine blocks of the kSeedBlocks best coarse blocks (csm_prune_kernel), and scores only the warp tiles
+// (theta group x warp of the row sweep) that hold a block with C[b] >= L and C[b] > thrAbs
+// (csm_sweep_tiles_kernel).  Matches whose projection may break the bound (csm_project_kernel's noBound flag)
+// get every tile, and csm_select_kernel treats them as it treats the exhaustive tables.
+//
+// Why C[b] >= F[b] holds for every block of an unflagged match: C[b] and each fine score of block b are sums
+// over the same beams in the same order, of coarse[p + o_b] and of fine[p + o_b + f] (0 <= f.x, f.y < L).
+// IEEE addition is monotone, so termwise coarse >= fine gives C >= F bit for bit.  coarse is the win-max of
+// fine over [c, c + L) on each axis (lgs_precompute), with the window moved to [n - L, n) at the upper map
+// edge, which still covers every in-map cell of [c, c + L); cells past the map read the zero apron on both
+// maps.  The one failure is a coarse index c in (-L, 0) on either axis: it reads 0 while fine cells
+// c + f >= 0 are in the map (SURVEY.md H12).  The projection flags every kept beam whose clamped cell plus a
+// block origin falls there (clamping keeps out-of-window points at c <= -L, so they never reach the band).
+// Near-edge points, which results() may re-derive one cell away on the host, are tested at cell +- 1.
+constexpr int kSeedBlocks = 4;       // coarse blocks whose fine blocks give the bound L
+constexpr int kPruneThreads = 128;   // csm_prune_kernel block
+constexpr int kTilesWarps = 4;       // csm_sweep_tiles_kernel warps per block
+
+// One warp per (theta group, match): grid = (theta groups, matches).
+template <int UNROLL, int TG>
+__global__ void __launch_bounds__(32)
+csm_coarse_kernel(const CsmDesc* __restrict__ descs, const double* __restrict__ coarseGrid, int pitch, CsmWindow w,
+                  const int* __restrict__ offs, double* __restrict__ coarseTab) {
+    extern __shared__ int sOff[];   // [beam][TG]
+    const CsmDesc d = descs[blockIdx.y];
+    const int t0 = blockIdx.x * TG;
+    if (t0 >= d.nT) return;
+    const int nTg = min(TG, d.nT - t0);
+    stage_theta_group<TG>(d, offs, t0, nTg, sOff, threadIdx.x, 32);
+    __syncwarp();
+    for (int h = threadIdx.x; h < w.nbx * w.nby; h += 32)
+        coarse_theta_group<UNROLL, TG>(d, w, sOff, coarseGrid, pitch, h, t0, nTg, coarseTab);
+}
+
+// (c, v) beats (bc, bv) in the order (score desc, visit asc)
+__device__ __forceinline__ bool csm_before(double c, int v, double bc, int bv) {
+    return c > bc || (c == bc && v < bv);
+}
+
+// Block-wide (score desc, visit asc) minimum of every thread's (c, v); every thread gets it.
+__device__ void csm_block_best(double& c, int& v, double* sC, int* sV) {
+    __syncthreads();
+    sC[threadIdx.x] = c; sV[threadIdx.x] = v;
+    __syncthreads();
+    for (int s = blockDim.x / 2; s > 0; s >>= 1) {
+        if (threadIdx.x < s && csm_before(sC[threadIdx.x + s], sV[threadIdx.x + s], sC[threadIdx.x], sV[threadIdx.x])) {
+            sC[threadIdx.x] = sC[threadIdx.x + s];
+            sV[threadIdx.x] = sV[threadIdx.x + s];
+        }
+        __syncthreads();
+    }
+    c = sC[0]; v = sV[0];
+}
+
+__device__ __forceinline__ bool csm_keep(double c, double bound, double thrAbs) { return c >= bound && c > thrAbs; }
+
+// One block per match.  Seed: the kSeedBlocks best coarse blocks in (C desc, visit asc) order; their fine
+// 5x5 (lowRes x lowRes) blocks are summed in beam order like the sweep, so L = their maximum is a fine score
+// of the window and L <= F*.  Keep: C[b] >= L (a tie with F* at an earlier visit must be scored) and
+// C[b] > thrAbs (no block at or below the threshold can make the match found).  Every warp tile of the row
+// sweep that holds a kept block of one of its slices goes to the work list; a flagged match lists them all.
+__global__ void __launch_bounds__(kPruneThreads)
+csm_prune_kernel(const CsmDesc* __restrict__ descs, const double* __restrict__ fineGrid, int pitch, CsmWindow w,
+                 const int* __restrict__ offs, const double* __restrict__ coarseTab,
+                 const int* __restrict__ noBound, double* __restrict__ bound, int tileG, int2* __restrict__ tiles,
+                 int* __restrict__ tileCount) {
+    __shared__ double sC[kPruneThreads];
+    __shared__ int sV[kPruneThreads];
+    const int m = blockIdx.x;
+    const CsmDesc d = descs[m];
+    const int nbxy = w.nbx * w.nby, nB = d.nT * nbxy;
+    const double* C = coarseTab + d.coarseBegin;
+    const bool full = noBound[m] != 0;
+    double L = -INFINITY;
+    if (!full) {
+        int seed[kSeedBlocks];
+        double pc = INFINITY;
+        int pv = -1;
+#pragma unroll
+        for (int k = 0; k < kSeedBlocks; ++k) {   // k-th best: the best of those after the (k-1)-th
+            double bc = -INFINITY;
+            int bv = 0x7fffffff;
+            for (int v = threadIdx.x; v < nB; v += blockDim.x) {
+                const double c = C[v];
+                if (csm_before(pc, pv, c, v) && csm_before(c, v, bc, bv)) { bc = c; bv = v; }
+            }
+            csm_block_best(bc, bv, sC, sV);
+            seed[k] = bv < nB ? bv : -1;
+            pc = bc; pv = bv;
+        }
+        const int cells = w.lowRes * w.lowRes;
+        double best = -INFINITY;
+        for (int p = threadIdx.x; p < kSeedBlocks * cells; p += blockDim.x) {
+            int v = -1;
+#pragma unroll
+            for (int k = 0; k < kSeedBlocks; ++k) if (p / cells == k) v = seed[k];
+            if (v < 0) continue;
+            const int t = v / nbxy, bx = (v / w.nby) % w.nbx, by = v % w.nby;
+            const int f = p % cells;
+            const double* __restrict__ gp = fineGrid + (-w.winY + by * w.lowRes + f % w.lowRes) * pitch +
+                                            (-w.winX + bx * w.lowRes + f / w.lowRes);
+            const int* __restrict__ o = offs + d.offBegin + (long long)t * d.nKeptPad;
+            double acc = 0.0;
+#pragma unroll 4
+            for (int i = 0; i < d.nKeptPad; ++i) acc = __dadd_rn(acc, __ldg(gp + __ldg(o + i)));   // beam order
+            best = fmax(best, acc);
+        }
+        int dummy = 0;
+        csm_block_best(best, dummy, sC, sV);
+        L = best;
+    }
+    if (threadIdx.x == 0) bound[m] = L;
+    const int wpt = w.xChunks * w.rowGroups;        // warps per slice group
+    const int nG = (d.nT + tileG - 1) / tileG;
+    for (int p = threadIdx.x; p < nG * wpt; p += blockDim.x) {
+        const int g = p / wpt, wg = p - g * wpt;
+        bool need = full;
+        if (!need) {
+            const int xc = wg % w.xChunks, rg = wg / w.xChunks;
+            const int x0 = xc * 32, x1 = min(x0 + 32, w.nxw) - 1;
+            const int y0 = rg * w.rows, y1 = min(y0 + w.rows, w.nyw) - 1;
+            for (int t = g * tileG; t < min(d.nT, (g + 1) * tileG) && !need; ++t)
+                for (int bx = x0 / w.lowRes; bx <= x1 / w.lowRes && !need; ++bx)
+                    for (int by = y0 / w.lowRes; by <= y1 / w.lowRes && !need; ++by)
+                        need = csm_keep(C[(t * w.nbx + bx) * w.nby + by], L, d.thrAbs);
+        }
+        if (need) tiles[atomicAdd(tileCount, 1)] = make_int2(m, p);
+    }
+}
+
+// Grid-stride over the work list, one tile per warp; each warp stages its own group's offsets.
+template <int UNROLL, int ROWS, int TG>
+__global__ void __launch_bounds__(kTilesWarps * 32)
+csm_sweep_tiles_kernel(const CsmDesc* __restrict__ descs, const double* __restrict__ fineGrid, int pitch,
+                       CsmWindow w, const int* __restrict__ offs, const int2* __restrict__ tiles,
+                       const int* __restrict__ tileCount, int warpSmem, double* __restrict__ fineTab) {
+    extern __shared__ int sAll[];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, wpb = blockDim.x >> 5;
+    int* sOff = sAll + warp * warpSmem;
+    const int n = *tileCount;
+    const int wpt = w.xChunks * w.rowGroups;
+    for (int k = blockIdx.x * wpb + warp; k < n; k += gridDim.x * wpb) {
+        const int2 tile = tiles[k];
+        const CsmDesc d = descs[tile.x];
+        const int g = tile.y / wpt, wg = tile.y - g * wpt;
+        const int t0 = g * TG, nTg = min(TG, d.nT - t0);
+        __syncwarp();   // the previous tile's reads of sOff are done
+        stage_theta_group<TG>(d, offs, t0, nTg, sOff, lane, 32);
+        __syncwarp();
+        fine_theta_group<UNROLL, ROWS, TG>(d, w, sOff, fineGrid, pitch, wg, lane, t0, nTg, fineTab);
+    }
+}
+
 // ---- K3: block maxima + CPU-order selection -----------------------------------------------------
-// One thread block per match.
+// One thread block per match.  After the pruned sweep (noBound != nullptr) an unflagged match considers only
+// the kept blocks: the others were not scored, and every one of them is below F* or at most the threshold.
+// Should a kept block still show C < F there (a coarse map that is not lgs_precompute's win-max of the grid),
+// the match is flagged and marked needFull, and results() scores it again with every tile.
 __global__ void __launch_bounds__(256)
 csm_select_kernel(const CsmDesc* __restrict__ descs, CsmWindow w,
                   const double* __restrict__ fineTab, const double* __restrict__ coarseTab,
                   double* __restrict__ blockMax, int* __restrict__ blockArg,
+                  int* __restrict__ noBound, const double* __restrict__ bound,
                   DevResult* __restrict__ results) {
     const CsmDesc d = descs[blockIdx.x];
     const int nB = d.nT * w.nbx * w.nby;
@@ -379,6 +576,8 @@ csm_select_kernel(const CsmDesc* __restrict__ descs, CsmWindow w,
     int* A = blockArg + d.coarseBegin;
     const double* C = coarseTab + d.coarseBegin;
     const double* fine = fineTab + d.fineBegin;
+    const bool pruned = noBound && !noBound[blockIdx.x];
+    const double L = pruned ? bound[blockIdx.x] : 0.0;
     __shared__ int sInvalid;
     __shared__ double sBest[256];
     __shared__ int sIdx[256];
@@ -391,6 +590,7 @@ csm_select_kernel(const CsmDesc* __restrict__ descs, CsmWindow w,
     int myIdx = 0x7fffffff;
     bool invalid = false;
     for (int v = threadIdx.x; v < nB; v += blockDim.x) {
+        if (pruned && !csm_keep(C[v], L, d.thrAbs)) continue;
         const int by = v % w.nby;
         const int bx = (v / w.nby) % w.nbx;
         const int t = v / (w.nby * w.nbx);
@@ -413,7 +613,16 @@ csm_select_kernel(const CsmDesc* __restrict__ descs, CsmWindow w,
     __syncthreads();
 
     DevResult r;
-    r.pad = 0;
+    r.needFull = 0;
+    if (sInvalid && pruned) {
+        if (threadIdx.x != 0) return;
+        noBound[blockIdx.x] = 1;
+        r.needFull = 1; r.exactReplay = 0;
+        r.found = 0; r.score = d.thrAbs;
+        r.ix = -w.winX; r.iy = -w.winY; r.it = -d.winT;
+        results[blockIdx.x] = r;
+        return;
+    }
     if (!sInvalid) {
         // Every C[v] >= F[v]: the pruned CPU loop returns the first visit of the global maximum.
         for (int s = blockDim.x / 2; s > 0; s >>= 1) {
@@ -518,6 +727,16 @@ struct lgs_rtcsm_batch {
     PinBuf<int> hFlagCount;
     PinBuf<CsmDesc> hDescs;
     PinBuf<double> hStage;
+    // pruned sweep of row-mapped windows (K2c)
+    long long nTilesAll = 0;                     // warp tiles of the exhaustive fine sweep
+    int tilesGrid = 0;                           // csm_sweep_tiles_kernel blocks (all resident)
+    size_t tilesSmem = 0;
+    bool tablesFull = false;                     // dFine / dCoarse hold every hypothesis of every match
+    const lgs_grid* lastGrid = nullptr;          // maps of the last run (debug() re-scores against them)
+    const lgs_grid* lastCoarse = nullptr;
+    DevBuf<int> dNoBound, dTileCount;
+    DevBuf<double> dBound;
+    DevBuf<int2> dTiles;
     bool uploaded = false, ran = false;
 };
 
@@ -548,21 +767,64 @@ static int csm_launch_sweep(lgs_rtcsm_batch* b, const lgs_grid* grid, const lgs_
                 b->dFine.p, b->dCoarse.p);
         LGS_LAUNCH_CHECK(c);
     }
+    b->tablesFull = true;
+    return LGS_OK;
+}
+
+// Steps 2-5 of a run (coarse scores, bound, work list, fine scores): the exhaustive sweep for windows of the
+// flattened sweep, the pruned chain (K2c) for row-mapped ones.  Stream ordered, no host synchronisation.
+static int csm_launch_score(lgs_rtcsm_batch* b, const lgs_grid* grid, const lgs_grid* coarse) {
+    const CsmWindow& w = b->win;
+    if (!w.rows) return csm_launch_sweep(b, grid, coarse);
+    lgs_ctx* c = b->ctx;
+    LGS_CUDA(c, cudaMemsetAsync(b->dTileCount.p, 0, sizeof(int), c->stream));
+    const int nG = (b->maxNT + kThetaGroup - 1) / kThetaGroup;
+    for (int m0 = 0; m0 < b->nMatch; m0 += 65535) {
+        const int nm = std::min(65535, b->nMatch - m0);
+        csm_coarse_kernel<kRowsUnroll, kThetaGroup><<<dim3(nG, nm), 32, b->sweepSmem, c->stream>>>(
+            b->dDescs.p + m0, coarse->origin(), grid->pitch, w, b->dOffs.p, b->dCoarse.p);
+        LGS_LAUNCH_CHECK(c);
+    }
+    csm_prune_kernel<<<b->nMatch, kPruneThreads, 0, c->stream>>>(
+        b->dDescs.p, grid->origin(), grid->pitch, w, b->dOffs.p, b->dCoarse.p, b->dNoBound.p, b->dBound.p,
+        kThetaGroup, b->dTiles.p, b->dTileCount.p);
+    LGS_LAUNCH_CHECK(c);
+    const int warpSmem = kThetaGroup * b->maxKeptPad;
+    if (w.rows == 5)
+        csm_sweep_tiles_kernel<kRowsUnroll, 5, kThetaGroup><<<b->tilesGrid, kTilesWarps * 32, b->tilesSmem, c->stream>>>(
+            b->dDescs.p, grid->origin(), grid->pitch, w, b->dOffs.p, b->dTiles.p, b->dTileCount.p, warpSmem,
+            b->dFine.p);
+    else
+        csm_sweep_tiles_kernel<kRowsUnroll, 4, kThetaGroup><<<b->tilesGrid, kTilesWarps * 32, b->tilesSmem, c->stream>>>(
+            b->dDescs.p, grid->origin(), grid->pitch, w, b->dOffs.p, b->dTiles.p, b->dTileCount.p, warpSmem,
+            b->dFine.p);
+    LGS_LAUNCH_CHECK(c);
+    b->tablesFull = false;
     return LGS_OK;
 }
 
 static int csm_launch_select(lgs_rtcsm_batch* b) {
     lgs_ctx* c = b->ctx;
+    const bool pruned = b->win.rows != 0;
     csm_select_kernel<<<b->nMatch, 256, 0, c->stream>>>(b->dDescs.p, b->win, b->dFine.p,
                                                         b->dCoarse.p, b->dBlockMax.p,
-                                                        b->dBlockArg.p, b->dResults.p);
+                                                        b->dBlockArg.p, pruned ? b->dNoBound.p : nullptr,
+                                                        b->dBound.p, b->dResults.p);
     LGS_LAUNCH_CHECK(c);
     return LGS_OK;
 }
 
-static int csm_launch_sweep_select(lgs_rtcsm_batch* b, const lgs_grid* grid, const lgs_grid* coarse) {
-    const int rc = csm_launch_sweep(b, grid, coarse);
-    return rc != LGS_OK ? rc : csm_launch_select(b);
+// Scores and selects again (after near-edge fix-ups, or for matches the select marked needFull) and waits for
+// the result records.
+static int csm_rescore_results(lgs_rtcsm_batch* b, const lgs_grid* grid, const lgs_grid* coarse) {
+    lgs_ctx* c = b->ctx;
+    int rc = csm_launch_score(b, grid, coarse);
+    if (rc == LGS_OK) rc = csm_launch_select(b);
+    if (rc != LGS_OK) return rc;
+    LGS_CUDA(c, cudaMemcpyAsync(b->hResults.p, b->dResults.p, b->nMatch * sizeof(DevResult),
+                                cudaMemcpyDeviceToHost, c->stream));
+    LGS_CUDA(c, cudaStreamSynchronize(c->stream));
+    return LGS_OK;
 }
 
 extern "C" {
@@ -587,6 +849,7 @@ int lgs_rtcsm_batch_destroy(lgs_rtcsm_batch* b) {
     b->dCoarse.release(); b->dBlockMax.release(); b->dOffs.release(); b->dBlockArg.release();
     b->dFlagCount.release(); b->dCells.release(); b->dFlags.release(); b->dResults.release();
     b->dFixOff.release(); b->dFixCell.release(); b->dFixWhere.release();
+    b->dNoBound.release(); b->dTileCount.release(); b->dBound.release(); b->dTiles.release();
     b->hResults.release(); b->hFlagCount.release(); b->hDescs.release(); b->hStage.release();
     delete b;
     return LGS_OK;
@@ -649,7 +912,7 @@ int lgs_rtcsm_batch_upload(lgs_rtcsm_batch* b, const lgs_grid* grid, const lgs_s
     b->hAngles.clear(); b->hRanges.clear();
     b->maxNT = 0; b->maxKeptPad = kBeamPad;
     long long nOff = 0, nCell = 0, nFine = 0, nCoarse = 0;
-    b->workHyp = 0; b->workGather = 0;
+    b->workHyp = 0; b->workGather = 0; b->nTilesAll = 0;
     for (int m = 0; m < n; ++m) {
         const int b0 = scans->beam_begin[m], b1 = scans->beam_begin[m + 1];
         const int nb = b1 - b0;
@@ -688,6 +951,8 @@ int lgs_rtcsm_batch_upload(lgs_rtcsm_batch* b, const lgs_grid* grid, const lgs_s
         const long long hyp = (long long)d.nT * ((long long)w.nxw * w.nyw + (long long)w.nbx * w.nby);
         b->workHyp += hyp;
         b->workGather += hyp * d.nKept;
+        b->nTilesAll += w.rows ? (long long)((d.nT + kThetaGroup - 1) / kThetaGroup) * w.xChunks * w.rowGroups
+                               : (long long)d.nT * (w.slots / 32);
     }
     if (b->maxNT > 65535)
         return lgs_fail(c, LGS_ERR_INVALID, "rtcsm: %d theta slices exceed the launch grid", b->maxNT);
@@ -711,6 +976,10 @@ int lgs_rtcsm_batch_upload(lgs_rtcsm_batch* b, const lgs_grid* grid, const lgs_s
     LGS_CUDA(c, b->dFlagCount.reserve(1));
     LGS_CUDA(c, b->dFlags.reserve(b->flagCap));
     LGS_CUDA(c, b->dResults.reserve(n));
+    LGS_CUDA(c, b->dNoBound.reserve(n));
+    LGS_CUDA(c, b->dBound.reserve(n));
+    LGS_CUDA(c, b->dTileCount.reserve(1));
+    if (w.rows) LGS_CUDA(c, b->dTiles.reserve(b->nTilesAll));
     LGS_CUDA(c, b->hResults.reserve(n));
     LGS_CUDA(c, b->hFlagCount.reserve(1));
     LGS_CUDA(c, b->hDescs.reserve(n));
@@ -742,12 +1011,32 @@ int lgs_rtcsm_batch_upload(lgs_rtcsm_batch* b, const lgs_grid* grid, const lgs_s
                                              cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
         }
     }
+    if (w.rows) {
+        // coarse kernel: one group's offsets per block, like the exhaustive sweep; tiles kernel: one per warp
+        b->tilesSmem = (size_t)kTilesWarps * b->sweepSmem;
+        if (b->sweepSmem > 48 * 1024)
+            LGS_CUDA(c, cudaFuncSetAttribute(csm_coarse_kernel<kRowsUnroll, kThetaGroup>,
+                                             cudaFuncAttributeMaxDynamicSharedMemorySize, (int)b->sweepSmem));
+        const auto tilesKernel = w.rows == 5 ? csm_sweep_tiles_kernel<kRowsUnroll, 5, kThetaGroup>
+                                             : csm_sweep_tiles_kernel<kRowsUnroll, 4, kThetaGroup>;
+        if (b->tilesSmem > 48 * 1024)
+            LGS_CUDA(c, cudaFuncSetAttribute(tilesKernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                             (int)b->tilesSmem));
+        int perSm = 0;
+        LGS_CUDA(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSm, tilesKernel, kTilesWarps * 32,
+                                                                  b->tilesSmem));
+        if (perSm < 1)
+            return lgs_fail(c, LGS_ERR_INVALID, "rtcsm: %d beams leave no room for the pruned sweep", b->maxKeptPad);
+        b->tilesGrid = (int)std::min<long long>((long long)perSm * c->sm_count,
+                                                (b->nTilesAll + kTilesWarps - 1) / kTilesWarps);
+    }
     b->uploaded = true;
     return LGS_OK;
 }
 
 static int csm_launch_project(lgs_rtcsm_batch* b) {
     lgs_ctx* c = b->ctx;
+    LGS_CUDA(c, cudaMemsetAsync(b->dNoBound.p, 0, b->nMatch * sizeof(int), c->stream));
     for (int m0 = 0; m0 < b->nMatch; m0 += 65535) {
         const int nm = std::min(65535, b->nMatch - m0);
         const long long per = (long long)b->maxNT * b->maxKeptPad;
@@ -755,7 +1044,7 @@ static int csm_launch_project(lgs_rtcsm_batch* b) {
         csm_project_kernel<<<gridDim, 256, 0, c->stream>>>(b->dDescs.p + m0, b->dAngles.p,
                                                            b->dRanges.p, b->geom, b->win,
                                                            c->opt.edgeEps, b->dOffs.p, b->dCells.p, b->dFlags.p,
-                                                           b->flagCap, b->dFlagCount.p);
+                                                           b->flagCap, b->dFlagCount.p, b->dNoBound.p + m0);
         LGS_LAUNCH_CHECK(c);
     }
     return LGS_OK;
@@ -780,7 +1069,8 @@ static int csm_run_impl(lgs_rtcsm_batch* b, const lgs_grid* grid, const lgs_grid
     int rc = csm_launch_project(b);
     if (rc != LGS_OK) return rc;
     if (ms) LGS_CUDA(c, cudaEventRecord(ev[1], c->stream));
-    rc = csm_launch_sweep(b, grid, coarse);
+    b->lastGrid = grid; b->lastCoarse = coarse;
+    rc = csm_launch_score(b, grid, coarse);
     if (rc != LGS_OK) return rc;
     if (ms) LGS_CUDA(c, cudaEventRecord(ev[2], c->stream));
     rc = csm_launch_select(b);
@@ -871,13 +1161,16 @@ int lgs_rtcsm_batch_results(lgs_rtcsm_batch* b, const lgs_grid* grid, const lgs_
         csm_patch_kernel<<<(nFlag + 127) / 128, 128, 0, c->stream>>>(nullptr, dOffVal, dCellVal, dWhere,
                                                                      nFlag, b->dOffs.p, b->dCells.p);
         LGS_LAUNCH_CHECK(c);
-        const int rc = csm_launch_sweep_select(b, grid, coarse);
+        const int rc = csm_rescore_results(b, grid, coarse);
         if (rc != LGS_OK) return rc;
-        LGS_CUDA(c, cudaMemcpyAsync(b->hResults.p, b->dResults.p, b->nMatch * sizeof(DevResult),
-                                    cudaMemcpyDeviceToHost, c->stream));
-        LGS_CUDA(c, cudaStreamSynchronize(c->stream));
         // The patched offsets stay valid for a re-run of results(); a new run() re-projects.
         LGS_CUDA(c, cudaMemsetAsync(b->dFlagCount.p, 0, sizeof(int), c->stream));
+    }
+    bool needFull = false;
+    for (int m = 0; m < b->nMatch; ++m) needFull |= b->hResults.p[m].needFull != 0;
+    if (needFull) {   // the select flagged those matches: this pass scores all of their tiles
+        const int rc = csm_rescore_results(b, grid, coarse);
+        if (rc != LGS_OK) return rc;
     }
     for (int m = 0; m < b->nMatch; ++m) {
         const DevResult& r = b->hResults.p[m];
@@ -901,6 +1194,12 @@ int lgs_rtcsm_batch_debug(lgs_rtcsm_batch* b, int m, int* dims, double* fine, do
     lgs_ctx* c = b->ctx;
     if (!b->ran) return lgs_fail(c, LGS_ERR_INVALID, "rtcsm_batch_debug before run");
     LGS_CUDA(c, cudaSetDevice(c->device));
+    if ((fine || coarse) && !b->tablesFull) {   // after a pruned run: fill both tables with the exhaustive sweep
+        LGS_CUDA(c, lgs_grid_acquire(c, b->lastGrid));
+        LGS_CUDA(c, lgs_grid_acquire(c, b->lastCoarse));
+        const int rc = csm_launch_sweep(b, b->lastGrid, b->lastCoarse);
+        if (rc != LGS_OK) return rc;
+    }
     LGS_CUDA(c, cudaStreamSynchronize(c->stream));
     const CsmDesc& d = b->descs[m];
     const CsmWindow& w = b->win;
@@ -921,6 +1220,23 @@ int lgs_rtcsm_batch_work(const lgs_rtcsm_batch* b, long long* hyp, long long* ga
     if (!b) return LGS_ERR_INVALID;
     if (hyp) *hyp = b->workHyp;
     if (gathers) *gathers = b->workGather;
+    return LGS_OK;
+}
+
+int lgs_rtcsm_batch_fine_tiles(lgs_rtcsm_batch* b, long long* scored, long long* total) {
+    if (!b) return LGS_ERR_INVALID;
+    lgs_ctx* c = b->ctx;
+    if (!b->ran) return lgs_fail(c, LGS_ERR_INVALID, "rtcsm_batch_fine_tiles before run");
+    long long n = b->nTilesAll;
+    if (b->win.rows && b->nMatch > 0) {
+        LGS_CUDA(c, cudaSetDevice(c->device));
+        int k = 0;
+        LGS_CUDA(c, cudaMemcpyAsync(&k, b->dTileCount.p, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+        LGS_CUDA(c, cudaStreamSynchronize(c->stream));
+        n = k;
+    }
+    if (scored) *scored = n;
+    if (total) *total = b->nTilesAll;
     return LGS_OK;
 }
 
