@@ -9,6 +9,8 @@ csrc/lgs_csm.cu) on the reference's own score tables.
 
 The model must return the reference's answer, every match where a coarse score fails to bound its block
 must be flagged, and on the bench's C2 workload the scored tiles are a small part of the exhaustive sweep."""
+import math
+
 import numpy as np
 
 from my_lidar_graph_slam_b200 import synth
@@ -30,13 +32,34 @@ def _blocks(fine, coarse, L):
     return F, C, A
 
 
-def flagged(cells, win_x, win_y, nxw, nyw, L, nx, ny):
-    """csm_project_kernel's 'coarse may not bound' flag from projected cells [t][beam][2] (kept beams)."""
+def near_edge(pose, angles, ranges, step_t, win_t, min_x, min_y, res, eps):
+    """csm_project_kernel's near-edge test [t][beam] for kept beams: the projected point's fractional cell
+    lies within eps of a cell edge on either axis.  The projection's operation order, with the host's libm
+    (the device's sincos can differ by an ulp, which matters only within an ulp of the band's limits)."""
+    out = np.zeros((2 * win_t + 1, len(ranges)), bool)
+    for t in range(2 * win_t + 1):
+        theta = pose[2] + step_t * (t - win_t)
+        for i, (a, r) in enumerate(zip(angles, ranges)):
+            qx = (pose[0] + r * math.cos(theta + a) - min_x) / res
+            qy = (pose[1] + r * math.sin(theta + a) - min_y) / res
+            fx, fy = qx - math.floor(qx), qy - math.floor(qy)
+            out[t, i] = not (eps <= fx <= 1.0 - eps and eps <= fy <= 1.0 - eps)
+    return out
+
+
+def flagged(cells, win_x, win_y, nxw, nyw, L, nx, ny, edge=None):
+    """csm_project_kernel's 'coarse may not bound' flag from projected cells [t][beam][2] (kept beams).
+    Near-edge points (edge [t][beam], from near_edge) are tested at their clamped cell and one cell either
+    side, since results() may re-derive them one cell away."""
     cx = np.clip(cells[..., 0].astype(np.int64), win_x - nxw, nx + win_x)
     cy = np.clip(cells[..., 1].astype(np.int64), win_y - nyw, ny + win_y)
-    rx = cx[..., None] - win_x + L * np.arange(nxw // L)
-    ry = cy[..., None] - win_y + L * np.arange(nyw // L)
-    return bool((((rx > -L) & (rx < 0)).any()) or (((ry > -L) & (ry < 0)).any()))
+    band = False
+    for s in ((0,) if edge is None else (-1, 0, 1)):
+        use = np.ones(cx.shape, bool) if s == 0 else edge
+        rx = cx[..., None] + s - win_x + L * np.arange(nxw // L)
+        ry = cy[..., None] + s - win_y + L * np.arange(nyw // L)
+        band |= bool((((rx > -L) & (rx < 0)).any(-1) & use).any() or (((ry > -L) & (ry < 0)).any(-1) & use).any())
+    return band
 
 
 def prune(F, C, thr, k=K):
@@ -146,6 +169,58 @@ def test_model_flags_the_lower_edge_and_replays_it():
         flags += flag
         unbounded += not bounded
     assert unbounded > 0 and flags >= unbounded
+
+
+def band_edge_scene(rng, n_matches=6):
+    """Scans whose lowest projected cells sit one cell above the band (-lowRes, 0) of coarse indices at the
+    lower map edge: row 5 with lowRes 5 and winY 10 (5 - 10 + 5 = 0); every other cell has row and column
+    >= 10 in every theta slice.  The row-5 points lie mid-cell in even matches and within 0.3 of their cell's
+    lower edge in odd ones, where the +-1 test of near-edge points (edge_eps 0.3) reaches row 4, in the band
+(their x fractions stay mid-cell: the +-1 test shifts both axes of a point near an edge on either).
+    -> (dense, min_x, min_y, [(angles, ranges, init)], params)."""
+    n, mx, my, res = 128, -1.0, -2.0, 0.05
+    # the map: strong cells along the lower edge and at the other points of every scan, zero elsewhere, so the
+    # scans fit one pose and the pruned sweep of an unflagged match skips most tiles
+    ux, uy = rng.uniform(15.0, 100.0, 157), rng.uniform(15.0, 100.0, 157)
+    dense = np.zeros((n, n))
+    dense[:12, :] = rng.uniform(0.5, 0.99, (12, n))
+    dense[uy.astype(int), ux.astype(int)] = 0.9
+    params = dict(low_res=5, range_x=1.0, range_y=1.0, range_theta=0.02, scan_range_max=20.0)
+    ins = []
+    for k in range(n_matches):
+        cx, th = 40 + int(rng.integers(-2, 3)), rng.uniform(-0.05, 0.05)
+        sx, sy = mx + (cx + 0.5) * res, my + 12.5 * res
+        f = 0.5 if k % 2 == 0 else 0.15          # the rotation of the slices moves row-5 points < 0.15 cell
+        line = np.stack([mx + (cx + rng.integers(-3, 4, 24) + 0.5) * res, np.full(24, my + (5 + f) * res)], 1)
+        upper = np.stack([mx + ux * res, my + uy * res], 1)
+        d = np.concatenate([line, upper]) - (sx, sy)
+        ins.append((np.arctan2(d[:, 1], d[:, 0]) - th, np.hypot(d[:, 0], d[:, 1]), np.array([sx, sy, th])))
+    return dense, mx, my, ins, params
+
+
+def test_near_edge_points_are_tested_one_cell_either_side():
+    """band_edge_scene on the reference's tables: the plain flag never fires; with edge_eps 0.3 the +-1 test
+    of near-edge points flags exactly the scans whose row-5 points lie near their cells' lower edge, and with
+    a zero band it adds nothing.  Every match the extended flag leaves unflagged has bounded coarse scores."""
+    from oracle import backend
+    R = backend()
+    dense, mx, my, ins, params = band_edge_scene(np.random.default_rng(21))
+    refmap = R.RefMap.from_dense(dense, mx, my)
+    pre = refmap.precompute(5)
+    nx, ny = refmap.geometry()[:2]
+    for k, (angles, ranges, init) in enumerate(ins):
+        flag, bounded, _, _ = _check(R, refmap, pre, angles, ranges, init, params)
+        assert not flag and bounded
+        ref = R.rtcsm_match(refmap, angles, ranges, init, pre=pre, **params)
+        _, idx, cnt = R.rtcsm_score_table(refmap, pre, False, 5, params["scan_range_max"], init, angles, ranges,
+                                          ref.stepT, ref.winT, -ref.winX, 25, -ref.winY, 25, want_table=False)
+        cells = idx[:, :cnt[0]]
+        assert (cells[..., 1] == 5).any(-1).all()                       # row-5 points in every slice
+        assert ((cells[..., 1] == 5) | (cells[..., 1] >= 10)).all() and (cells[..., 0] >= 10).all()
+        geo = (ref.winX, ref.winY, 25, 25, 5, nx, ny)
+        for eps, want in ((0.3, k % 2 == 1), (0.0, False)):
+            edge = near_edge(init, angles, ranges, ref.stepT, ref.winT, mx, my, 0.05, eps)
+            assert flagged(cells, *geo, edge) == want, (k, eps)
 
 
 def test_model_ties_keep_the_first_visit():
